@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """SeqPAN hot-path benchmark: queries/s of forward + span decode on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload anet|charades|tacos]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload anet|charades|tacos] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (SeqPAN.forward + infer_basic span decode + IoU counters) over one
 ActivityNet-shaped batch (B=256, L=100, 1024-d features; BASELINE.json configs[1]) of synthetic input.
@@ -454,7 +454,14 @@ def main():
     ap.add_argument("--shared-video", action="store_true",
                     help="dense-query workloads (tacos: 128 pairs per clip): every clip is stored, copied and encoded once "
                          "(forward(video_index=...), SURVEY.md section 8 row f1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (slogits, elogits, match_score, "
+                         "span_fracs; rank 0) as DIR/<name>.npy in float32, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.train or args.sweep > 0):
+        ap.error("--dump-outputs applies to the step benchmark (not to --impl reference, --train or --sweep)")
 
     from vmrframe_b200 import synth
     w = synth.WORKLOADS[args.workload]
@@ -578,6 +585,13 @@ def main():
     timed_launches = launches[0]   # the timed region only (the sustained legs below keep calling step())
     host_enqueue_ms = (time.perf_counter() - th0) * 1e3 / args.steps
     barrier()
+    if args.dump_outputs and rank == 0:
+        # read back now: the e2e, sustained and profiling passes below reuse the lane buffers
+        import numpy as np
+        o = bufs[(args.steps - 1) % len(lanes)]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, key in (("slogits", "slogits"), ("elogits", "elogits"), ("match_score", "match"), ("span_fracs", "fracs")):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), o[key].cpu().numpy().astype(np.float32))
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -45,10 +45,12 @@ def manifest_state_dict(w):
 def golden_case(name):
     """(workload, state_dict, batch, fixture) of one golden case, regenerated from seeds and
     checked against the checksums stored by tests/golden/make_golden.py."""
-    from cases import CASES
+    from cases import CASES, TAPPED
     from vmrframe_b200 import synth
     w = CASES[name]
     fx = dict(np.load(os.path.join(GOLDEN, f"{name}.npz")))
+    if name in TAPPED:
+        fx.update(np.load(os.path.join(GOLDEN, f"{name}_taps.npz")))
     sd = synth.randomize_state_dict(manifest_state_dict(w), seed=w.config_id)
     batch = synth.make_batch(w, 0)
     chk = np.asarray([float(batch["vfeats"].double().sum()), float(batch["vfeats"].double().abs().sum())])

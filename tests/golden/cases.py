@@ -16,3 +16,5 @@ CASES = {
 }
 # cases whose hooked intermediate tensors are stored (kept to one to bound the fixture size)
 TAPPED = {"charades_small"}
+# taps of a TAPPED case stored in <case>_taps.npz instead of <case>.npz: all of them in one file would exceed 1 MB
+LATE_TAPS = ("t2v", "v2t", "fuse", "fep_s", "fep_e")

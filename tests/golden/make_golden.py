@@ -46,7 +46,7 @@ def checksum(t):
 
 def main():
     from vmrframe_b200 import synth
-    from cases import CASES, TAPPED
+    from cases import CASES, LATE_TAPS, TAPPED
     S, CP, infer_basic, append_ious, get_i345_mi = import_reference()
     torch.set_num_threads(8)
     manifest_written = False
@@ -104,6 +104,7 @@ def main():
             "dab2_v": taps["dab2"][0].numpy(), "dab2_t": taps["dab2"][1].numpy(),
             "t2v": taps["t2v"][0].numpy(), "v2t": taps["v2t"][0].numpy(), "fuse": taps["fuse"][0].numpy(),
             "fep_s": taps["fep"][0].numpy(), "fep_e": taps["fep"][1].numpy()})
+            np.savez_compressed(os.path.join(HERE, f"{name}_taps.npz"), **{k: fx.pop(k) for k in LATE_TAPS})
         np.savez_compressed(os.path.join(HERE, f"{name}.npz"), **fx)
         print(name, {k: v.shape for k, v in fx.items() if v.ndim > 1}, "metrics", metrics)
 

@@ -5,6 +5,7 @@ import math
 import os
 
 import numpy as np
+import pytest
 import torch
 
 from conftest import ROOT
@@ -92,3 +93,39 @@ def test_reference_arm_prints_the_contract_line():
     assert line["value"] > 0 and math.isclose(line["value"], line["cpu_baseline"]["value"]) and math.isclose(line["value"], line["e2e"]["value"])
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1 and "charades" in line["cpu_baseline"]["sample"]
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and line["gpu_launches"] == 0
+
+
+def test_bench_rejects_what_it_cannot_time_or_dump():
+    import subprocess
+    import sys
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"], ["--train", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr[-2000:])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's outputs; with the same arguments every run sees the same inputs,
+    so two runs write the same arrays."""
+    import json
+    import subprocess
+    import sys
+    from vmrframe_b200 import synth
+    w = synth.WORKLOADS["charades"]
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "charades", "--steps", "3", "--warmup", "1",
+                            "--no-cpu-baseline", "--no-profile", "--no-sustained", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 3
+        dumps.append({f.stem: np.load(f) for f in d.glob("*.npy")})
+    a, b = dumps
+    shapes = {"slogits": (w.batch, w.vlen), "elogits": (w.batch, w.vlen), "match_score": (w.batch, w.vlen, 4), "span_fracs": (w.batch, 2)}
+    assert {k: v.shape for k, v in a.items()} == shapes and all(v.dtype == np.float32 for v in a.values())
+    assert np.allclose(a["match_score"].sum(-1), 1.0, atol=1e-5)
+    assert np.all(a["span_fracs"][:, 0] <= a["span_fracs"][:, 1]) and np.all((a["span_fracs"] >= 0) & (a["span_fracs"] <= 1))
+    for k in ("slogits", "elogits", "match_score"):
+        assert np.allclose(a[k], b[k], rtol=0, atol=1e-6), k
+    assert np.array_equal(a["span_fracs"], b["span_fracs"])
