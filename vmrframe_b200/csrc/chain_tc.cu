@@ -2,7 +2,7 @@
 // chain of row-local 128-wide projections on them without leaving the SM.  Activations between projections live
 // in TMEM (fp32 accumulators, 4 x 128 columns) and in shared memory (bf16 operand tiles, 128-byte swizzle);
 // weights stream through a 2-slot ring by TMA.  Thread layout: warp 0 = control (one elected thread issues the
-// weight TMA loads and every tcgen05.mma), warps 1..4 = workers (one TMEM lane = one row per thread): they build
+// weight TMA loads and every tcgen05.mma), the other warps = workers (TMEM lane = row of the thread): they build
 // the first operand tiles cooperatively (coalesced global reads, LayerNorm by warp shuffles) and run every
 // epilogue, each of which produces the next operand tile.  Control and workers hand over through two mbarriers
 // (operand tiles ready / accumulators ready) whose phases alternate step by step.
@@ -21,7 +21,6 @@ namespace {
 
 constexpr int KBB = 16384;          // one k-block of an operand tile: [128 rows][64 bf16]
 constexpr int TILE_B = 2 * KBB;     // [128][128] bf16
-constexpr int NTHREADS = 160;
 constexpr int CB_THREADS = 288;   // warp 0 control + 8 worker warps
 
 __device__ __forceinline__ void mma_tile(uint32_t tmem_d, uint32_t abuf, uint32_t wbuf, uint32_t idesc, bool accumulate) {
@@ -43,225 +42,8 @@ __device__ __forceinline__ void store_a16(uint32_t abuf, int row, int col, const
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// One DepthwiseSeparableConvBlock layer (models/layers.py:139-148), all of it in one launch:
-//   out = x0 + ReLU(PW(DW7(LN(x0))) + b),  x0 = x (+ pos[l] for the first layer, models/layers.py:396-399)
-// A CTA owns 128 consecutive rows of the flat row buffer.  Each worker warp walks its 32 rows (+3 halo rows each
-// side) once with coalesced 512-byte row loads, LayerNorm by warp shuffles, and a register-resident sliding window
-// for the 7-tap depthwise conv (every lane only ever needs its own 4 channels), writing the bf16 operand tile;
-// taps that would cross a segment (sample) boundary are masked, which is the conv's zero padding.  Then one
-// 128x128x128 UMMA and a ReLU/bias/residual epilogue straight to global memory.
+// Shared pieces of the chain kernels
 // ------------------------------------------------------------------------------------------------------------
-struct EncLayerParams {
-  const float* x;      // [Mtot,128] layer input
-  const float* pos;    // [>=len,128] position table or null
-  float* out;          // [Mtot,128] (must not alias x: neighbouring CTAs read halo rows of x)
-  const float* ln_g; const float* ln_b; const float* dw;  // [128], [128], [128,1,7]
-  const float* bias;   // [128] pointwise bias
-  long long Mtot;      // rows in the buffer
-  long long R1;        // first row of segment group 1 (== rows of group 0)
-  int len0, len1;      // segment lengths of the two groups (len1 unused when R1 == Mtot)
-};
-
-__global__ void __launch_bounds__(NTHREADS)
-enc_layer_kernel(const __grid_constant__ CUtensorMap tm_w, EncLayerParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t A = base, Wt = base + TILE_B;
-  uint8_t* tail = gen + 2 * TILE_B;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(tail);  // wfull, bar_a, bar_mma
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tail + 32);
-  float* fb = reinterpret_cast<float*>(tail + 64);     // pointwise bias [128]
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long m0 = (long long)blockIdx.x * 128;
-  const uint32_t wfull = smem_u32(bars), bar_a = smem_u32(bars + 1), bar_mma = smem_u32(bars + 2);
-
-  if (threadIdx.x == 0) {
-    mbar_init(wfull, 1);
-    mbar_init(bar_a, 128);
-    mbar_init(bar_mma, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(128)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  if (threadIdx.x < 128) fb[threadIdx.x] = __ldg(p.bias + threadIdx.x);
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-
-  if (warp == 0) {
-    if (lane == 0) {
-      mbar_expect_tx(wfull, TILE_B);
-      tma_load_2d(Wt, &tm_w, wfull, 0, 0);
-      tma_load_2d(Wt + KBB, &tm_w, wfull, 64, 0);
-      mbar_wait(bar_a, 0);
-      tcgen05_fence_after();
-      mbar_wait(wfull, 0);
-      mma_tile(tmem, A, Wt, make_idesc(128, 128), false);
-      umma_commit(bar_mma);
-    }
-  } else {
-    const int q = warp & 3;
-    const int col = lane * 4;
-    // segment position of a flat row: l in [0,len) or -1 when the row does not exist
-    auto seg_of = [&](long long fr, int& len) -> int {
-      if (fr < 0 || fr >= p.Mtot) { len = 1; return -1; }
-      if (fr < p.R1) { len = p.len0; return (int)(fr % p.len0); }
-      len = p.len1;
-      return (int)((fr - p.R1) % p.len1);
-    };
-    {
-      const float4 g = __ldg(reinterpret_cast<const float4*>(p.ln_g + col));
-      const float4 bt = __ldg(reinterpret_cast<const float4*>(p.ln_b + col));
-      float wg[4][7];
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-#pragma unroll
-        for (int j = 0; j < 7; ++j) wg[c][j] = __ldg(p.dw + (col + c) * 7 + j);
-      float4 win[8];  // LN'd rows k-7..k of this lane's 4 channels, slot = k & 7
-      const long long rbase = m0 + q * 32 - 3;
-#pragma unroll 1
-      for (int k0 = 0; k0 < 40; k0 += 8) {
-        float4 xv[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const long long fr = rbase + k0 + i;
-          float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (k0 + i < 38 && fr >= 0 && fr < p.Mtot) {
-            v = __ldg(reinterpret_cast<const float4*>(p.x + fr * 128 + col));
-            if (p.pos) {
-              int len;
-              const int l = seg_of(fr, len);
-              const float4 pp = __ldg(reinterpret_cast<const float4*>(p.pos + (long long)l * 128 + col));
-              v.x += pp.x; v.y += pp.y; v.z += pp.z; v.w += pp.w;
-            }
-          }
-          xv[i] = v;
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int k = k0 + i;
-          if (k < 38) {
-            const float4 x = xv[i];
-            float mean = x.x + x.y + x.z + x.w;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) mean += __shfl_xor_sync(0xffffffffu, mean, o);
-            mean *= (1.0f / 128.0f);
-            const float dx = x.x - mean, dy = x.y - mean, dz = x.z - mean, dw_ = x.w - mean;
-            float var = dx * dx + dy * dy + dz * dz + dw_ * dw_;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) var += __shfl_xor_sync(0xffffffffu, var, o);
-            const float rstd = rsqrtf(var * (1.0f / 128.0f) + 1e-6f);
-            win[i] = make_float4(dx * rstd * g.x + bt.x, dy * rstd * g.y + bt.y, dz * rstd * g.z + bt.z,
-                                 dw_ * rstd * g.w + bt.w);
-            if (k >= 6) {  // output row r = k - 6 of this warp: taps are flat rows k-6..k (slots (i+2+j)&7)
-              const int r = q * 32 + k - 6;
-              int len;
-              const int l = seg_of(m0 + r, len);
-              float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-              for (int j = 0; j < 7; ++j) {
-                const float4 t = win[(i + 2 + j) & 7];
-                const bool ok = l >= 0 && (l + j - 3) >= 0 && (l + j - 3) < len;
-                if (ok) {
-                  acc.x = fmaf(wg[0][j], t.x, acc.x);
-                  acc.y = fmaf(wg[1][j], t.y, acc.y);
-                  acc.z = fmaf(wg[2][j], t.z, acc.z);
-                  acc.w = fmaf(wg[3][j], t.w, acc.w);
-                }
-              }
-              st_shared_v2(A + sw128_chunk_offset<KBB>(r, col & ~7) + (col & 7) * 2, pack_bf16(acc.x, acc.y),
-                           pack_bf16(acc.z, acc.w));
-            }
-          }
-        }
-      }
-      tcgen05_fence_before();
-      fence_proxy_async();
-      mbar_arrive(bar_a);
-    }
-    // ---- epilogue: out = x0 + ReLU(acc + b) ----
-    const int row = q * 32 + lane;
-    const long long grow = m0 + row;
-    const bool valid = grow < p.Mtot;
-    int len;
-    const int l = seg_of(grow, len);
-    const uint32_t tq = tmem + ((uint32_t)(q * 32) << 16);
-    float4 nx[4];
-    auto load_res = [&](int c) {
-#pragma unroll
-      for (int j4 = 0; j4 < 4; ++j4) {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (valid) {
-          v = __ldg(reinterpret_cast<const float4*>(p.x + grow * 128 + c * 16 + j4 * 4));
-          if (p.pos) {
-            const float4 pp = __ldg(reinterpret_cast<const float4*>(p.pos + (long long)l * 128 + c * 16 + j4 * 4));
-            v.x += pp.x; v.y += pp.y; v.z += pp.z; v.w += pp.w;
-          }
-        }
-        nx[j4] = v;
-      }
-    };
-    load_res(0);
-    mbar_wait(bar_mma, 0);
-    tcgen05_fence_after();
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16];
-      tmem_ld16(tq + c * 16, r0);
-      float4 cx[4];
-#pragma unroll
-      for (int j4 = 0; j4 < 4; ++j4) cx[j4] = nx[j4];
-      if (c < 7) load_res(c + 1);
-      tmem_ld_wait();
-      if (valid) {
-#pragma unroll
-        for (int j4 = 0; j4 < 4; ++j4) {
-          float4 v;
-          v.x = cx[j4].x + fmaxf(__uint_as_float(r0[j4 * 4 + 0]) + fb[c * 16 + j4 * 4 + 0], 0.f);
-          v.y = cx[j4].y + fmaxf(__uint_as_float(r0[j4 * 4 + 1]) + fb[c * 16 + j4 * 4 + 1], 0.f);
-          v.z = cx[j4].z + fmaxf(__uint_as_float(r0[j4 * 4 + 2]) + fb[c * 16 + j4 * 4 + 2], 0.f);
-          v.w = cx[j4].w + fmaxf(__uint_as_float(r0[j4 * 4 + 3]) + fb[c * 16 + j4 * 4 + 3], 0.f);
-          *reinterpret_cast<float4*>(p.out + grow * 128 + c * 16 + j4 * 4) = v;
-        }
-      }
-    }
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(128) : "memory");
-  }
-}
-
-constexpr size_t ENC_LAYER_SMEM = 1024 + 2 * TILE_B + 64 + 128 * sizeof(float);
-
-// ------------------------------------------------------------------------------------------------------------
-// Shared pieces of the smaller chain kernels
-// ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t chain_begin(uint64_t* bars, int nbars, uint32_t worker_mask, uint32_t* tmem_slot,
-                                                int tmem_cols) {
-  // worker_mask bit i: barrier i is arrived on by all 128 worker threads (else by one thread / one commit)
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < nbars; ++i) mbar_init(smem_u32(bars + i), ((worker_mask >> i) & 1u) ? 128u : 1u);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if ((threadIdx.x >> 5) == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  return *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-}
 __device__ __forceinline__ void chain_end(uint32_t tmem, int tmem_cols) {
   tcgen05_fence_before();
   __syncthreads();
@@ -475,206 +257,6 @@ proj_ln_kernel(const __grid_constant__ CUtensorMap tm_wA, const __grid_constant_
   chain_end(tmem, 256);
 }
 constexpr size_t PROJ_LN_SMEM = 1024 + 3 * TILE_B + 128 + 5 * 128 * sizeof(float);
-
-// ------------------------------------------------------------------------------------------------------------
-// Tail of FeatureEncoderPredict (models/layers.py:632-639):  r = out_proj(att) + h;  out = dense(LN_1e-5(r)) + r
-// att arrives as bf16 by TMA; r stays in TMEM between the two projections.
-// ------------------------------------------------------------------------------------------------------------
-struct FepTailParams {
-  const float* h;    // residual input [M,128] fp32
-  float* out;        // [M,128] fp32 (may alias h)
-  long long M;
-  const float* b_o; const float* ln_g; const float* ln_b; const float* b_d;
-};
-
-__global__ void __launch_bounds__(NTHREADS)
-fep_tail_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_constant__ CUtensorMap tm_wo,
-                const __grid_constant__ CUtensorMap tm_wd, FepTailParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t P0 = base, W0 = base + TILE_B, W1 = base + 2 * TILE_B;  // P0: att, then LN(r)
-  uint8_t* tail = gen + 3 * TILE_B;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(tail);  // 0 in_full, 1 w1_full, 2 bar_a, 3 bar_mma
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tail + 64);
-  float* fp = reinterpret_cast<float*>(tail + 128);    // b_o, ln_g, ln_b, b_d
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long m0 = (long long)blockIdx.x * 128;
-  for (int i = threadIdx.x; i < 512; i += NTHREADS) {
-    const float* src = i < 128 ? p.b_o : (i < 256 ? p.ln_g : (i < 384 ? p.ln_b : p.b_d));
-    fp[i] = __ldg(src + (i & 127));
-  }
-  const uint32_t tmem = chain_begin(bars, 4, 1u << 2, tmem_slot, 256);
-  const uint32_t in_full = smem_u32(bars), w1_full = smem_u32(bars + 1), bar_a = smem_u32(bars + 2),
-                 bar_mma = smem_u32(bars + 3);
-  if (warp == 0) {
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc(128, 128);
-      mbar_expect_tx(in_full, 2 * TILE_B);
-      tma_load_2d(P0, &tm_att, in_full, 0, (int)m0);
-      tma_load_2d(P0 + KBB, &tm_att, in_full, 64, (int)m0);
-      tma_load_2d(W0, &tm_wo, in_full, 0, 0);
-      tma_load_2d(W0 + KBB, &tm_wo, in_full, 64, 0);
-      mbar_expect_tx(w1_full, TILE_B);
-      tma_load_2d(W1, &tm_wd, w1_full, 0, 0);
-      tma_load_2d(W1 + KBB, &tm_wd, w1_full, 64, 0);
-      mbar_wait(in_full, 0);
-      mma_tile(tmem, P0, W0, idesc, false);
-      umma_commit(bar_mma);
-      mbar_wait(bar_a, 0);
-      tcgen05_fence_after();
-      mbar_wait(w1_full, 0);
-      mma_tile(tmem + 128, P0, W1, idesc, false);
-      umma_commit(bar_mma);
-    }
-  } else {
-    const int q = warp & 3, row = q * 32 + lane;
-    const long long grow = m0 + row;
-    const bool valid = grow < p.M;
-    const uint32_t tq = tmem + ((uint32_t)(q * 32) << 16);
-    float4 nx[4];
-    auto load_res = [&](int c) {
-#pragma unroll
-      for (int j4 = 0; j4 < 4; ++j4)
-        nx[j4] = valid ? __ldg(reinterpret_cast<const float4*>(p.h + grow * 128 + c * 16 + j4 * 4))
-                       : make_float4(0.f, 0.f, 0.f, 0.f);
-    };
-    load_res(0);
-    mbar_wait(bar_mma, 0);
-    tcgen05_fence_after();
-    float sum = 0.f;
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16];
-      tmem_ld16(tq + c * 16, r0);
-      float xi[16];
-#pragma unroll
-      for (int j4 = 0; j4 < 4; ++j4) { xi[j4 * 4] = nx[j4].x; xi[j4 * 4 + 1] = nx[j4].y; xi[j4 * 4 + 2] = nx[j4].z; xi[j4 * 4 + 3] = nx[j4].w; }
-      if (c < 7) load_res(c + 1);
-      tmem_ld_wait();
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const float r = __uint_as_float(r0[j]) + fp[c * 16 + j] + xi[j];
-        sum += r;
-        r0[j] = __float_as_uint(r);
-      }
-      tmem_st16(tq + c * 16, r0);
-    }
-    tmem_st_wait();
-    const float mean = sum * (1.0f / 128.0f);
-    float var = 0.f;
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16];
-      tmem_ld16(tq + c * 16, r0);
-      tmem_ld_wait();
-#pragma unroll
-      for (int j = 0; j < 16; ++j) { const float d = __uint_as_float(r0[j]) - mean; var = fmaf(d, d, var); }
-    }
-    const float rstd = rsqrtf(var * (1.0f / 128.0f) + 1e-5f);
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16];
-      tmem_ld16(tq + c * 16, r0);
-      tmem_ld_wait();
-      float n[16];
-#pragma unroll
-      for (int j = 0; j < 16; ++j) n[j] = (__uint_as_float(r0[j]) - mean) * rstd * fp[128 + c * 16 + j] + fp[256 + c * 16 + j];
-      store_a16(P0, row, c * 16, n);
-    }
-    tcgen05_fence_before();
-    fence_proxy_async();
-    mbar_arrive(bar_a);
-    mbar_wait(bar_mma, 1);
-    tcgen05_fence_after();
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16], r1[16];
-      tmem_ld16(tq + c * 16, r0);
-      tmem_ld16(tq + 128 + c * 16, r1);
-      tmem_ld_wait();
-      if (valid) {
-#pragma unroll
-        for (int j4 = 0; j4 < 4; ++j4) {
-          float4 v;
-          v.x = __uint_as_float(r1[j4 * 4 + 0]) + fp[384 + c * 16 + j4 * 4 + 0] + __uint_as_float(r0[j4 * 4 + 0]);
-          v.y = __uint_as_float(r1[j4 * 4 + 1]) + fp[384 + c * 16 + j4 * 4 + 1] + __uint_as_float(r0[j4 * 4 + 1]);
-          v.z = __uint_as_float(r1[j4 * 4 + 2]) + fp[384 + c * 16 + j4 * 4 + 2] + __uint_as_float(r0[j4 * 4 + 2]);
-          v.w = __uint_as_float(r1[j4 * 4 + 3]) + fp[384 + c * 16 + j4 * 4 + 3] + __uint_as_float(r0[j4 * 4 + 3]);
-          *reinterpret_cast<float4*>(p.out + grow * 128 + c * 16 + j4 * 4) = v;
-        }
-      }
-    }
-  }
-  chain_end(tmem, 256);
-}
-constexpr size_t FEP_TAIL_SMEM = 1024 + 3 * TILE_B + 128 + 512 * sizeof(float);
-
-// ------------------------------------------------------------------------------------------------------------
-// Start/end logit head (models/layers.py:663-670): logits = dense(hidden(cat[LN_1e-6(feat), x])) per row.
-// The 256-wide concat is never materialised: the K=256 projection is two accumulating UMMAs over the two operand
-// tiles; the 128 -> 1 projection is a thread-local dot product over the accumulator row in TMEM.
-// ------------------------------------------------------------------------------------------------------------
-struct HeadParams {
-  const float* feat;  // [M,128] s or e
-  const float* x;     // [M,128] predictor input (fuse2)
-  long long M;
-  const float* ln_g; const float* ln_b; const float* b_h; const float* w_d; const float* b_d;
-  float* logits;      // [M]
-};
-
-__global__ void __launch_bounds__(NTHREADS)
-head_kernel(const __grid_constant__ CUtensorMap tm_wh, HeadParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t P0 = base, P1 = base + TILE_B, Wt = base + 2 * TILE_B;   // Wt: [128][256] bf16 = 4 k-blocks
-  uint8_t* tail = gen + 4 * TILE_B;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(tail);  // 0 wfull, 1 bar_a, 2 bar_mma
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tail + 64);
-  float* fp = reinterpret_cast<float*>(tail + 128);    // b_h, w_d
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long m0 = (long long)blockIdx.x * 128;
-  for (int i = threadIdx.x; i < 256; i += NTHREADS) fp[i] = __ldg((i < 128 ? p.b_h : p.w_d) + (i & 127));
-  const uint32_t tmem = chain_begin(bars, 3, 1u << 1, tmem_slot, 128);
-  const uint32_t wfull = smem_u32(bars), bar_a = smem_u32(bars + 1), bar_mma = smem_u32(bars + 2);
-  if (warp == 0) {
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc(128, 128);
-      mbar_expect_tx(wfull, 2 * TILE_B);
-      for (int kb = 0; kb < 4; ++kb) tma_load_2d(Wt + kb * KBB, &tm_wh, wfull, kb * 64, 0);
-      mbar_wait(bar_a, 0);
-      tcgen05_fence_after();
-      mbar_wait(wfull, 0);
-      mma_tile(tmem, P0, Wt, idesc, false);
-      mma_tile(tmem, P1, Wt + TILE_B, idesc, true);
-      umma_commit(bar_mma);
-    }
-  } else {
-    const int q = warp & 3, row = q * 32 + lane;
-    const long long grow = m0 + row;
-    rows_to_tiles(p.feat, p.M, m0, q * 32, lane, 1e-6f, p.ln_g, p.ln_b, P0, nullptr, nullptr, 0u);
-    rows_to_tiles(p.x, p.M, m0, q * 32, lane, 0.f, nullptr, nullptr, P1, nullptr, nullptr, 0u);
-    tcgen05_fence_before();
-    fence_proxy_async();
-    mbar_arrive(bar_a);
-    mbar_wait(bar_mma, 0);
-    tcgen05_fence_after();
-    const uint32_t tq = tmem + ((uint32_t)(q * 32) << 16);
-    float acc = 0.f;
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      uint32_t r0[16];
-      tmem_ld16(tq + c * 16, r0);
-      tmem_ld_wait();
-#pragma unroll
-      for (int j = 0; j < 16; ++j) acc = fmaf(__uint_as_float(r0[j]) + fp[c * 16 + j], fp[128 + c * 16 + j], acc);
-    }
-    if (grow < p.M) p.logits[grow] = acc + __ldg(p.b_d);
-  }
-  chain_end(tmem, 128);
-}
-constexpr size_t HEAD_SMEM = 1024 + 4 * TILE_B + 128 + 256 * sizeof(float);
 
 // ------------------------------------------------------------------------------------------------------------
 // Whole DepthwiseSeparableConvBlock (4 layers, models/layers.py:139-148) + the position add of FeatureEncoder
@@ -1189,26 +771,6 @@ const char* chain_last_error() { return g_chain_err; }
 
 int chain_read_timeline(long long* out64) { return tl_read(out64); }
 
-int chain_enc_layer(const TcArena& a, int slot, const float* x, const float* pos, float* out, const float* ln_g,
-                    const float* ln_b, const float* dw, const float* bias, long long Mtot, long long R1, int len0,
-                    int len1, cudaStream_t st) {
-  if (Mtot <= 0) return SEQPAN_OK;
-  if (x == out) { snprintf(g_chain_err, sizeof(g_chain_err), "enc_layer: out must not alias x"); return SEQPAN_E_INVALID; }
-  static SqSmemOptIn optin;
-  {
-    cudaError_t e = optin.ensure((const void*)enc_layer_kernel, ENC_LAYER_SMEM);
-    if (e != cudaSuccess) { snprintf(g_chain_err, sizeof(g_chain_err), "%s", cudaGetErrorString(e)); return SEQPAN_E_CUDA; }
-  }
-  EncLayerParams p;
-  p.x = x; p.pos = pos; p.out = out; p.ln_g = ln_g; p.ln_b = ln_b; p.dw = dw; p.bias = bias;
-  p.Mtot = Mtot; p.R1 = R1; p.len0 = len0; p.len1 = len1 > 0 ? len1 : 1;
-  enc_layer_kernel<<<(unsigned)((Mtot + 127) / 128), NTHREADS, ENC_LAYER_SMEM, st>>>(
-      *reinterpret_cast<const CUtensorMap*>(a.slot[slot].tmap), p);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) { snprintf(g_chain_err, sizeof(g_chain_err), "%s", cudaGetErrorString(e)); return SEQPAN_E_CUDA; }
-  return SEQPAN_OK;
-}
-
 static int chain_set_smem(SqSmemOptIn& optin, const void* fn, size_t bytes) {
   cudaError_t e = optin.ensure(fn, bytes);
   if (e != cudaSuccess) { snprintf(g_chain_err, sizeof(g_chain_err), "%s", cudaGetErrorString(e)); return SEQPAN_E_CUDA; }
@@ -1240,39 +802,6 @@ int chain_proj_ln(const TcArena& a, int slotA, int slotB, const float* x, long l
   return chain_check_launch();
 }
 
-int chain_fep_tail(const TcArena& a, const void* att_bf16, const float* h, float* out, long long M, const float* b_o,
-                   const float* ln_g, const float* ln_b, const float* b_d, cudaStream_t st) {
-  if (M <= 0) return SEQPAN_OK;
-  static SqSmemOptIn optin;
-  { int rc = chain_set_smem(optin, (const void*)fep_tail_kernel, FEP_TAIL_SMEM); if (rc) return rc; }
-  CUtensorMap tm_att;
-  if (tc_make_act_tmap(&tm_att, att_bf16, M, 128, 128) != SEQPAN_OK) {
-    snprintf(g_chain_err, sizeof(g_chain_err), "%s", tc_last_error());
-    return SEQPAN_E_CUDA;
-  }
-  FepTailParams p;
-  p.h = h; p.out = out; p.M = M; p.b_o = b_o; p.ln_g = ln_g; p.ln_b = ln_b; p.b_d = b_d;
-  fep_tail_kernel<<<(unsigned)((M + 127) / 128), NTHREADS, FEP_TAIL_SMEM, st>>>(
-      tm_att, *reinterpret_cast<const CUtensorMap*>(a.slot[TC_OUTPROJ].tmap),
-      *reinterpret_cast<const CUtensorMap*>(a.slot[TC_PRED_DENSE].tmap), p);
-  return chain_check_launch();
-}
-
-int chain_head(const TcArena& a, int slot_hidden, const float* feat, const float* x, long long M, const float* ln_g,
-               const float* ln_b, const float* b_h, const float* w_d, const float* b_d, float* logits, cudaStream_t st) {
-  if (M <= 0) return SEQPAN_OK;
-  static SqSmemOptIn optin;
-  { int rc = chain_set_smem(optin, (const void*)head_kernel, HEAD_SMEM); if (rc) return rc; }
-  HeadParams p;
-  p.feat = feat; p.x = x; p.M = M; p.ln_g = ln_g; p.ln_b = ln_b; p.b_h = b_h; p.w_d = w_d; p.b_d = b_d; p.logits = logits;
-  head_kernel<<<(unsigned)((M + 127) / 128), NTHREADS, HEAD_SMEM, st>>>(
-      *reinterpret_cast<const CUtensorMap*>(a.slot[slot_hidden].tmap), p);
-  return chain_check_launch();
-}
-
-// group 0 may hold long segments (tiled with halos, at most SEQPAN_MAX_VLEN rows); group 1 segments must fit one tile
-bool chain_conv_block_supported(int len0, int len1) { return len0 >= 1 && len0 <= SEQPAN_MAX_VLEN && len1 <= 128 && !(len0 > 128 && sq_env().no_halo); }
-
 size_t chain_conv_tab_floats() { return CONV_TAB_FLOATS; }
 
 int chain_conv_tables(const float* const* ln_g, const float* const* ln_b, const float* const* dw, const float* const* bias,
@@ -1285,6 +814,11 @@ int chain_conv_tables(const float* const* ln_g, const float* const* ln_b, const 
 int chain_conv_block(const TcArena& a, int slot0, const float* x, const float* pos, float* out, const float* tab, int nseg0,
                      int len0, int nseg1, int len1, cudaStream_t st, const ChainProjTail* tail, int nlayers) {
   if (nlayers != 2 && nlayers != 4) { snprintf(g_chain_err, sizeof(g_chain_err), "conv block: 2 or 4 layers"); return SEQPAN_E_INVALID; }
+  // group 0 may hold long segments (tiled with halos, at most SEQPAN_MAX_VLEN rows); group 1 segments must fit one tile
+  if (len0 < 1 || len0 > SEQPAN_MAX_VLEN || len1 > 128) {
+    snprintf(g_chain_err, sizeof(g_chain_err), "conv block: segment lengths %d / %d outside [1,%d] / [0,128]", len0, len1, SEQPAN_MAX_VLEN);
+    return SEQPAN_E_INVALID;
+  }
   static SqSmemOptIn optin;
   { int rc = chain_set_smem(optin, (const void*)conv_block4_kernel, CONV_BLOCK_SMEM); if (rc) return rc; }
   ConvBlockParams p;
@@ -1297,7 +831,7 @@ int chain_conv_block(const TcArena& a, int slot0, const float* x, const float* p
   int tiles1 = (len1 > 0 && nseg1 > 0) ? (nseg1 + G1 - 1) / G1 : 0;
   // pair mode: one long segment + the short segments that fit behind it in the same 128-row tile (a clip and its query)
   p.pair = 0;
-  if (tiles1 > 0 && G0 == 1 && !p.halo0 && len0 + len1 <= 128 && !sq_env().no_pair) {
+  if (tiles1 > 0 && G0 == 1 && !p.halo0 && len0 + len1 <= 128) {
     const int g1 = (128 - len0) / len1;
     if ((long long)nseg0 * g1 >= nseg1) { p.pair = g1; tiles1 = 0; }
   }
@@ -1316,7 +850,7 @@ int chain_conv_block(const TcArena& a, int slot0, const float* x, const float* p
     for (int i = 0; i < 3; ++i) { pt.hb[i] = tail->hb ? tail->hb[i] : nullptr; pt.hb_stride[i] = i < 2 ? 64 : 32; }
     pt.hbL = tail->hbL > 0 ? tail->hbL : 1; pt.hbB = tail->hbB; pt.hb_mask = tail->hb_mask;
     // head-blocked outputs by TMA: one whole sample per tile (so a tile is one (b, all l) block) and no second operand tile
-    pt.hb_tma = (tail->hb && G0 == 1 && !p.halo0 && nseg1 == 0 && pt.nB == 0 && len0 == pt.hbL && !sq_env().no_hb_tma) ? 1 : 0;
+    pt.hb_tma = (tail->hb && G0 == 1 && !p.halo0 && nseg1 == 0 && pt.nB == 0 && len0 == pt.hbL) ? 1 : 0;
   }
   CUtensorMap hq, hk, hv, hq16, hk16;
   memset(&hq, 0, sizeof(hq)); memset(&hk, 0, sizeof(hk)); memset(&hv, 0, sizeof(hv)); memset(&hq16, 0, sizeof(hq16)); memset(&hk16, 0, sizeof(hk16));

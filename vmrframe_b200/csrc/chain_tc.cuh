@@ -18,12 +18,6 @@ int chain_dab_post(const TcArena& a, int block, const void* sa_bf16, const void*
                    const float* vmask, const float* tmask, long long Mv, long long M, const float* const* hostv,
                    const float* ln1_g, const float* ln1_b, cudaStream_t st);
 
-// One conv-block layer in one launch: out = x0 + ReLU(PW(DW7(LN(x0))) + b), x0 = x (+ pos).  Rows [0,R1) are segments
-// of len0 rows, rows [R1,Mtot) segments of len1 rows.  `slot` = tensor-core slot of the pointwise weight.
-int chain_enc_layer(const TcArena& a, int slot, const float* x, const float* pos, float* out, const float* ln_g,
-                    const float* ln_b, const float* dw, const float* bias, long long Mtot, long long R1, int len0,
-                    int len1, cudaStream_t st);
-
 // out_A = LN_A(x).W_A^T + b_A and (slotB >= 0) out_B = LN_B(x).W_B^T + b_B from one read of x (fp32 outputs).
 int chain_proj_ln(const TcArena& a, int slotA, int slotB, const float* x, long long M, float eps, const float* gA,
                   const float* bA, const float* gB, const float* bB, float* outA, const float* biasA, float* outB,
@@ -37,15 +31,11 @@ int chain_proj_ln(const TcArena& a, int slotA, int slotB, const float* x, long l
 // (position l, head); q/k/v are the head-blocked bf16 tensors above; out is bf16 [B*L,128].  B <= 256.
 int attn_batch_tc(const void* q_hb, const void* k_hb, const void* v_hb, const float* vmask, void* out_bf16, int B, int L,
                   cudaStream_t st);
-// FeatureEncoderPredict tail: r = out_proj(att) + h; out = dense(LN_1e-5(r)) + r.  att is bf16 [M,128].
-int chain_fep_tail(const TcArena& a, const void* att_bf16, const float* h, float* out, long long M, const float* b_o,
-                   const float* ln_g, const float* ln_b, const float* b_d, cudaStream_t st);
-// logits[m] = dense(hidden(cat[LN_1e-6(feat[m]), x[m]])): slot_hidden = TC_START_HID / TC_END_HID.
-int chain_head(const TcArena& a, int slot_hidden, const float* feat, const float* x, long long M, const float* ln_g,
-               const float* ln_b, const float* b_h, const float* w_d, const float* b_d, float* logits, cudaStream_t st);
 
 // Fused row-local tails (tail_tc.cu).
-//   chain_fep_head   = chain_fep_tail + chain_head in one launch; x_bf16 = bf16 copy of the predictor input [M,128].
+//   chain_fep_head   = FeatureEncoderPredict tail r = out_proj(att) + h; out = dense(LN_1e-5(r)) + r (att bf16 [M,128]),
+//                      then the logit head logits = dense(hidden(cat[LN_1e-6(out), x])) in one launch;
+//                      slot_hidden = TC_START_HID / TC_END_HID, x_bf16 = bf16 copy of the predictor input [M,128].
 //   chain_fuse_match = CQConcatenate's projection (t2v half by tensor core, pooled half as the per-sample bias `pbias`
 //                      [B,128]) + the match head; writes fuse, fuse2 (fp32), fuse2_bf16 and match_score.
 //   launch_pool_bias = WeightedPool + its half of the concat projection: pbias[b] = Wcat[:, 128:] . pool(v2t[b]).
@@ -68,8 +58,9 @@ bool attn_dual_tc_supported(int L, int T);
 int attn_dual_tc(const void* qkv_bf16, const void* tkv_bf16, const float* vmask, const float* tmask, void* sa_bf16,
                  void* xa_bf16, int B, int L, int T, cudaStream_t st);
 
-// Whole 4-layer conv block + position add in one launch for segments of <= 128 rows (group 0: nseg0 x len0 rows
-// starting at row 0, group 1: nseg1 x len1 rows right after).  slot0 = tensor-core slot of the first pointwise weight.
+// Whole 4-layer conv block + position add in one launch (group 0: nseg0 x len0 rows starting at row 0, len0 <=
+// SEQPAN_MAX_VLEN, segments longer than 128 rows are tiled with halos; group 1: nseg1 x len1 rows right after, len1 <= 128;
+// other lengths are SEQPAN_E_INVALID).  slot0 = tensor-core slot of the first pointwise weight.
 // Optional tail: the LayerNorm + projections that consume the block's output (same semantics as chain_proj_ln with bf16
 // row-major outputs, or head-blocked q/k/v when hb != nullptr), computed from the rows while they are still on the SM.
 struct ChainProjTail {
@@ -80,7 +71,6 @@ struct ChainProjTail {
   void* outA; void* outB;      // bf16 [Mtot, N]
   void* const* hb; int hbL, hbB; const float* hb_mask;
 };
-bool chain_conv_block_supported(int len0, int len1);
 // `tab` = chain_conv_tab_floats() floats built once per weight set by chain_conv_tables (pointwise biases + depthwise tap
 // tables with the LayerNorm affine folded in): every CTA bulk-copies them instead of rebuilding them.
 size_t chain_conv_tab_floats();

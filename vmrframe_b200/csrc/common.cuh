@@ -11,12 +11,11 @@
 #define SQ_MASK (-1e30f)  // models/layers.py:9 mask_value
 
 // ---- host-side process state shared by the launchers -------------------------------------------------------------------
-// A/B switches of the kernel selection (DESIGN.md section 5).  The environment is read ONCE per seqpan_create (not on the
-// forward path): sq_env() is the snapshot the launchers consult, sq_env_refresh() re-reads it.
+// SEQPAN_* run-time switches (DESIGN.md section 5).  The environment is read ONCE per seqpan_create (not on the forward
+// path): sq_env() is the snapshot the launchers consult, sq_env_refresh() re-reads it.
 struct SqEnv {
-  bool no_fuse = false, no_tc_attn = false, no_fuse_tails = false, no_tf32_cqlin = false, no_ln_fuse = false, no_tail_fuse = false,
-       no_joint_attn = false, no_halo = false, no_pair = false, no_hb_tma = false, no_graph = false, force_graph = false, no_cq_wide = false, no_side_stream = false;
-  int cq_threads = 1024, h2d_threads = 128, tf32_diag = 0, tl_query = 0;
+  bool no_joint_attn = false, no_graph = false, force_graph = false, no_side_stream = false;
+  int h2d_threads = 128;
 };
 const SqEnv& sq_env();
 void sq_env_refresh();

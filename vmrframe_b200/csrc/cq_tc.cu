@@ -21,7 +21,7 @@ namespace {
 
 constexpr int KBB = 16384;
 constexpr int TILE_B = 2 * KBB;
-constexpr int CQ_THREADS = 288;
+constexpr int CQ_TC_THREADS = 288;
 constexpr float MASKV = -1e30f;
 constexpr float LOG2E = 1.4426950408889634f;
 
@@ -55,7 +55,7 @@ __device__ __forceinline__ void store_a16(uint32_t abuf, int row, int col, const
                pack_bf16(v[12], v[13]), pack_bf16(v[14], v[15]));
 }
 
-__global__ void __launch_bounds__(CQ_THREADS, 1)
+__global__ void __launch_bounds__(CQ_TC_THREADS, 1)
 cq_tc_kernel(const __grid_constant__ CUtensorMap tm_w0, const __grid_constant__ CUtensorMap tm_w1, CqTcParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -407,7 +407,7 @@ int cq_attention_tc(const TcArena& a, const float* x, const float* vmask, const 
   for (int d = 0; d < 2; ++d) { p.w4c[d] = w4c[d]; p.w4q[d] = w4q[d]; p.w4mlu[d] = w4mlu[d]; p.bias[d] = bias[d]; }
   p.out[0] = out_v; p.out[1] = out_t; p.ldo[0] = ldo_v; p.ldo[1] = ldo_t;
   p.B = B; p.L = L; p.T = T;
-  cq_tc_kernel<<<dim3(B, 2), CQ_THREADS, CQ_TC_SMEM, st>>>(*reinterpret_cast<const CUtensorMap*>(a.slot[TC_Q2V_LIN].tmap),
+  cq_tc_kernel<<<dim3(B, 2), CQ_TC_THREADS, CQ_TC_SMEM, st>>>(*reinterpret_cast<const CUtensorMap*>(a.slot[TC_Q2V_LIN].tmap),
                                                            *reinterpret_cast<const CUtensorMap*>(a.slot[TC_V2Q_LIN].tmap), p);
   return cudaGetLastError() == cudaSuccess ? SEQPAN_OK : SEQPAN_E_CUDA;
 }

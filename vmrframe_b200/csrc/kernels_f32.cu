@@ -746,15 +746,14 @@ cudaError_t launch_cq_attention(const CqArgs& a_in, cudaStream_t st) {
   CqArgs a = a_in;
   a.stage_video = cq_smem_bytes(a.L, a.T, true) <= 200 * 1024 ? 1 : 0;
   const size_t smem = cq_smem_bytes(a.L, a.T, a.stage_video != 0);
-  const int big = sq_env().cq_threads;   // block size when only one CTA fits an SM (SEQPAN_CQ_THREADS, A/B tests)
-  const int nt = smem > 100 * 1024 ? big : 256;
+  const int nt = smem > 100 * 1024 ? 1024 : 256;   // block size 1024 when only one CTA fits an SM
   auto launch = [&](auto kern) -> cudaError_t {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return e;
     kern<<<dim3(a.B, 2), nt, smem, st>>>(a);
     return cudaSuccess;
   };
-  cudaError_t e = nt == 256 ? launch(cq_attention_kernel<256>) : (nt == 512 ? launch(cq_attention_kernel<512>) : launch(cq_attention_kernel<1024>));
+  cudaError_t e = nt == 256 ? launch(cq_attention_kernel<256>) : launch(cq_attention_kernel<1024>);
   if (e != cudaSuccess) return e;
   return cudaGetLastError();
 }

@@ -6,7 +6,8 @@
 //               releases stages back to the producer and finally signals the epilogue
 //   warps 2..5  epilogue: tcgen05.ld of the accumulator (one TMEM lane = one output row per thread), transposed
 //               through shared memory so that bias/ReLU/residual and the global stores are fully coalesced
-// Replaces Conv1D(k=1) (models/layers.py:15-26) wherever the bf16 mode runs a projection.
+// Replaces Conv1D(k=1) (models/layers.py:15-26) wherever no fused chain kernel does: every projection of the tf32 mode, the
+// two embedding projections (+ LayerNorm) and the L > 128 cqa_linear of the bf16 mode (kind::tf32), and seqpan_op_linear.
 #include <cuda.h>
 #include <cuda_bf16.h>
 
@@ -43,7 +44,6 @@ struct TcParams {
   int N;
   int num_kb;   // ceil(K / 64)
   int stages;   // 1..MAX_STAGES
-  int diag;     // timing diagnostics only (SEQPAN_TF32_DIAG): bit 0 skips the activation loads, bit 1 the weight loads
   int relu;
   // LayerNorm fused behind the projection (N == 128 only): y = LN(x.w^T + bias; ln_g, ln_b, ln_eps); the tile leaves through
   // the TMA store map `tmY` (fp32 [M,128], 4 boxes of 32 floats)
@@ -71,8 +71,9 @@ __global__ void __launch_bounds__(NUM_THREADS) tc_linear_kernel(const __grid_con
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m0 = blockIdx.x * BM, n0 = blockIdx.y * BN;
-#define LTL(i) do { if (p.diag & 4) TL(i); } while (0)
-#define LTLC(i, t) do { if ((p.diag & 4) && threadIdx.x == (t)) TLC(i); } while (0)
+  // phase timeline of the instrumented build: stamped by the kind::tf32 launches with M >= 10000 (the video affine)
+#define LTL(i) do { if (TF32 && p.M >= 10000) TL(i); } while (0)
+#define LTLC(i, t) do { if (TF32 && p.M >= 10000 && threadIdx.x == (t)) TLC(i); } while (0)
   LTL(0);
 
   if (threadIdx.x == 0) {
@@ -85,12 +86,10 @@ __global__ void __launch_bounds__(NUM_THREADS) tc_linear_kernel(const __grid_con
     // the first ring of loads needs no free slot: on its way before the TMEM allocation / CTA barrier below
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmW);
-    if ((p.diag & 3) == 0) {
-      for (int kb = 0; kb < stages; ++kb) {   // stages <= num_kb
-        mbar_expect_tx(full0 + 8 * kb, A_STAGE + W_STAGE);
-        tma_load_2d(a_smem + kb * A_STAGE, &tmA, full0 + 8 * kb, kb * BKE, m0);
-        tma_load_2d(w_smem + kb * W_STAGE, &tmW, full0 + 8 * kb, kb * BKE, n0);
-      }
+    for (int kb = 0; kb < stages; ++kb) {   // stages <= num_kb
+      mbar_expect_tx(full0 + 8 * kb, A_STAGE + W_STAGE);
+      tma_load_2d(a_smem + kb * A_STAGE, &tmA, full0 + 8 * kb, kb * BKE, m0);
+      tma_load_2d(w_smem + kb * W_STAGE, &tmW, full0 + 8 * kb, kb * BKE, n0);
     }
   }
   if (warp == 1) {  // whole warp: allocate BN TMEM columns (fp32 accumulator 128 lanes x BN columns)
@@ -106,21 +105,12 @@ __global__ void __launch_bounds__(NUM_THREADS) tc_linear_kernel(const __grid_con
 
   if (warp == 0) {
     if (lane == 0) {
-      const bool pre = (p.diag & 3) == 0;
-      int s = 0; uint32_t ph = pre ? 1u : 0u;   // running stage / phase: no integer division in the single-thread loops
-      for (int kb = pre ? stages : 0; kb < p.num_kb; ++kb) {
+      int s = 0; uint32_t ph = 1;   // running stage / phase: no integer division in the single-thread loops
+      for (int kb = stages; kb < p.num_kb; ++kb) {
         mbar_wait(empty0 + 8 * s, ph ^ 1);
-        if ((p.diag & 3) == 0) {
-          mbar_expect_tx(full0 + 8 * s, A_STAGE + W_STAGE);
-          tma_load_2d(a_smem + s * A_STAGE, &tmA, full0 + 8 * s, kb * BKE, m0);
-          tma_load_2d(w_smem + s * W_STAGE, &tmW, full0 + 8 * s, kb * BKE, n0);
-        } else if ((p.diag & 3) == 3) {
-          mbar_arrive(full0 + 8 * s);
-        } else {
-          mbar_expect_tx(full0 + 8 * s, A_STAGE);
-          if ((p.diag & 3) == 2) tma_load_2d(a_smem + s * A_STAGE, &tmA, full0 + 8 * s, kb * BKE, m0);
-          else tma_load_2d(w_smem + s * W_STAGE, &tmW, full0 + 8 * s, kb * BKE, n0);
-        }
+        mbar_expect_tx(full0 + 8 * s, A_STAGE + W_STAGE);
+        tma_load_2d(a_smem + s * A_STAGE, &tmA, full0 + 8 * s, kb * BKE, m0);
+        tma_load_2d(w_smem + s * W_STAGE, &tmW, full0 + 8 * s, kb * BKE, n0);
         if (++s == stages) { s = 0; ph ^= 1; }
       }
     }
@@ -145,7 +135,9 @@ __global__ void __launch_bounds__(NUM_THREADS) tc_linear_kernel(const __grid_con
       }
       umma_commit(tfull);  // accumulator complete
       LTL(3);
-      if (p.diag & 4) { mbar_wait(tfull, 0); LTL(4); }
+#ifdef SEQPAN_TIMELINE
+      if (TF32 && p.M >= 10000) { mbar_wait(tfull, 0); LTL(4); }   // stamp 4: the last MMA has finished
+#endif
     }
   } else {
     // epilogue warps 2..5: TMEM lane quadrant = warp % 4
@@ -341,8 +333,6 @@ int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmW, const float* bias,
   p.stages = p.num_kb < MAX_STAGES ? p.num_kb : MAX_STAGES;
   if (tf32 && p.stages > 3) p.stages = 3;   // 3 x 32 KB stages: two CTAs per SM overlap loads with epilogues
   p.relu = relu;
-  p.diag = tf32 ? sq_env().tf32_diag : 0;
-  if (tf32 && ((M < 10000) == (sq_env().tl_query != 0))) p.diag |= 4;
   dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)(N / BN));
   if (tf32) tc_linear_kernel<true><<<grid, NUM_THREADS, tc_smem_bytes(p.stages), st>>>(tmA, tmW, tmY, p);
   else tc_linear_kernel<false><<<grid, NUM_THREADS, tc_smem_bytes(p.stages), st>>>(tmA, tmW, tmY, p);
@@ -359,13 +349,10 @@ inline size_t al256(size_t x) { return (x + 255) / 256 * 256; }
 // ---- interface -------------------------------------------------------------------------------------------------
 const char* tc_last_error() { return g_tc_err; }
 int tc_read_timeline(long long* out64) { return tl_read(out64); }
-int tc_extra_launches() { return 1; }  // the fp32 -> bf16 staging pass of the activation operand
 
-void tc_slot_shape(const SeqpanShapes& s, int slot, int& N, int& K) {
+static void tc_slot_shape(int slot, int& N, int& K) {
   N = 128; K = 128;
-  if (slot == TC_QUERY) K = 400;
-  else if (slot == TC_VIDEO) K = s.vdim;
-  else if (slot == TC_Q2V_LIN || slot == TC_V2Q_LIN) K = 512;
+  if (slot == TC_Q2V_LIN || slot == TC_V2Q_LIN) K = 512;
   else if (slot == TC_CAT || slot == TC_START_HID || slot == TC_END_HID) K = 256;
   else if (slot == TC_INPROJ) N = 384;
   else if (slot >= TC_DAB0 && slot < TC_DAB0 + 2 * TC_DAB_STRIDE) {
@@ -379,7 +366,7 @@ void tc_carve_arena(char* base, size_t& off, const SeqpanShapes& s, TcArena& a) 
   if (s.precision != SEQPAN_PREC_BF16) return;
   for (int i = 0; i < TC_NUM_SLOTS; ++i) {
     int N, K;
-    tc_slot_shape(s, i, N, K);
+    tc_slot_shape(i, N, K);
     off = al256(off);
     a.slot[i].w_bf16 = base ? base + off : nullptr;
     a.slot[i].N = N;
@@ -391,12 +378,6 @@ void tc_carve_arena(char* base, size_t& off, const SeqpanShapes& s, TcArena& a) 
 void tc_carve_workspace(char* base, size_t& off, const SeqpanShapes& s, int B, int T, TcWorkspace& w) {
   if (s.precision != SEQPAN_PREC_BF16) return;
   const size_t Mv = (size_t)B * s.vlen, M = Mv + (size_t)B * T;
-  size_t cap = Mv * (size_t)round8(s.vdim);           // video_affine input
-  if (M * 512 > cap) cap = M * 512;                   // widest concat input
-  off = al256(off);
-  w.a_bf16 = base ? base + off : nullptr;
-  w.a_capacity = cap;
-  off += cap * 2;
   off = al256(off);
   w.sa_bf16 = base ? base + off : nullptr;
   off += M * 128 * 2;
@@ -480,21 +461,6 @@ int tc_pack(const SeqpanShapes& s, const float* const* slot_src, TcArena& a, cud
   return SEQPAN_OK;
 }
 
-int tc_linear(const TcArena& a, const TcWorkspace& w, int slot, const float* x, int ldx, const float* bias,
-              const float* res, float* y, int ldy, long long M, int N, int K, bool relu, cudaStream_t st) {
-  if (M <= 0) return SEQPAN_OK;
-  const TcSlotInfo& si = a.slot[slot];
-  if (si.N != N || si.K != K) return tc_fail(SEQPAN_E_INVALID, "tensor-core slot shape mismatch");
-  const int Kp = round8(K);
-  if ((size_t)M * Kp > w.a_capacity) return tc_fail(SEQPAN_E_WORKSPACE, "bf16 staging buffer too small");
-  cudaError_t e = convert_bf16(x, ldx, M, K, Kp, w.a_bf16, st);
-  if (e != cudaSuccess) return tc_fail(SEQPAN_E_CUDA, cudaGetErrorString(e));
-  CUtensorMap tmA;
-  int rc = make_tmap(&tmA, w.a_bf16, M, K, Kp, BM);
-  if (rc != SEQPAN_OK) return rc;
-  return launch_tc(tmA, *reinterpret_cast<const CUtensorMap*>(si.tmap), bias, res, y, ldy, M, N, K, relu, st);
-}
-
 // fp32 operands straight from global memory (TMA) on kind::tf32: y = act(x.w^T + bias) (+res); no staging pass.
 int tc_linear_tf32(const float* x, int ldx, const float* w, const float* bias, const float* res, float* y, int ldy,
                    long long M, int N, int K, bool relu, cudaStream_t st, const float* ln_g, const float* ln_b, float ln_eps) {
@@ -506,18 +472,6 @@ int tc_linear_tf32(const float* x, int ldx, const float* w, const float* bias, c
   if (rc == SEQPAN_OK) rc = make_tmap(&tmW, w, N, K, K, BN, true);
   if (rc != SEQPAN_OK) return rc;
   return launch_tc(tmA, tmW, bias, res, y, ldy, M, N, K, relu, st, true, ln_g, ln_b, ln_eps);
-}
-
-// bf16 activation already in memory (written by the producing kernel): no staging pass.
-int tc_linear_bf16in(const TcArena& a, int slot, const void* x_bf16, int ldx, const float* bias, const float* res, float* y,
-                     int ldy, long long M, int N, int K, bool relu, cudaStream_t st) {
-  if (M <= 0) return SEQPAN_OK;
-  const TcSlotInfo& si = a.slot[slot];
-  if (si.N != N || si.K != K) return tc_fail(SEQPAN_E_INVALID, "tensor-core slot shape mismatch");
-  CUtensorMap tmA;
-  int rc = make_tmap(&tmA, x_bf16, M, K, ldx, BM);
-  if (rc != SEQPAN_OK) return rc;
-  return launch_tc(tmA, *reinterpret_cast<const CUtensorMap*>(si.tmap), bias, res, y, ldy, M, N, K, relu, st);
 }
 
 size_t tc_op_scratch_bytes(long long M, int N, int K) {

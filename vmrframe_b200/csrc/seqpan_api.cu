@@ -48,15 +48,10 @@ void sq_env_refresh() {
   auto on = [](const char* name) { const char* v = getenv(name); return v && v[0] == '1'; };
   auto num = [](const char* name, int dflt) { const char* v = getenv(name); return v ? atoi(v) : dflt; };
   SqEnv e;
-  e.no_fuse = on("SEQPAN_NO_FUSE"); e.no_tc_attn = on("SEQPAN_NO_TC_ATTN"); e.no_fuse_tails = on("SEQPAN_NO_FUSE_TAILS");
-  e.no_tf32_cqlin = on("SEQPAN_NO_TF32_CQLIN"); e.no_ln_fuse = on("SEQPAN_NO_LN_FUSE"); e.no_tail_fuse = on("SEQPAN_NO_TAIL_FUSE");
-  e.no_joint_attn = on("SEQPAN_NO_JOINT_ATTN"); e.no_halo = on("SEQPAN_NO_HALO"); e.no_pair = on("SEQPAN_NO_PAIR");
-  e.no_hb_tma = on("SEQPAN_NO_HB_TMA"); e.no_graph = on("SEQPAN_NO_GRAPH"); e.force_graph = on("SEQPAN_GRAPH"); e.no_side_stream = on("SEQPAN_NO_SIDE_STREAM"); e.no_cq_wide = on("SEQPAN_NO_CQ_WIDE");
-  e.cq_threads = num("SEQPAN_CQ_THREADS", 1024);
-  if (e.cq_threads != 256 && e.cq_threads != 512 && e.cq_threads != 1024) e.cq_threads = 1024;
+  e.no_joint_attn = on("SEQPAN_NO_JOINT_ATTN"); e.no_graph = on("SEQPAN_NO_GRAPH"); e.force_graph = on("SEQPAN_GRAPH");
+  e.no_side_stream = on("SEQPAN_NO_SIDE_STREAM");
   e.h2d_threads = num("SEQPAN_H2D_THREADS", 128);
   if (e.h2d_threads < 32 || e.h2d_threads > 1024 || (e.h2d_threads & 31)) e.h2d_threads = 128;
-  e.tf32_diag = num("SEQPAN_TF32_DIAG", 0); e.tl_query = num("SEQPAN_TL_QUERY", 0);
   g_env = e;
 }
 extern "C" int seqpan_num_weights(void) { return W_COUNT; }
@@ -213,9 +208,6 @@ struct SeqpanHandle {
   }
   // optional per-launch CUDA-event timing (seqpan_set_profile): tag -> events on the launching stream
   int profile = 0;
-  int tc_attn = 1;  // tcgen05 attention cores (SEQPAN_NO_TC_ATTN=1 selects the CUDA-core attention kernels)
-  int fuse_tails = 1;  // fused concat+match and FEP-tail+logit-head launches (SEQPAN_NO_FUSE_TAILS=1: separate kernels)
-  int fuse = 1;  // fused tcgen05 chain kernels (bf16 mode); SEQPAN_NO_FUSE=1 selects the per-projection kernels
   struct Rec { char tag[48]; cudaEvent_t a, b; };
   std::vector<Rec> recs;
   std::vector<cudaEvent_t> pool;
@@ -388,7 +380,6 @@ static int pack_weights(SeqpanHandle* h, cudaStream_t st) {
       if (rc != SEQPAN_OK) return fail(rc, "conv block table packing failed: %s", chain_last_error());
     }
     const float* src[TC_NUM_SLOTS] = {};
-    src[TC_QUERY] = w[W_QUERY_W]; src[TC_VIDEO] = w[W_VIDEO_W];
     for (int i = 0; i < 4; ++i) {
       src[TC_ENC_PW0 + i] = i < enc_layers ? w[W_ENC_PW0_W + 5 * i] : nullptr;   // nullptr: slot not used by this variant
       src[TC_PRED_PW0 + i] = w[W_PRED_PW0_W + 5 * i];
@@ -398,8 +389,6 @@ static int pack_weights(SeqpanHandle* h, cudaStream_t st) {
       const int d = base[k] - W_DAB1_LN1_W, ts = TC_DAB0 + k * TC_DAB_STRIDE;
       src[ts + TC_DAB_QKV] = a.dab[k].qkv_w; src[ts + TC_DAB_TKV] = a.dab[k].tkv_w; src[ts + TC_DAB_BIL] = a.dab[k].bil_w;
       src[ts + TC_DAB_SDENSE] = w[W_DAB1_SDENSE_W + d]; src[ts + TC_DAB_XDENSE] = w[W_DAB1_XDENSE_W + d];
-      src[ts + TC_DAB_SGATE] = w[W_DAB1_SGATE_W + d]; src[ts + TC_DAB_XGATE] = w[W_DAB1_XGATE_W + d];
-      src[ts + TC_DAB_GUIDED] = w[W_DAB1_GUIDED_W + d];
       src[ts + TC_DAB_D1] = w[W_DAB1_D1_W + d]; src[ts + TC_DAB_D2] = w[W_DAB1_D2_W + d];
       src[ts + TC_DAB_SGSD] = a.dab[k].sgsd_w; src[ts + TC_DAB_XGXD] = a.dab[k].xgxd_w; src[ts + TC_DAB_BILGD] = a.dab[k].bilgd_w;
     }
@@ -435,7 +424,6 @@ extern "C" int seqpan_create(const SeqpanShapes* shapes, const float* const* wei
   if (!h) return fail(SEQPAN_E_INVALID, "out of host memory");
   h->s = *shapes;
   sq_env_refresh();   // the only place the SEQPAN_* switches are read: once per handle, never on the forward path
-  h->fuse = !sq_env().no_fuse; h->tc_attn = !sq_env().no_tc_attn; h->fuse_tails = !sq_env().no_fuse_tails;
   h->use_graph = sq_env().no_graph ? 0 : (sq_env().force_graph ? 1 : 2);
   if (!sq_env().no_side_stream && cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) == cudaSuccess) {
     if (cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
@@ -526,41 +514,23 @@ struct Fwd {
   cudaStream_t st;
   int B, L, T, C;
   long long Mv, Mt, M;
-  bool tc;
+  bool tc;             // SEQPAN_PREC_BF16: the fused tcgen05 chain kernels
   bool tf32 = false;   // SEQPAN_PREC_TF32: the fp32 schedule with every projection on tcgen05 kind::tf32
 
-  // y = act(x.w^T + b) (+res); tensor-core path when the handle runs in bf16 and the shape allows it
+  // y = act(x.w^T + b) (+res).  tf32 mode: kind::tf32 wherever the shape allows it.  bf16 mode reaches this only from the
+  // CUDA-core CQAttention path (L > 128): its two K = 512 cqa_linear projections read the fp32 concat once by TMA on
+  // kind::tf32, with no fp32 -> bf16 staging pass.
   int linear(const float* x, int ldx, const float* w, const float* b, const float* res, float* y, int ldy, long long M_,
-             int N, int K, bool relu, int tc_slot = -1) {
-    // fp32 input read once by TMA, kind::tf32, no fp32 -> bf16 staging pass: the K = 1024 video affine and the K = 512
-    // cqa_linear projections of the unfused CQAttention path (L > 128)
-    if (tc && (tc_slot == TC_VIDEO || tc_slot == TC_Q2V_LIN || tc_slot == TC_V2Q_LIN) && h->fuse && !sq_env().no_tf32_cqlin) {
-      h->begin(tc_slot == TC_VIDEO ? "tc_linear_tf32_video" : "tc_linear_tf32_cqa", st);
-      int rc = tc_linear_tf32(x, ldx, w, b, res, y, ldy, M_, N, K, relu, st);
-      h->end(st);
-      if (rc != SEQPAN_OK) return fail(rc, "tc_linear_tf32 failed: %s", tc_last_error());
-      ++h->launches;
-      return SEQPAN_OK;
-    }
-    if (tf32 && N % 128 == 0 && !(K & 3) && !(ldx & 3)) {
+             int N, int K, bool relu) {
+    if (tc || (tf32 && N % 128 == 0 && !(K & 3) && !(ldx & 3))) {
       char tag[48];
-      snprintf(tag, sizeof(tag), "tc_linear_tf32_N%d_K%d", N, K);
+      if (tc) snprintf(tag, sizeof(tag), "tc_linear_tf32_cqa");
+      else snprintf(tag, sizeof(tag), "tc_linear_tf32_N%d_K%d", N, K);
       h->begin(tag, st);
       int rc = tc_linear_tf32(x, ldx, w, b, res, y, ldy, M_, N, K, relu, st);
       h->end(st);
       if (rc != SEQPAN_OK) return fail(rc, "tc_linear_tf32 failed: %s", tc_last_error());
       ++h->launches;
-      return SEQPAN_OK;
-    }
-    if (tc && tc_slot >= 0) {
-      char tag[48];
-      snprintf(tag, sizeof(tag), "tc_linear_N%d_K%d", N, K);
-      h->begin(tag, st);
-      int rc = tc_linear(h->arena.tc, ws.tc, tc_slot, x, ldx, b, res, y, ldy, M_, N, K, relu, st);
-      h->end(st);
-      if (rc != SEQPAN_OK) return fail(rc, "tc_linear(slot %d) failed: %s", tc_slot, tc_last_error());
-      ++h->launches;
-      h->launches += tc_extra_launches();
       return SEQPAN_OK;
     }
     LinearArgs a{};
@@ -574,12 +544,12 @@ struct Fwd {
     ++h->launches;
     return SEQPAN_OK;
   }
-  // VisualProjection (models/layers.py:118-123): Conv1D(vdim -> 128) + LayerNorm(1e-6).  bf16 mode: one launch, the fp32
-  // features are read once by TMA (kind::tf32) and the LayerNorm rides in the epilogue; `tmp` is the pre-LN buffer otherwise.
+  // VisualProjection (models/layers.py:118-123): Conv1D(vdim -> 128) + LayerNorm(1e-6).  bf16 / tf32 mode: one launch, the
+  // fp32 features are read once by TMA (kind::tf32) and the LayerNorm rides in the epilogue; `tmp` is the pre-LN buffer in fp32 mode.
   int video_affine(const float* x, long long rows, float* tmp, float* y) {
     const float* const* w = h->w;
     const SeqpanShapes& s = h->s;
-    if ((tf32 || (tc && h->fuse)) && !sq_env().no_ln_fuse) {
+    if (tf32 || tc) {
       h->begin("tc_linear_tf32_video+ln", st);
       int rc = tc_linear_tf32(x, s.vdim, w[W_VIDEO_W], w[W_VIDEO_B], nullptr, y, SQ_D, rows, SQ_D, s.vdim, false, st, w[W_VLN_W],
                               w[W_VLN_B], 1e-6f);
@@ -588,15 +558,15 @@ struct Fwd {
       ++h->launches;
       return SEQPAN_OK;
     }
-    int rc = linear(x, s.vdim, w[W_VIDEO_W], w[W_VIDEO_B], nullptr, tmp, SQ_D, rows, SQ_D, s.vdim, false, TC_VIDEO);
+    int rc = linear(x, s.vdim, w[W_VIDEO_W], w[W_VIDEO_B], nullptr, tmp, SQ_D, rows, SQ_D, s.vdim, false);
     return rc ? rc : ln(tmp, rows, W_VLN_W, 1e-6f, y);
   }
   int linear2(const float* x0, const float* w0, const float* b0, float* y0, const float* x1, const float* w1,
-              const float* b1, float* y1, long long M_, int slot0 = -1, int slot1 = -1) {
-    if ((tc && slot0 >= 0) || tf32) {
-      int rc = linear(x0, SQ_D, w0, b0, nullptr, y0, SQ_D, M_, SQ_D, SQ_D, false, slot0);
+              const float* b1, float* y1, long long M_) {
+    if (tf32) {
+      int rc = linear(x0, SQ_D, w0, b0, nullptr, y0, SQ_D, M_, SQ_D, SQ_D, false);
       if (rc != SEQPAN_OK) return rc;
-      return linear(x1, SQ_D, w1, b1, nullptr, y1, SQ_D, M_, SQ_D, SQ_D, false, slot1);
+      return linear(x1, SQ_D, w1, b1, nullptr, y1, SQ_D, M_, SQ_D, SQ_D, false);
     }
     LinearArgs a{};
     a.x[0] = x0; a.w[0] = w0; a.bias[0] = b0; a.y[0] = y0;
@@ -621,44 +591,23 @@ struct Fwd {
 
   // FeatureEncoder conv block (models/layers.py:139-148, 396-399): x0 = in + pos; 4x { x += ReLU(PW(DW(LN(x)))) }.
   // `enc` is the first weight id of the ENCODER() group; the result is left in `xout` (must differ from `in`).
-  // `tail` (optional): LayerNorm + projections of the block's consumer, fused behind the last layer when the whole-block
-  // kernel runs; *tail_done reports whether that happened (otherwise the caller launches chain_proj_ln itself).
+  // `tail` (optional, bf16 mode): LayerNorm + projections of the block's consumer, fused behind the last layer.
   int conv_block(const float* in, float* xout, int enc, const Segs& sg, long long rows, int tc_slot0,
-                 const ChainProjTail* tail = nullptr, bool* tail_done = nullptr) {
+                 const ChainProjTail* tail = nullptr) {
     // the shared FeatureEncoder of BaseFast has 2 layers (models/BaseFast.py:27); every other conv block has 4
     const int nl = (enc == W_ENC_POS && (h->s.variant == SEQPAN_VARIANT_BASEFAST || h->s.variant == SEQPAN_VARIANT_MULTITEACHER)) ? 2 : 4;
     float* tab = h->arena.conv_tab[enc == W_ENC_POS ? 0 : (enc == W_PRED_POS ? 1 : 2)];
-    if (tail_done) *tail_done = false;
-    if (tc && h->fuse && chain_conv_block_supported(sg.len[0], sg.nseg[1] > 0 ? sg.len[1] : 0)) {
-      const bool with_tail = tail && !sq_env().no_tail_fuse;
-      CHAIN(h, with_tail ? "chain_conv_block+proj" : "chain_conv_block",
+    if (tc) {
+      CHAIN(h, tail ? "chain_conv_block+proj" : "chain_conv_block",
             chain_conv_block(h->arena.tc, tc_slot0, in, h->w[enc], xout, tab, sg.nseg[0],
-                             sg.len[0], sg.nseg[1], sg.nseg[1] > 0 ? sg.len[1] : 0, st, with_tail ? tail : nullptr, nl));
-      if (tail_done) *tail_done = with_tail;
-      return SEQPAN_OK;
-    }
-    if (tc && h->fuse) {  // one fused launch per layer, ping-pong in -> z -> xout -> z -> xout
-      const long long R1 = (long long)sg.nseg[0] * sg.len[0];
-      const float* src = in;
-      for (int i = 0; i < nl; ++i) {
-        const int dwid = enc + 1 + 5 * i;
-        float* dst = (i & 1) ? xout : ws.z;
-        h->begin("chain_enc_layer", st);
-        int rc = chain_enc_layer(h->arena.tc, tc_slot0 + i, src, i == 0 ? h->w[enc] : nullptr, dst, h->w[dwid + 3],
-                                 h->w[dwid + 4], h->w[dwid], h->w[dwid + 2], rows, R1, sg.len[0], sg.len[1], st);
-        h->end(st);
-        ++h->launches;
-        if (rc != SEQPAN_OK) return fail(rc, "chain_enc_layer failed: %s", chain_last_error());
-        src = dst;
-      }
+                             sg.len[0], sg.nseg[1], sg.nseg[1] > 0 ? sg.len[1] : 0, st, tail, nl));
       return SEQPAN_OK;
     }
     for (int i = 0; i < nl; ++i) {
       const int dwid = enc + 1 + 5 * i;  // DWi, PWi_W, PWi_B, LNi_W, LNi_B
       LAUNCH(h, launch_ln_dwconv(i == 0 ? in : xout, i == 0 ? h->w[enc] : nullptr, i == 0 ? xout : nullptr,
                                  h->w[dwid + 3], h->w[dwid + 4], 1e-6f, h->w[dwid], ws.z, sg, st));
-      int rc = linear(ws.z, SQ_D, h->w[dwid + 1], h->w[dwid + 2], xout, xout, SQ_D, rows, SQ_D, SQ_D, true,
-                      tc_slot0 >= 0 ? tc_slot0 + i : -1);
+      int rc = linear(ws.z, SQ_D, h->w[dwid + 1], h->w[dwid + 2], xout, xout, SQ_D, rows, SQ_D, SQ_D, true);
       if (rc != SEQPAN_OK) return rc;
     }
     return SEQPAN_OK;
@@ -670,9 +619,8 @@ struct Fwd {
     const DabPacked& p = h->arena.dab[k];
     const float* const* w = h->w;
     const int ts = TC_DAB0 + k * TC_DAB_STRIDE;
-    const bool fused = tc && h->fuse;
     int rc;
-    const bool tc_att = fused && h->tc_attn && attn_dual_tc_supported(L, T);
+    const bool tc_att = tc && attn_dual_tc_supported(L, T);
     if (tc_att) {
       if (!proj_done)
         CHAIN(h, "chain_proj_ln", chain_proj_ln(h->arena.tc, ts + TC_DAB_QKV, ts + TC_DAB_TKV, cur, M, 1e-6f, w[W_DAB1_LN1_W + d],
@@ -680,22 +628,22 @@ struct Fwd {
                                                 (float*)ws.tc.qkv_bf16, p.qkv_b, (float*)ws.tc.tkv_bf16, p.tkv_b, st, nullptr, 0,
                                                 0, nullptr, true));
       CHAIN(h, "attn_dual_tc", attn_dual_tc(ws.tc.qkv_bf16, ws.tc.tkv_bf16, vmask, tmask, ws.tc.sa_bf16, ws.tc.xa_bf16, B, L, T, st));
-    } else if (fused) {
+    } else if (tc) {
       CHAIN(h, "chain_proj_ln", chain_proj_ln(h->arena.tc, ts + TC_DAB_QKV, ts + TC_DAB_TKV, cur, M, 1e-6f, w[W_DAB1_LN1_W + d],
                                               w[W_DAB1_LN1_B + d], w[W_DAB1_LNT_W + d], w[W_DAB1_LNT_B + d], ws.qkv, p.qkv_b,
                                               ws.tkv, p.tkv_b, st));
     } else {
       LAUNCH(h, launch_layernorm(cur, SQ_D, M, w[W_DAB1_LN1_W + d], w[W_DAB1_LN1_B + d], 1e-6f, ws.o, SQ_D,
                                  w[W_DAB1_LNT_W + d], w[W_DAB1_LNT_B + d], ws.u, SQ_D, nullptr, nullptr, 0, st));
-      if ((rc = linear(ws.o, SQ_D, p.qkv_w, p.qkv_b, nullptr, ws.qkv, 384, M, 384, SQ_D, false, ts + TC_DAB_QKV))) return rc;
-      if ((rc = linear(ws.u, SQ_D, p.tkv_w, p.tkv_b, nullptr, ws.tkv, 256, M, 256, SQ_D, false, ts + TC_DAB_TKV))) return rc;
+      if ((rc = linear(ws.o, SQ_D, p.qkv_w, p.qkv_b, nullptr, ws.qkv, 384, M, 384, SQ_D, false))) return rc;
+      if ((rc = linear(ws.u, SQ_D, p.tkv_w, p.tkv_b, nullptr, ws.tkv, 256, M, 256, SQ_D, false))) return rc;
     }
     if (!tc_att) {
-      DualAttnArgs aa{ws.qkv, ws.tkv, vmask, tmask, ws.sa, ws.xa, B, L, T, fused ? ws.tc.sa_bf16 : nullptr,
-                      fused ? ws.tc.xa_bf16 : nullptr};
+      DualAttnArgs aa{ws.qkv, ws.tkv, vmask, tmask, ws.sa, ws.xa, B, L, T, tc ? ws.tc.sa_bf16 : nullptr,
+                      tc ? ws.tc.xa_bf16 : nullptr};
       LAUNCH(h, launch_dual_attention(aa, st));
     }
-    if (fused) {
+    if (tc) {
       auto hv = [&](int id) { return h->hostw[id + d].data(); };
       // gate / bilinear biases with the folded projections' contributions (DabPacked::fold_b, mirrored at pack time)
       const float* fb = h->dab_fold_host[k];
@@ -710,65 +658,53 @@ struct Fwd {
       return SEQPAN_OK;
     }
     if ((rc = linear2(ws.sa, w[W_DAB1_SDENSE_W + d], w[W_DAB1_SDENSE_B + d], ws.s, ws.xa, w[W_DAB1_XDENSE_W + d],
-                      w[W_DAB1_XDENSE_B + d], ws.xx, M, ts + TC_DAB_SDENSE, ts + TC_DAB_XDENSE))) return rc;
+                      w[W_DAB1_XDENSE_B + d], ws.xx, M))) return rc;
     if ((rc = linear2(ws.s, w[W_DAB1_SGATE_W + d], w[W_DAB1_SGATE_B + d], ws.sg, ws.xx, w[W_DAB1_XGATE_W + d],
-                      w[W_DAB1_XGATE_B + d], ws.xg, M, ts + TC_DAB_SGATE, ts + TC_DAB_XGATE))) return rc;
+                      w[W_DAB1_XGATE_B + d], ws.xg, M))) return rc;
     LAUNCH(h, launch_gate_combine(ws.sg, ws.xx, ws.xg, ws.s, ws.zin, M * SQ_D / 4, st));
     // W1.o + W1.z = W1.(o + z): the guided_dense epilogue adds o, one 256-wide GEMM yields scores|values
-    if ((rc = linear(ws.zin, SQ_D, w[W_DAB1_GUIDED_W + d], w[W_DAB1_GUIDED_B + d], ws.o, ws.oz, SQ_D, M, SQ_D, SQ_D, false,
-                     ts + TC_DAB_GUIDED))) return rc;
-    if ((rc = linear(ws.oz, SQ_D, p.bil_w, p.bil_b, nullptr, ws.scva, 256, M, 256, SQ_D, false, ts + TC_DAB_BIL))) return rc;
+    if ((rc = linear(ws.zin, SQ_D, w[W_DAB1_GUIDED_W + d], w[W_DAB1_GUIDED_B + d], ws.o, ws.oz, SQ_D, M, SQ_D, SQ_D, false))) return rc;
+    if ((rc = linear(ws.oz, SQ_D, p.bil_w, p.bil_b, nullptr, ws.scva, 256, M, 256, SQ_D, false))) return rc;
     LAUNCH(h, launch_sigmoid_gate(ws.scva, ws.rowmask, ws.y, M, st));
-    if ((rc = linear(ws.y, SQ_D, w[W_DAB1_D1_W + d], w[W_DAB1_D1_B + d], cur, cur, SQ_D, M, SQ_D, SQ_D, false,
-                     ts + TC_DAB_D1))) return rc;
+    if ((rc = linear(ws.y, SQ_D, w[W_DAB1_D1_W + d], w[W_DAB1_D1_B + d], cur, cur, SQ_D, M, SQ_D, SQ_D, false))) return rc;
     if ((rc = ln(cur, M, W_DAB1_LN2_W + d, 1e-6f, ws.lnr))) return rc;
-    return linear(ws.lnr, SQ_D, w[W_DAB1_D2_W + d], w[W_DAB1_D2_B + d], cur, cur, SQ_D, M, SQ_D, SQ_D, false,
-                  ts + TC_DAB_D2);
+    return linear(ws.lnr, SQ_D, w[W_DAB1_D2_W + d], w[W_DAB1_D2_B + d], cur, cur, SQ_D, M, SQ_D, SQ_D, false);
   }
 
   // FeatureEncoderPredict (models/layers.py:626-639); result in `out`
-  // head != nullptr (fused path): the start/end logit head rides behind the FEP tail (chain_fep_head)
+  // bf16 mode: the start/end logit head `head` rides behind the FEP tail (chain_fep_head); fp32 / tf32 mode ignore it
   struct HeadArgs { int slot; int ln_w, ln_b, hid_b, dense_w, dense_b; float* logits; };
   int fep(const float* in, float* out, const HeadArgs* head = nullptr) {
     const float* const* w = h->w;
     Segs sg{{0, 0}, {B, 0}, {L, 0}};
     int rc;
     void* hb[3] = {ws.tc.hb_q, ws.tc.hb_k, ws.tc.hb_v};
-    const bool tc_batt = tc && h->fuse && B <= 256 && h->tc_attn;
+    const bool tc_batt = tc && B <= 256;   // in_proj rides behind the conv block as head-blocked q/k/v for attn_batch_tc
     ChainProjTail tl{};
     tl.slotA = TC_INPROJ; tl.slotB = -1; tl.eps = 1e-5f; tl.gA = w[W_PRED_LNA_W]; tl.bA = w[W_PRED_LNA_B];
     tl.biasA = w[W_INPROJ_B]; tl.hb = hb; tl.hbL = L; tl.hbB = B; tl.hb_mask = vmask;
-    bool proj_done = false;
-    if ((rc = conv_block(in, ws.ph, W_PRED_POS, sg, Mv, TC_PRED_PW0, tc_batt ? &tl : nullptr, &proj_done))) return rc;
-    if (tc && h->fuse) {
+    if ((rc = conv_block(in, ws.ph, W_PRED_POS, sg, Mv, TC_PRED_PW0, tc_batt ? &tl : nullptr))) return rc;
+    if (tc) {
       if (tc_batt) {
-        if (!proj_done)
-          CHAIN(h, "chain_proj_ln", chain_proj_ln(h->arena.tc, TC_INPROJ, -1, ws.ph, Mv, 1e-5f, w[W_PRED_LNA_W], w[W_PRED_LNA_B],
-                                                  nullptr, nullptr, ws.pqkv, w[W_INPROJ_B], nullptr, nullptr, st, hb, L, B, vmask));
         CHAIN(h, "attn_batch_tc", attn_batch_tc(ws.tc.hb_q, ws.tc.hb_k, ws.tc.hb_v, vmask, ws.tc.sa_bf16, B, L, st));
       } else {
         CHAIN(h, "chain_proj_ln", chain_proj_ln(h->arena.tc, TC_INPROJ, -1, ws.ph, Mv, 1e-5f, w[W_PRED_LNA_W], w[W_PRED_LNA_B],
                                                 nullptr, nullptr, ws.pqkv, w[W_INPROJ_B], nullptr, nullptr, st));
         LAUNCH(h, launch_batch_attention(ws.pqkv, vmask, nullptr, ws.tc.sa_bf16, B, L, st));
       }
-      if (head) {
-        auto hv = [&](int id) { return h->hostw[id].data(); };
-        const float* hostv[9] = {hv(W_OUTPROJ_B), hv(W_PRED_LNB_W), hv(W_PRED_LNB_B), hv(W_PRED_DENSE_B), hv(head->ln_w),
-                                 hv(head->ln_b), hv(head->hid_b), hv(head->dense_w), hv(head->dense_b)};
-        CHAIN(h, "chain_fep_head", chain_fep_head(h->arena.tc, head->slot, ws.tc.sa_bf16, ws.fuse2_bf16, ws.ph, out, Mv, hostv,
-                                                  head->logits, st));
-        return SEQPAN_OK;
-      }
-      CHAIN(h, "chain_fep_tail", chain_fep_tail(h->arena.tc, ws.tc.sa_bf16, ws.ph, out, Mv, w[W_OUTPROJ_B], w[W_PRED_LNB_W],
-                                                w[W_PRED_LNB_B], w[W_PRED_DENSE_B], st));
+      auto hv = [&](int id) { return h->hostw[id].data(); };
+      const float* hostv[9] = {hv(W_OUTPROJ_B), hv(W_PRED_LNB_W), hv(W_PRED_LNB_B), hv(W_PRED_DENSE_B), hv(head->ln_w),
+                               hv(head->ln_b), hv(head->hid_b), hv(head->dense_w), hv(head->dense_b)};
+      CHAIN(h, "chain_fep_head", chain_fep_head(h->arena.tc, head->slot, ws.tc.sa_bf16, ws.fuse2_bf16, ws.ph, out, Mv, hostv,
+                                                head->logits, st));
       return SEQPAN_OK;
     }
     if ((rc = ln(ws.ph, Mv, W_PRED_LNA_W, 1e-5f, ws.pa))) return rc;
-    if ((rc = linear(ws.pa, SQ_D, w[W_INPROJ_W], w[W_INPROJ_B], nullptr, ws.pqkv, 384, Mv, 384, SQ_D, false, TC_INPROJ))) return rc;
+    if ((rc = linear(ws.pa, SQ_D, w[W_INPROJ_W], w[W_INPROJ_B], nullptr, ws.pqkv, 384, Mv, 384, SQ_D, false))) return rc;
     LAUNCH(h, launch_batch_attention(ws.pqkv, vmask, ws.patt, nullptr, B, L, st));
-    if ((rc = linear(ws.patt, SQ_D, w[W_OUTPROJ_W], w[W_OUTPROJ_B], ws.ph, ws.ph, SQ_D, Mv, SQ_D, SQ_D, false, TC_OUTPROJ))) return rc;
+    if ((rc = linear(ws.patt, SQ_D, w[W_OUTPROJ_W], w[W_OUTPROJ_B], ws.ph, ws.ph, SQ_D, Mv, SQ_D, SQ_D, false))) return rc;
     if ((rc = ln(ws.ph, Mv, W_PRED_LNB_W, 1e-5f, ws.pa))) return rc;
-    return linear(ws.pa, SQ_D, w[W_PRED_DENSE_W], w[W_PRED_DENSE_B], ws.ph, out, SQ_D, Mv, SQ_D, SQ_D, false, TC_PRED_DENSE);
+    return linear(ws.pa, SQ_D, w[W_PRED_DENSE_W], w[W_PRED_DENSE_B], ws.ph, out, SQ_D, Mv, SQ_D, SQ_D, false);
   }
 
   const int64_t* word_ids; const int64_t* char_ids; const float* vfeat; const float* vmask; const float* tmask;
@@ -780,7 +716,7 @@ struct Fwd {
     const float* const* w = h->w;
     const SeqpanShapes& s = h->s;
     int rc;
-    if (!(tc && h->fuse))   // the fused DualAttentionBlock chain reads vmask / tmask in place
+    if (!tc)   // the fused DualAttentionBlock chain reads vmask / tmask in place
       LAUNCH(h, launch_build_rowmask(vmask, Mv, tmask, Mt, ws.rowmask, st));
     // text embedding (models/layers.py:87-93) -> rows [Mv, M) of x; on the side stream, concurrently with the video affine
     cudaStream_t main_st = st;
@@ -795,14 +731,14 @@ struct Fwd {
                                 h->arena.cbias, ws.et, st));
     float* xt = ws.x + Mv * SQ_D;
     float* zt = ws.z + Mv * SQ_D;
-    if ((tf32 || (tc && h->fuse)) && !sq_env().no_ln_fuse) {   // Conv1D(400 -> 128) on kind::tf32 straight from the fp32 concat + fused LayerNorm
+    if (tf32 || tc) {   // Conv1D(400 -> 128) on kind::tf32 straight from the fp32 concat + fused LayerNorm
       h->begin("tc_linear_tf32_query+ln", st);
       rc = tc_linear_tf32(ws.et, 400, w[W_QUERY_W], w[W_QUERY_B], nullptr, xt, SQ_D, Mt, SQ_D, 400, false, st, w[W_QLN_W], w[W_QLN_B], 1e-6f);
       h->end(st);
       if (rc != SEQPAN_OK) return fail(rc, "tc_linear_tf32 (query + LayerNorm) failed: %s", tc_last_error());
       ++h->launches;
     } else {
-      if ((rc = linear(ws.et, 400, w[W_QUERY_W], w[W_QUERY_B], nullptr, zt, SQ_D, Mt, SQ_D, 400, false, TC_QUERY))) return rc;
+      if ((rc = linear(ws.et, 400, w[W_QUERY_W], w[W_QUERY_B], nullptr, zt, SQ_D, Mt, SQ_D, 400, false))) return rc;
       if ((rc = ln(zt, Mt, W_QLN_W, 1e-6f, xt))) return rc;
     }
     if (fork) {
@@ -819,12 +755,11 @@ struct Fwd {
     Segs joint{{0, Mv}, {B, B}, {L, T}};
     // the first DualAttentionBlock's LN1 -> q|fk|fv and LNt -> tk|tv projections ride behind the encoder's last layer
     const bool has_dab = s.variant != SEQPAN_VARIANT_BASEFAST && s.variant != SEQPAN_VARIANT_STUDENT4;
-    const bool tc_att0 = has_dab && tc && h->fuse && h->tc_attn && attn_dual_tc_supported(L, T);
+    const bool tc_att0 = has_dab && tc && attn_dual_tc_supported(L, T);
     ChainProjTail dt{};
     dt.slotA = TC_DAB0 + TC_DAB_QKV; dt.slotB = TC_DAB0 + TC_DAB_TKV; dt.eps = 1e-6f;
     dt.gA = w[W_DAB1_LN1_W]; dt.bA = w[W_DAB1_LN1_B]; dt.gB = w[W_DAB1_LNT_W]; dt.bB = w[W_DAB1_LNT_B];
     dt.biasA = h->arena.dab[0].qkv_b; dt.biasB = h->arena.dab[0].tkv_b; dt.outA = ws.tc.qkv_bf16; dt.outB = ws.tc.tkv_bf16;
-    bool dab0_proj_done = false;
     if (s.variant == SEQPAN_VARIANT_BACKBONE) {
       // models/BackBone.py:48-49: vfeat_encoder on the video rows, the text's own tfeat_encoder on the text rows; the fused
       // LN + projection tail indexes its outputs by the rows of the call, so the text call gets offset output pointers
@@ -832,13 +767,12 @@ struct Fwd {
       ChainProjTail dtt = dt;
       dtt.outA = reinterpret_cast<char*>(dt.outA) + Mv * 384 * 2;
       dtt.outB = reinterpret_cast<char*>(dt.outB) + Mv * 256 * 2;
-      bool d0 = false, d1 = false;
-      if ((rc = conv_block(ws.x, ws.xb, W_ENC_POS, vs, Mv, TC_ENC_PW0, tc_att0 ? &dt : nullptr, &d0))) return rc;
-      if ((rc = conv_block(xt, ws.xb + Mv * SQ_D, W_TENC_POS, ts, Mt, TC_TENC_PW0, tc_att0 ? &dtt : nullptr, &d1))) return rc;
-      return run_after_encoder(d0 && d1);
+      if ((rc = conv_block(ws.x, ws.xb, W_ENC_POS, vs, Mv, TC_ENC_PW0, tc_att0 ? &dt : nullptr))) return rc;
+      if ((rc = conv_block(xt, ws.xb + Mv * SQ_D, W_TENC_POS, ts, Mt, TC_TENC_PW0, tc_att0 ? &dtt : nullptr))) return rc;
+      return run_after_encoder(tc_att0);
     }
-    if ((rc = conv_block(ws.x, ws.xb, W_ENC_POS, joint, M, TC_ENC_PW0, tc_att0 ? &dt : nullptr, &dab0_proj_done))) return rc;
-    return run_after_encoder(dab0_proj_done);
+    if ((rc = conv_block(ws.x, ws.xb, W_ENC_POS, joint, M, TC_ENC_PW0, tc_att0 ? &dt : nullptr))) return rc;
+    return run_after_encoder(tc_att0);
   }
 
   // Query-independent video branch once per UNIQUE clip (SURVEY.md section 8 (f1)): VisualProjection + the video half of the
@@ -878,7 +812,7 @@ struct Fwd {
       if ((rc = tap(4 + 2 * k, cur, SQ_D)) || (rc = tap(5 + 2 * k, cur + Mv * SQ_D, SQ_D))) return rc;
     }
     // CQAttention both ways + CQConcatenate (models/SeqPAN.py:73-75)
-    if (tc && h->fuse && h->tc_attn && cq_tc_supported(L, T)) {
+    if (tc && cq_tc_supported(L, T)) {
       const float* w4c[2] = {w[W_Q2V_W4C], w[W_V2Q_W4C]};
       const float* w4q[2] = {w[W_Q2V_W4Q], w[W_V2Q_W4Q]};
       const float* w4m[2] = {w[W_Q2V_W4MLU], w[W_V2Q_W4MLU]};
@@ -892,12 +826,11 @@ struct Fwd {
       CqArgs ca{cur, vmask, tmask, {w[W_Q2V_W4C], w[W_V2Q_W4C]}, {w[W_Q2V_W4Q], w[W_V2Q_W4Q]},
                 {w[W_Q2V_W4MLU], w[W_V2Q_W4MLU]}, {ws.catv, ws.catt}, B, L, T};
       LAUNCH(h, launch_cq_attention(ca, st));
-      if ((rc = linear(ws.catv, 512, w[W_Q2V_LIN_W], w[W_Q2V_LIN_B], nullptr, ws.cat2, 256, Mv, SQ_D, 512, false, TC_Q2V_LIN))) return rc;
-      if ((rc = linear(ws.catt, 512, w[W_V2Q_LIN_W], w[W_V2Q_LIN_B], nullptr, ws.v2t, SQ_D, Mt, SQ_D, 512, false, TC_V2Q_LIN))) return rc;
+      if ((rc = linear(ws.catv, 512, w[W_Q2V_LIN_W], w[W_Q2V_LIN_B], nullptr, ws.cat2, 256, Mv, SQ_D, 512, false))) return rc;
+      if ((rc = linear(ws.catt, 512, w[W_V2Q_LIN_W], w[W_V2Q_LIN_B], nullptr, ws.v2t, SQ_D, Mt, SQ_D, 512, false))) return rc;
     }
     if ((rc = tap(8, ws.cat2, 256)) || (rc = tap(9, ws.v2t, SQ_D))) return rc;
-    const bool tails = tc && h->fuse && h->fuse_tails;
-    if (tails) {
+    if (tc) {
       // CQConcatenate + match head in two launches: the pooled half of the concat is a per-sample bias
       CHAIN(h, "pool_bias", launch_pool_bias(ws.v2t, tmask, w[W_POOL_W], w[W_CAT_W], ws.pbias, B, T, st));
       const bool no_match = h->s.variant == SEQPAN_VARIANT_BACKBONE;
@@ -913,7 +846,7 @@ struct Fwd {
       return (rc = tap(12, ws.ps, SQ_D)) ? rc : tap(13, ws.pe, SQ_D);
     }
     LAUNCH(h, launch_pool_tile(ws.v2t, tmask, w[W_POOL_W], ws.cat2, B, L, T, st));
-    if ((rc = linear(ws.cat2, 256, w[W_CAT_W], w[W_CAT_B], nullptr, ws.fuse, SQ_D, Mv, SQ_D, 256, false, TC_CAT))) return rc;
+    if ((rc = linear(ws.cat2, 256, w[W_CAT_W], w[W_CAT_B], nullptr, ws.fuse, SQ_D, Mv, SQ_D, 256, false))) return rc;
     if ((rc = tap(10, ws.fuse, SQ_D))) return rc;
     // match head (models/SeqPAN.py:78-82); BackBone has none: the concat output feeds the predictor (models/BackBone.py:62-63)
     if (h->s.variant == SEQPAN_VARIANT_BACKBONE) {
@@ -927,18 +860,11 @@ struct Fwd {
     if ((rc = fep(ws.fuse2, ws.ps))) return rc;
     if ((rc = fep(ws.ps, ws.pe))) return rc;
     if ((rc = tap(12, ws.ps, SQ_D)) || (rc = tap(13, ws.pe, SQ_D))) return rc;
-    if (tc && h->fuse) {
-      CHAIN(h, "chain_head", chain_head(h->arena.tc, TC_START_HID, ws.ps, ws.fuse2, Mv, w[W_START_LN_W], w[W_START_LN_B],
-                                        w[W_START_HID_B], w[W_START_DENSE_W], w[W_START_DENSE_B], slogits, st));
-      CHAIN(h, "chain_head", chain_head(h->arena.tc, TC_END_HID, ws.pe, ws.fuse2, Mv, w[W_END_LN_W], w[W_END_LN_B],
-                                        w[W_END_HID_B], w[W_END_DENSE_W], w[W_END_DENSE_B], elogits, st));
-      return SEQPAN_OK;
-    }
     if ((rc = ln(ws.ps, Mv, W_START_LN_W, 1e-6f, ws.cat3, 256, ws.fuse2, ws.cat3 + SQ_D))) return rc;
-    if ((rc = linear(ws.cat3, 256, w[W_START_HID_W], w[W_START_HID_B], nullptr, ws.hid, SQ_D, Mv, SQ_D, 256, false, TC_START_HID))) return rc;
+    if ((rc = linear(ws.cat3, 256, w[W_START_HID_W], w[W_START_HID_B], nullptr, ws.hid, SQ_D, Mv, SQ_D, 256, false))) return rc;
     LAUNCH(h, launch_rowdot(ws.hid, SQ_D, w[W_START_DENSE_W], w[W_START_DENSE_B], slogits, Mv, st));
     if ((rc = ln(ws.pe, Mv, W_END_LN_W, 1e-6f, ws.cat3, 256, ws.fuse2, ws.cat3 + SQ_D))) return rc;
-    if ((rc = linear(ws.cat3, 256, w[W_END_HID_W], w[W_END_HID_B], nullptr, ws.hid, SQ_D, Mv, SQ_D, 256, false, TC_END_HID))) return rc;
+    if ((rc = linear(ws.cat3, 256, w[W_END_HID_W], w[W_END_HID_B], nullptr, ws.hid, SQ_D, Mv, SQ_D, 256, false))) return rc;
     LAUNCH(h, launch_rowdot(ws.hid, SQ_D, w[W_END_DENSE_W], w[W_END_DENSE_B], elogits, Mv, st));
     return SEQPAN_OK;
   }

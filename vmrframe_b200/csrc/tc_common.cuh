@@ -19,11 +19,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
-#ifdef SEQPAN_SPIN_WAIT
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#else
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#endif
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(ok)
       : "r"(bar), "r"(parity)
