@@ -220,6 +220,11 @@ typedef struct SeqpanGemm {       /* C[b0,b1] = alpha * A . B + beta * C;  X(i,j
 } SeqpanGemm;
 /* bias (may be NULL): a [N] vector added to every row of the product (the bias of a Conv1D / nn.Linear) */
 int seqpan_t_gemm(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* g, void* stream);
+/* The same product on the tensor cores (bf16 mixed precision): every element of A and B is rounded to bf16
+ * (round-to-nearest-even) before the product, products accumulate in fp32; C, bias, alpha and beta stay fp32.  Every other
+ * field of SeqpanGemm means what it means for seqpan_t_gemm, and the same bad arguments give the same errors.  Operands need
+ * no alignment; elements of C outside the (M, N, c_rs, c_cs) view are never touched. */
+int seqpan_t_gemm_bf16(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* g, void* stream);
 
 enum {   /* out = f(a, b, c) element-wise over a 4-D index space with per-operand strides (0 = broadcast) */
   SEQPAN_EW_COPY = 0,        /* a                                    */

@@ -82,6 +82,7 @@ SIGNATURES = {
     "seqpan_op_linear": (_i, [_vp] * 5 + [_i64, _i, _i, _i, _i, _vp, _sz, _vp]),
     "seqpan_op_layernorm": (_i, [_vp, _vp, _vp, C.c_float, _vp, _i64, _vp]),
     "seqpan_t_gemm": (_i, [_vp, _vp, _vp, _vp, C.POINTER(SeqpanGemm), _vp]),
+    "seqpan_t_gemm_bf16": (_i, [_vp, _vp, _vp, _vp, C.POINTER(SeqpanGemm), _vp]),
     "seqpan_t_ewise": (_i, [_vp, _vp, _vp, _vp, C.POINTER(SeqpanEwise), _vp]),
     "seqpan_t_softmax": (_i, [_vp, _vp, C.POINTER(SeqpanSoftmax), _vp]),
     "seqpan_t_softmax_bwd": (_i, [_vp, _vp, _vp, C.POINTER(SeqpanSoftmax), _vp]),

@@ -15,7 +15,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 OBJ = os.path.join(CSRC, os.environ.get("SEQPAN_OBJDIR", "_obj"))
 LIB = os.environ.get("SEQPAN_LIB") or os.path.join(PKG, "libseqpan_b200.so")
-SOURCES = ["kernels_f32.cu", "linear_tc.cu", "chain_tc.cu", "tail_tc.cu", "attn_tc.cu", "cq_tc.cu", "train_ops.cu", "seqpan_api.cu"]
+SOURCES = ["kernels_f32.cu", "linear_tc.cu", "chain_tc.cu", "tail_tc.cu", "attn_tc.cu", "cq_tc.cu", "train_ops.cu", "train_tc.cu", "seqpan_api.cu"]
 # diagnostics (tcgen05 descriptor probe) live in their own library: the product library exports no test entry points
 DIAG_SOURCES = ["umma_probe.cu"]
 DIAG_LIB = os.path.join(os.path.dirname(LIB), "libseqpan_diag.so")

@@ -7,6 +7,7 @@
 #include <cstdio>
 
 #include "common.cuh"
+#include "train_ops.cuh"
 
 namespace {
 
@@ -281,12 +282,6 @@ __global__ void __launch_bounds__(256) t_adamw_kernel(float* __restrict__ p, con
 }
 
 thread_local char g_terr[256] = "";
-int tfail(const char* msg) { snprintf(g_terr, sizeof(g_terr), "%s", msg); return SEQPAN_E_INVALID; }
-int tcheck() {
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) { snprintf(g_terr, sizeof(g_terr), "%s", cudaGetErrorString(e)); return SEQPAN_E_CUDA; }
-  return SEQPAN_OK;
-}
 unsigned grid_for(long long n, int per_block, long long cap = 148 * 16) {
   long long b = (n + per_block - 1) / per_block;
   return (unsigned)(b < 1 ? 1 : (b > cap ? cap : b));
@@ -294,15 +289,20 @@ unsigned grid_for(long long n, int per_block, long long cap = 148 * 16) {
 
 }  // namespace
 
-extern "C" const char* seqpan_t_last_error(void) { return g_terr; }
+int tfail(const char* msg) { snprintf(g_terr, sizeof(g_terr), "%s", msg); return SEQPAN_E_INVALID; }
+int tcheck() {
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) { snprintf(g_terr, sizeof(g_terr), "%s", cudaGetErrorString(e)); return SEQPAN_E_CUDA; }
+  return SEQPAN_OK;
+}
 
-extern "C" int seqpan_t_gemm(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, void* stream) {
+int t_gemm_prepare(const float* A, const float* B, float* C, const SeqpanGemm* gp, cudaStream_t st, int& split, long long& gz) {
+  gz = 0;
   if (!A || !B || !C || !gp) return tfail("gemm: NULL argument");
-  SeqpanGemm g = *gp;
+  const SeqpanGemm& g = *gp;
   if (g.M < 0 || g.N < 0 || g.K < 0 || g.batch0 < 1 || g.batch1 < 1) return tfail("gemm: bad sizes");
   if (g.M == 0 || g.N == 0) return SEQPAN_OK;
-  cudaStream_t st = (cudaStream_t)stream;
-  int split = g.splitk > 1 ? g.splitk : 1;
+  split = g.splitk > 1 ? g.splitk : 1;
   if (split > 1) {
     if (g.beta != 0.f && g.beta != 1.f) return tfail("gemm: split-K needs beta 0 or 1");
     if (g.batch0 * g.batch1 != 1 || g.c_cs != 1) return tfail("gemm: split-K needs one batch and a row-major C");
@@ -310,8 +310,21 @@ extern "C" int seqpan_t_gemm(const float* A, const float* B, float* C, const flo
       if (cudaMemset2DAsync(C, (size_t)g.c_rs * sizeof(float), 0, (size_t)g.N * sizeof(float), (size_t)g.M, st) != cudaSuccess) return tcheck();
     }
   }
-  const long long gz = (long long)g.batch0 * g.batch1 * split;
-  if (gz > 65535) return tfail("gemm: too many batches");
+  const long long z = (long long)g.batch0 * g.batch1 * split;
+  if (z > 65535) return tfail("gemm: too many batches");
+  gz = z;
+  return SEQPAN_OK;
+}
+
+extern "C" const char* seqpan_t_last_error(void) { return g_terr; }
+
+extern "C" int seqpan_t_gemm(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  int split = 1;
+  long long gz = 0;
+  const int rc = t_gemm_prepare(A, B, C, gp, st, split, gz);
+  if (rc != SEQPAN_OK || gz == 0) return rc;
+  const SeqpanGemm g = *gp;
   dim3 grid((unsigned)((g.N + GT - 1) / GT), (unsigned)((g.M + GT - 1) / GT), (unsigned)gz);
   t_gemm_kernel<<<grid, 256, 0, st>>>(A, B, C, bias, g);
   return tcheck();

@@ -19,7 +19,9 @@ tape and the adjoint rules against the oracle's autograd without a GPU; the prod
 
 The forward here is the reference's training forward restated primitive by primitive (same dropout sites, same order:
 models/layers.py:48,67,119,146,284,291,294,296,352,357,431-432,570,631-638).  It deliberately does not reuse the fused
-tcgen05 inference kernels yet: those keep no activations.  fp32 throughout.
+tcgen05 inference kernels yet: those keep no activations.  fp32 by default; ``precision="bf16"`` (``TrainStep`` /
+``configs.model.train_precision``) runs the model's matrix products on the tensor cores (csrc/train_tc.cu) with bf16 operands
+and fp32 accumulation, and keeps everything else fp32.
 """
 from __future__ import annotations
 
@@ -32,6 +34,22 @@ from . import _cabi
 
 D, H, HD = 128, 4, 32
 MASKV = -1e30
+PRECISIONS = ("fp32", "bf16")      # training precision modes (see SeqpanTape)
+
+
+def _check_precision(precision):
+    if precision not in PRECISIONS:
+        raise ValueError(f"training precision {precision!r}: expected one of {PRECISIONS}")
+    return precision
+
+
+def train_precision(model, precision=None):
+    """The training precision of ``model``: ``precision`` when given, else ``configs.model.train_precision`` (so the reference's
+    own loop opts in from its YAML), else ``"fp32"``.  The module's inference ``precision=`` is a different setting and is not
+    consulted."""
+    if precision is None:
+        precision = getattr(model.configs.model, "train_precision", "fp32")
+    return _check_precision(precision)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -93,7 +111,9 @@ class CudaBackend:
         return -torch.empty(tuple(shape), dtype=torch.float32, device=self.device).exponential_().log()
 
     # -- C[..., M, N] = alpha * A[..., M, K] @ B[..., K, N] + beta * C --
-    def gemm(self, A, B, out=None, alpha=1.0, beta=0.0, splitk=1, bias=None):
+    def gemm(self, A, B, out=None, alpha=1.0, beta=0.0, splitk=1, bias=None, mixed=False):
+        """``mixed=True``: bf16 operands (rounded to nearest even), fp32 accumulation, on the tensor cores
+        (``seqpan_t_gemm_bf16``); otherwise the fp32 kernel."""
         self._req(A, B, out, bias)
         nb = A.dim() - 2
         assert B.dim() == A.dim() and 0 <= nb <= 2 and A.shape[-1] == B.shape[-2] and A.shape[:nb] == B.shape[:nb]
@@ -110,8 +130,8 @@ class CudaBackend:
         sa, sb, sc = (_pad4(t.stride()[:nb], 0)[2:] for t in (A, B, out))
         g.a_b0, g.a_b1, g.b_b0, g.b_b1, g.c_b0, g.c_b1 = sa[0], sa[1], sb[0], sb[1], sc[0], sc[1]
         g.alpha, g.beta, g.splitk = alpha, beta, splitk if nb == 0 and out.stride(-1) == 1 else 1
-        self._chk(self.L.seqpan_t_gemm(A.data_ptr(), B.data_ptr(), out.data_ptr(), bias.data_ptr() if bias is not None else None,
-                                       C.byref(g), self._st()))
+        fn = self.L.seqpan_t_gemm_bf16 if mixed else self.L.seqpan_t_gemm
+        self._chk(fn(A.data_ptr(), B.data_ptr(), out.data_ptr(), bias.data_ptr() if bias is not None else None, C.byref(g), self._st()))
         return out
 
     # -- element-wise with broadcasting over <= 4 dims --
@@ -244,13 +264,19 @@ class Var:
 
 
 class SeqpanTape:
-    """Records the training forward of SeqPAN; ``backward`` replays the adjoint rules in reverse order."""
+    """Records the training forward of SeqPAN; ``backward`` replays the adjoint rules in reverse order.
 
-    def __init__(self, backend, droprate=0.0, training=True, mask_fn=None):
+    ``precision="bf16"``: the model's matrix products (``linear`` y / dx / dW, the forward ``bmm``, the six products of
+    ``attention``, the char-CNN window products) and their adjoints run with bf16 operands and fp32 accumulation; ones-vector
+    reductions, bias gradients, the loss functions, LayerNorm, softmax, element-wise ops and the optimizer stay fp32 -- the
+    autocast policy.  ``"fp32"`` calls ``backend.gemm`` exactly as before the mode existed (no ``mixed`` keyword)."""
+
+    def __init__(self, backend, droprate=0.0, training=True, mask_fn=None, precision="fp32"):
         self.be = backend
         self.p = float(droprate) if training else 0.0
         self.mask_fn = mask_fn          # optional: (shape) -> keep-mask tensor of 0/1 (parity tests inject the oracle's draws)
         self.nodes = []
+        self.mm = {"mixed": True} if _check_precision(precision) == "bf16" else {}    # keywords of a model product's be.gemm
 
     # -- bookkeeping --
     def leaf(self, t, needs=False):
@@ -293,13 +319,13 @@ class SeqpanTape:
         K, N = x.v.shape[-1], W.v.shape[0]
         x2, W2 = x.v.reshape(-1, K), W.v.reshape(N, K)
         M = x2.shape[0]
-        y = be.gemm(x2, W2.t(), bias=b.v.reshape(N) if b is not None else None)
+        y = be.gemm(x2, W2.t(), bias=b.v.reshape(N) if b is not None else None, **self.mm)
         sk = 1 if M < 1024 else min(64, max(1, M // 128))     # K-splits of the two long reductions (dW, db): fill the 148 SMs
 
         def bwd(g):
             g2 = g.reshape(M, N)
-            dx = be.gemm(g2, W2).reshape(x.v.shape) if x.needs else None
-            dW = be.gemm(g2.t(), x2, splitk=sk).reshape(W.v.shape) if W.needs else None
+            dx = be.gemm(g2, W2, **self.mm).reshape(x.v.shape) if x.needs else None
+            dW = be.gemm(g2.t(), x2, splitk=sk, **self.mm).reshape(W.v.shape) if W.needs else None
             db = be.gemm(be.ones(M).reshape(1, M), g2, splitk=sk).reshape(b.v.shape) if (b is not None and b.needs) else None
             return (dx, dW, db) if b is not None else (dx, dW)
         return self._rec(y.reshape(tuple(x.v.shape[:-1]) + (N,)), [x, W] + ([b] if b is not None else []), bwd)
@@ -397,23 +423,25 @@ class SeqpanTape:
         y = be.softmax(ac, dim)
         return self._rec(y, [a], lambda g: (be.softmax_bwd(y, g, dim),))
 
-    def bmm(self, a, b, ta=False, tb=False):
+    def bmm(self, a, b, ta=False, tb=False, keep_fp32=False):
         """Batched a @ b over <= 2 leading dims; ta / tb transpose the last two dims of an operand (a stride swap).  A ``b``
-        with batch size 1 (a weight shared by the batch: w4C, w4Q, the pool weight) is broadcast; its gradient is the batch sum."""
+        with batch size 1 (a weight shared by the batch: w4C, w4Q, the pool weight) is broadcast; its gradient is the batch sum.
+        ``keep_fp32``: a product of the loss functions, fp32 in every precision mode."""
         be = self.be
+        mm = {} if keep_fp32 else self.mm
         if b.v.dim() == 3 and a.v.dim() == 3 and b.v.shape[0] == 1 and a.v.shape[0] != 1:
             b0 = b
             b = self._rec(b0.v.expand(a.v.shape[0], *b0.v.shape[1:]), [b0], lambda g: (self._sum_to(g, b0.v.shape),))
         A = a.v.transpose(-1, -2) if ta else a.v
         B = b.v.transpose(-1, -2) if tb else b.v
-        y = be.gemm(A, B)
+        y = be.gemm(A, B, **mm)
 
         def bwd(g):
             da = db = None
             if a.needs:
-                da = be.gemm(B, g.transpose(-1, -2)) if ta else be.gemm(g, B.transpose(-1, -2))
+                da = be.gemm(B, g.transpose(-1, -2), **mm) if ta else be.gemm(g, B.transpose(-1, -2), **mm)
             if b.needs:
-                db = be.gemm(g.transpose(-1, -2), A) if tb else be.gemm(A.transpose(-1, -2), g)
+                db = be.gemm(g.transpose(-1, -2), A, **mm) if tb else be.gemm(A.transpose(-1, -2), g, **mm)
             return da, db
         return self._rec(y, [a, b], bwd)
 
@@ -532,7 +560,7 @@ class SeqpanTape:
         Dropout acts on the attention probabilities (models/layers.py:352,357; nn.MultiheadAttention's own dropout)."""
         be = self.be
         qh, kh, vh = q_heads(q.v), k_heads(k.v), k_heads(v.v)
-        s = be.gemm(qh, kh.transpose(-1, -2), alpha=scale)
+        s = be.gemm(qh, kh.transpose(-1, -2), alpha=scale, **self.mm)
         s = be.ewise("AXPBY", s, add_mask, out=s, alpha=1.0, beta=1.0)
         p = be.softmax(s, -1)
         pd, r, thr, dsc = p, None, 0.5, 1.0
@@ -543,13 +571,13 @@ class SeqpanTape:
                 r, thr, dsc = be.dropout_mask(p.shape, self.p), 0.5, 1.0
             pd = be.ewise("DROPOUT", p, r, alpha=thr, beta=dsc) if self.mask_fn is not None else be.ewise("MUL", p, r)
         out = be.empty(out_shape)
-        be.gemm(pd, vh, out=out_heads(out))
+        be.gemm(pd, vh, out=out_heads(out), **self.mm)
 
         def bwd(g):
             gh = out_heads(g if g.is_contiguous() else be.ewise("COPY", g))
             dv = torch.zeros_like(v.v)
-            be.gemm(pd.transpose(-1, -2), gh, out=k_heads(dv))
-            dpd = be.gemm(gh, vh.transpose(-1, -2))
+            be.gemm(pd.transpose(-1, -2), gh, out=k_heads(dv), **self.mm)
+            dpd = be.gemm(gh, vh.transpose(-1, -2), **self.mm)
             if r is None:
                 dp = dpd
             elif self.mask_fn is not None:
@@ -558,8 +586,8 @@ class SeqpanTape:
                 dp = be.ewise("MUL", dpd, r)
             ds = be.softmax_bwd(p, dp, -1)
             dq, dk = torch.zeros_like(q.v), torch.zeros_like(k.v)
-            be.gemm(ds, kh, out=q_heads(dq), alpha=scale)
-            be.gemm(ds.transpose(-1, -2), qh, out=k_heads(dk), alpha=scale)
+            be.gemm(ds, kh, out=q_heads(dq), alpha=scale, **self.mm)
+            be.gemm(ds.transpose(-1, -2), qh, out=k_heads(dk), alpha=scale, **self.mm)
             return dq, dk, dv
         return self._rec(out, [q, k, v], bwd)
 
@@ -623,7 +651,7 @@ def _text_embedding(tp, P, word_ids, char_ids):
         win = ce_c.as_strided((Rk, k * 100), (100, 1), ce_c.storage_offset())
         Wp2 = be.ewise("COPY", Wk.v.reshape(ch, 100, k).permute(0, 2, 1)).reshape(ch, k * 100)       # (o, j, i) order
         yfull = be.zeros((R, ch))
-        be.gemm(win, Wp2.t(), out=yfull[:Rk])
+        be.gemm(win, Wp2.t(), out=yfull[:Rk], **tp.mm)
         y = be.ewise("AXPBY", yfull.reshape(B * T, Cc, ch)[:, :npos, :], bk.v.reshape(1, 1, ch), alpha=1.0, beta=1.0)   # [B*T, npos, ch]
 
         def bwd(g, win=win, Wp2=Wp2, Wk=Wk, k=k, ch=ch, npos=npos, Rk=Rk):
@@ -632,11 +660,11 @@ def _text_embedding(tp, P, word_ids, char_ids):
             g2 = gfull.reshape(R, ch)
             dce = None
             if ce.needs:
-                dwin = be.gemm(g2[:Rk], Wp2)                                                        # [Rk, k*100]
+                dwin = be.gemm(g2[:Rk], Wp2, **tp.mm)                                               # [Rk, k*100]
                 dce = be.zeros((R, 100))
                 for j in range(k):                       # overlapping windows add up: k shifted accumulations
                     be.ewise("AXPBY", dce[j:j + Rk], dwin[:, j * 100:(j + 1) * 100], out=dce[j:j + Rk], alpha=1.0, beta=1.0)
-            dWp = be.gemm(g2[:Rk].t(), win, splitk=min(64, max(1, Rk // 128)))                      # [ch, k*100]
+            dWp = be.gemm(g2[:Rk].t(), win, splitk=min(64, max(1, Rk // 128)), **tp.mm)             # [ch, k*100]
             dW = be.ewise("COPY", dWp.reshape(ch, k, 100).permute(0, 2, 1)).reshape(Wk.v.shape)
             db = be.gemm(be.ones(R).reshape(1, R), g2, splitk=min(64, max(1, R // 128))).reshape(ch)
             return dce, dW, db
@@ -874,7 +902,7 @@ def loss_match(tp, match_score, label_embs, ner_labels, vmask):
     denom = be.ewise("AFFINE", be.gemm(be.ones(n).reshape(1, n), vmask.reshape(n, 1)), alpha=1.0, beta=1e-12).reshape(())
     per = tp.scale(tp.div(tp.sum_all(tp.mul_const(match_score, w)), tp.leaf(denom)), -1.0)
     E = label_embs
-    G = tp.bmm(tp.reshape(E, (1, D, 4)), tp.reshape(E, (1, D, 4)), ta=True)           # [1,4,4] = E^T E
+    G = tp.bmm(tp.reshape(E, (1, D, 4)), tp.reshape(E, (1, D, 4)), ta=True, keep_fp32=True)   # [1,4,4] = E^T E
     off = tp.mul_const(G, (1.0 - torch.eye(4, device=vmask.device)).reshape(1, 4, 4))
     return tp.add(per, tp.norm2(off))
 
@@ -882,7 +910,7 @@ def loss_match(tp, match_score, label_embs, ner_labels, vmask):
 def _soft_dist(tp, x, temperature):
     """``softmax(F.normalize(x, p=2, dim=1) / temperature, dim=-1)`` of a ``[B,L]`` Var (models/loss.py:187-190)."""
     B, L = x.v.shape
-    n = tp.sqrt(tp.bmm(tp.reshape(tp.mul(x, x), (1, B, L)), tp.leaf(tp.be.ones(L).reshape(1, L, 1))))   # row norms [1,B,1]
+    n = tp.sqrt(tp.bmm(tp.reshape(tp.mul(x, x), (1, B, L)), tp.leaf(tp.be.ones(L).reshape(1, L, 1)), keep_fp32=True))   # row norms [1,B,1]
     n = tp.scale(tp.relu(tp.scale(n, 1.0, -1e-12)), 1.0, 1e-12)                                          # F.normalize: clamp_min(eps)
     return tp.softmax(tp.scale(tp.div(x, tp.reshape(n, (B, 1))), 1.0 / temperature), 1)
 
@@ -956,8 +984,9 @@ class TrainStep:
     world size before clipping (data parallel, one batch of ``B`` pairs per rank)."""
 
     def __init__(self, model, lr=1e-4, warmup_proportion=0.0, num_train_steps=1, weight_decay=0.01, clip_norm=1.0, backend=None,
-                 mask_fn=None):
+                 mask_fn=None, precision=None):
         self.model = model
+        self.precision = train_precision(model, precision)      # "fp32" or "bf16" (mixed: bf16 products, fp32 everything else)
         self.named = {k: p for k, p in model.named_parameters()}
         dev = next(model.parameters()).device
         self.be = backend if backend is not None else CudaBackend(dev)
@@ -989,7 +1018,7 @@ class TrainStep:
         """Forward + both losses + backward.  Returns ``(loss tensor (device scalar), {name: grad}, outputs)``."""
         be = self.be
         m = self.model
-        tp = SeqpanTape(be, droprate=m.configs.model.droprate, training=m.training, mask_fn=self.mask_fn)
+        tp = SeqpanTape(be, droprate=m.configs.model.droprate, training=m.training, mask_fn=self.mask_fn, precision=self.precision)
         P = _Params(tp, self.named)
         vmask, tmask = data["vmasks"].to(torch.float32), data["tmasks"].to(torch.float32)
         spec = train_spec(m)
@@ -1157,7 +1186,7 @@ def forward_only(model, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel=None)
     """``SeqPAN.forward`` in TRAINING mode (dropout active) without recording a tape: what ``model(...)`` returns when the
     module is in ``train()``; gradients come from :func:`tape_loss` / :class:`TrainStep`."""
     be = CudaBackend(vfeat_in.device)
-    tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=True)
+    tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=True, precision=train_precision(model))
     P = _Params(tp, {k: p.detach() for k, p in model.named_parameters()})
     for v in P.vars.values():
         v.needs = False
