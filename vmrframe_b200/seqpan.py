@@ -446,12 +446,20 @@ class SeqPAN(nn.Module):
         ``video_index`` (keyword-only, optional; SURVEY.md section 8 row f1): ``vfeat_in`` then holds every clip ONCE,
         ``[U,vlen,vdim]``, and ``video_index[b]`` names the clip of pair ``b``.  The query-independent video branch
         (VisualProjection + the video half of the shared encoder, models/SeqPAN.py:57,59) runs once per clip; the
-        outputs equal the plain call on ``vfeat_in[video_index]``."""
+        outputs equal the plain call on ``vfeat_in[video_index]``.
+
+        In ``train()`` mode (no ``video_index``) the forward runs with dropout on the training kernels.  When grad mode is on
+        and some parameter or ``vfeat_in`` requires grad, the outputs carry an autograd graph: ``loss.backward()`` of any torch
+        loss on them fills ``p.grad`` (and ``vfeat_in.grad``) through the training kernels' backward, once per forward (no
+        double backward, no ``retain_graph``).  ``eval()`` mode never records one."""
         _cabi.require_device()
         if self.training:
             # training mode (dropout active, models/layers.py nn.Dropout sites): the primitive-by-primitive forward of
-            # vmrframe_b200/train.py.  The returned tensors carry no autograd graph: gradients come from
-            # train_engine_SeqPAN / vmrframe_b200.train.TrainStep, which run forward AND backward on the kernels.
+            # vmrframe_b200/train.py.  With grad mode on and a parameter (or vfeat_in) that requires grad, the outputs are
+            # attached to the autograd graph through one node whose backward runs the tape's adjoints on the training
+            # kernels, so any torch loss on them backpropagates; otherwise (no_grad, inference_mode, all frozen) no tape is
+            # recorded.  Both routes compute bit-identical values.  train_engine_SeqPAN / TrainStep run forward, the
+            # reference's losses and backward in one call instead.
             if self._VARIANT not in (_cabi.VARIANT_SEQPAN, _cabi.VARIANT_BASEFAST, _cabi.VARIANT_MULTITEACHER,
                                      _cabi.VARIANT_BACKBONE) or video_index is not None:
                 raise NotImplementedError("the training forward exists for SeqPAN, BaseFast, MultiTeacher and BackBone (no video_index)")
@@ -460,9 +468,11 @@ class SeqPAN(nn.Module):
             if self.sync_timing:
                 torch.cuda.synchronize()
             start = time.time()
+            graph = torch.is_grad_enabled() and (vfeat_in.requires_grad or any(p.requires_grad for p in self.parameters()))
+            fwd = _train.forward_differentiable if graph else _train.forward_only
             with torch.cuda.device(device):
-                sl, el, ms = _train.forward_only(self, word_ids.to(torch.int64).contiguous(), char_ids.to(torch.int64).contiguous(),
-                                                 vfeat_in.contiguous(), vmask, tmask, gumbel)
+                sl, el, ms = fwd(self, word_ids.to(torch.int64).contiguous(), char_ids.to(torch.int64).contiguous(),
+                                 vfeat_in.contiguous(), vmask, tmask, gumbel)
             consume_time = 0.0
             if self.sync_timing:
                 torch.cuda.synchronize()

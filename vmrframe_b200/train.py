@@ -301,8 +301,11 @@ class SeqpanTape:
         else:
             self.be.ewise("AXPBY", var.g, g, out=var.g, alpha=1.0, beta=1.0)
 
-    def backward(self, out, gout):
-        self._acc(out, gout)
+    def backward(self, out, gout=None):
+        """Reverse sweep from ``out`` with cotangent ``gout``, or from several outputs at once: ``out`` a list of
+        ``(Var, cotangent)`` pairs, where a pair whose cotangent is None contributes nothing.  Cotangents are only read."""
+        for o, g in ([(out, gout)] if isinstance(out, Var) else out):
+            self._acc(o, g)
         for o, inputs, bwd in reversed(self.nodes):
             if o.g is None:
                 continue
@@ -825,13 +828,14 @@ def _predictor(tp, P, x, vmask):
 def forward_train(tp, P, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel, dual_blocks=True, text_encoder="vfeat_encoder",
                   match_head=True):
     """``SeqPAN.forward`` in training mode (models/SeqPAN.py:50-95) on the tape; returns Vars
-    ``(slogits [B,L], elogits [B,L], match_score [B,L,4])``.  ``dual_blocks=False``: ``BaseFast.forward`` (models/BaseFast.py:49-97:
-    the two DualAttentionBlock passes are commented out there; its 2-layer encoder is read off the parameters -- so is
-    MultiTeacher's, models/MultiTeacher.py:26).  ``text_encoder="tfeat_encoder"``, ``match_head=False``: ``BackBone.forward``
+    ``(slogits [B,L], elogits [B,L], match_score [B,L,4])``.  ``vfeat_in`` is a tensor (a constant of the tape) or a leaf Var
+    (``tp.leaf(v, needs=True)``: its ``.g`` holds the gradient of the video features after ``backward``).
+    ``dual_blocks=False``: ``BaseFast.forward`` (models/BaseFast.py:49-97: the two DualAttentionBlock passes are commented out
+    there; its 2-layer encoder is read off the parameters -- so is MultiTeacher's, models/MultiTeacher.py:26).  ``text_encoder="tfeat_encoder"``, ``match_head=False``: ``BackBone.forward``
     (models/BackBone.py:40-75: the text has its own FeatureEncoder, the CQConcatenate output feeds the predictor directly and
     unmasked; ``match_score`` is None)."""
     t = _text_embedding(tp, P, word_ids, char_ids)                                   # :56
-    v = tp.dropout(tp.leaf(vfeat_in))                                                # VisualProjection.drop (:119)
+    v = tp.dropout(vfeat_in if isinstance(vfeat_in, Var) else tp.leaf(vfeat_in))      # VisualProjection.drop (:119)
     v = _ln(tp, P, "video_affine.v_layer_norm", _conv1d(tp, P, "video_affine.video_conv1d", v), 1e-6)   # :57
     v = _feature_encoder(tp, P, "vfeat_encoder", v)                                  # :59
     t = _feature_encoder(tp, P, text_encoder, t)                                     # :60 (shared weights; BackBone.py:49: its own)
@@ -1182,9 +1186,92 @@ def tape_loss(model, data, gumbel=None, mask_fn=None, runtype="train"):
     return _TapeLoss.apply(value, glist, *params), out
 
 
+# ---- the training forward as one torch autograd node: any torch loss on its outputs backpropagates through the tape ----------
+_EMB_PAD_ROW = ("text_encoder.char_emb.char_emb.weight", "text_encoder.word_emb.word_emb.weight")
+
+
+class _Recording:
+    """What the node's backward needs: the tape, its output Vars, the video leaf and the parameter Vars.  The tape's nodes are
+    closures over the tape (a reference cycle); clearing them when the recording dies lets reference counting free a forward
+    that is never backpropagated as soon as its outputs are dropped, as it frees :func:`forward_only`'s."""
+    __slots__ = ("tp", "outs", "xv", "P")
+
+    def __init__(self, tp, outs, xv, P):
+        self.tp, self.outs, self.xv, self.P = tp, outs, xv, P
+
+    def __del__(self):
+        self.tp.nodes = []
+
+
+class _TapeForward(torch.autograd.Function):
+    """Forward: the training forward recorded on a ``SeqpanTape`` (kept on ``ctx``).  Backward: the tape's adjoints from the
+    cotangents of ``slogits`` / ``elogits`` / ``match_score`` that autograd hands in, one gradient per parameter and for
+    ``vfeat_in``.  Once-differentiable, and the tape frees its nodes as it runs: a second backward raises.
+
+    The outputs are fresh views of the tape's tensors, never the tensors the tape (and so ``ctx``) holds: a returned tensor
+    reachable from ``ctx`` would close the cycle output -> grad_fn -> ctx -> output, and a forward dropped without a backward
+    would keep its whole tape alive until a full garbage collection."""
+
+    @staticmethod
+    def forward(ctx, model, be, word_ids, char_ids, vmask, tmask, gumbel, vfeat_in, names, *params):
+        ctx.set_materialize_grads(False)          # an output nobody used arrives as None and costs nothing
+        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model))
+        P = _Params(tp, dict(zip(names, params)))
+        xv = tp.leaf(vfeat_in, needs=ctx.needs_input_grad[7])
+        outs = [o for o in forward_train(tp, P, word_ids, char_ids, xv, vmask, tmask, gumbel, **train_spec(model)["fwd"])
+                if o is not None]
+        ctx.rec, ctx.names, ctx.shapes = _Recording(tp, outs, xv, P), names, [p.shape for p in params]
+        return tuple(o.v.view_as(o.v) for o in outs)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, *gouts):
+        rec = ctx.rec
+        if rec is None:
+            raise RuntimeError("backward through the SeqPAN training forward a second time: the tape is freed by the first "
+                               "backward (retain_graph is not supported); run the forward again")
+        ctx.rec = None
+        be = rec.tp.be
+        gouts = [g if g is None or g.is_contiguous() else be.ewise("COPY", g) for g in gouts]   # e.g. .sum()'s expanded views
+        rec.tp.backward(list(zip(rec.outs, gouts)))
+        grads = [rec.xv.g] + [rec.P[k].g for k in ctx.names]
+        for k in _EMB_PAD_ROW:                     # nn.Embedding(padding_idx=0): row 0 gets no gradient
+            if k in rec.P.vars and rec.P[k].g is not None:
+                rec.P[k].g[0].zero_()
+        # Every returned gradient must be a tensor of its own: AccumulateGrad may adopt it as p.grad and later add into it in
+        # place.  The tape lets siblings share one gradient tensor (a + b) and passes cotangents through untouched, so a
+        # gradient whose storage is already taken by a cotangent or an earlier gradient is copied.
+        taken = {g.untyped_storage().data_ptr() for g in gouts if g is not None}
+        res = []
+        for g, shape in zip(grads, [rec.xv.v.shape] + ctx.shapes):
+            if g is not None:
+                key = g.untyped_storage().data_ptr()
+                if key in taken:
+                    g = be.ewise("COPY", g)
+                taken.add(g.untyped_storage().data_ptr())
+                g = g.reshape(shape)
+            res.append(g)
+        return (None,) * 7 + tuple(res[:1]) + (None,) + tuple(res[1:])
+
+
+def forward_differentiable(model, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel=None, backend=None):
+    """``SeqPAN.forward`` in training mode on the tape, as one torch autograd node: returns ``(slogits, elogits, match_score or
+    None)`` attached to every parameter that requires grad and to ``vfeat_in`` when it does, so that ``loss.backward()`` of any
+    torch loss on them fills ``p.grad`` / ``vfeat_in.grad`` through the training kernels.  The same kernels, in the same order,
+    with the same dropout and Gumbel draws as :func:`forward_only`: the values are bit-identical.  ``backend`` defaults to the
+    CUDA kernels of ``vfeat_in``'s device."""
+    be = backend if backend is not None else CudaBackend(vfeat_in.device)
+    names, params = zip(*model.named_parameters())
+    outs = _TapeForward.apply(model, be, word_ids, char_ids, vmask.to(torch.float32), tmask.to(torch.float32), gumbel,
+                              vfeat_in.to(torch.float32), names, *params)
+    return outs if len(outs) == 3 else (outs[0], outs[1], None)
+
+
 def forward_only(model, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel=None):
     """``SeqPAN.forward`` in TRAINING mode (dropout active) without recording a tape: what ``model(...)`` returns when the
-    module is in ``train()``; gradients come from :func:`tape_loss` / :class:`TrainStep`."""
+    module is in ``train()`` and no gradient is wanted (``torch.no_grad()`` / ``inference_mode()``, or nothing requires grad).
+    :func:`forward_differentiable` is the same forward with a graph; :func:`tape_loss` / :class:`TrainStep` run forward, the
+    reference's losses and backward in one call."""
     be = CudaBackend(vfeat_in.device)
     tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=True, precision=train_precision(model))
     P = _Params(tp, {k: p.detach() for k, p in model.named_parameters()})
