@@ -284,6 +284,39 @@ int seqpan_t_adamw(float* p, const float* g, float* m, float* v, int64_t n, cons
                    const float* dyn, void* stream);
 const char* seqpan_t_last_error(void);
 
+/* ---- deterministic training mode --------------------------------------------------------------------------------------------
+ * The entry points above combine partial sums with float atomics (split-K GEMM, LayerNorm dgamma / dbeta, depthwise-conv dw,
+ * embedding scatter-add, the clipping norm), so their last bits depend on CTA scheduling.  The entry points below compute the
+ * same quantities with every output element written by one thread, or combined from partials in a fixed order; the work split
+ * depends only on the shapes.  Run twice on the same inputs they give bit-identical results.  Arguments, errors and the
+ * ACCUMULATE contracts are those of the atomic entry points.  The library still never allocates: where partials are needed the
+ * caller passes device scratch of at least the bytes the matching *_scratch_bytes query returns (SEQPAN_E_WORKSPACE when it
+ * is NULL or smaller).  The scratch is only written before it is read: it needs no initialisation.
+ *
+ * seqpan_t_gemm_det / seqpan_t_gemm_bf16_det: split-K > 1 stores the raw product of each K-split (K ranges as in
+ *   seqpan_t_gemm) to scratch [split][M][N], then C = alpha * (((p0 + p1) + p2) + ...) + bias + beta * C, one thread per
+ *   element, splits in ascending order.  Without split-K they equal seqpan_t_gemm / _bf16 (and need no scratch). */
+size_t seqpan_t_gemm_det_scratch_bytes(const SeqpanGemm* g);     /* splitk * M * N * 4 for splitk > 1, else 0 */
+int seqpan_t_gemm_det(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* g, void* scratch,
+                      size_t scratch_bytes, void* stream);
+int seqpan_t_gemm_bf16_det(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* g, void* scratch,
+                           size_t scratch_bytes, void* stream);
+/* Each CTA of a grid fixed by M (resp. rows) writes its partial dgamma | dbeta rows (resp. its [128 x 7] dw) to scratch; one
+ * ordered pass adds the partials in ascending CTA order and adds the result once into dgamma / dbeta (resp. dw). */
+size_t seqpan_t_layernorm_bwd_det_scratch_bytes(int64_t M);
+int seqpan_t_layernorm_bwd_det(float* dx, float* dgamma, float* dbeta, const float* x, const float* dy, const float* gamma,
+                               float eps, int64_t M, void* scratch, size_t scratch_bytes, void* stream);
+size_t seqpan_t_dwconv_bwd_w_det_scratch_bytes(int64_t rows);
+int seqpan_t_dwconv_bwd_w_det(float* dw, const float* x, const float* dy, int64_t rows, int len, void* scratch,
+                              size_t scratch_bytes, void* stream);
+/* dtable[r,:] += s_r with s_r = (((0 + dout[n0,:]) + dout[n1,:]) + ...) over the positions n0 < n1 < ... whose clamped id is r,
+ * in ascending n, in fp32; a row that no id hits is left untouched.  One CTA owns each table row: no scratch. */
+int seqpan_t_scatter_add_rows_det(float* dtable, const float* dout, const int64_t* ids, int64_t n, int dim, int64_t table_rows,
+                                  void* stream);
+/* fp64 partial sums of a grid fixed by n (8-byte aligned scratch), added in ascending order by one thread, once into *out_accum. */
+size_t seqpan_t_sumsq_det_scratch_bytes(int64_t n);
+int seqpan_t_sumsq_det(const float* x, int64_t n, double* out_accum, void* scratch, size_t scratch_bytes, void* stream);
+
 /* ---- single-block entry points (tests / micro-benchmarks) --------------------------------------- */
 /* y[M,N] (+)= x[M,K] . w[N,K]^T + bias ; flags: bit0 ReLU, bit1 add `residual` [M,N] after activation.
  * precision SEQPAN_PREC_FP32: fp32 FFMA kernel.  SEQPAN_PREC_BF16: x and w are rounded to bf16 and the

@@ -95,6 +95,16 @@ SIGNATURES = {
     "seqpan_t_maxpool_bwd": (_i, [_vp, _vp, _vp, _i64, _i, _i, _vp]),
     "seqpan_t_sumsq": (_i, [_vp, _i64, _vp, _vp]),
     "seqpan_t_adamw": (_i, [_vp, _vp, _vp, _vp, _i64, C.POINTER(SeqpanAdamW), _vp, _vp, _vp]),
+    "seqpan_t_gemm_det_scratch_bytes": (_sz, [C.POINTER(SeqpanGemm)]),
+    "seqpan_t_gemm_det": (_i, [_vp, _vp, _vp, _vp, C.POINTER(SeqpanGemm), _vp, _sz, _vp]),
+    "seqpan_t_gemm_bf16_det": (_i, [_vp, _vp, _vp, _vp, C.POINTER(SeqpanGemm), _vp, _sz, _vp]),
+    "seqpan_t_layernorm_bwd_det_scratch_bytes": (_sz, [_i64]),
+    "seqpan_t_layernorm_bwd_det": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_float, _i64, _vp, _sz, _vp]),
+    "seqpan_t_dwconv_bwd_w_det_scratch_bytes": (_sz, [_i64]),
+    "seqpan_t_dwconv_bwd_w_det": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _sz, _vp]),
+    "seqpan_t_scatter_add_rows_det": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _vp]),
+    "seqpan_t_sumsq_det_scratch_bytes": (_sz, [_i64]),
+    "seqpan_t_sumsq_det": (_i, [_vp, _i64, _vp, _vp, _sz, _vp]),
     "seqpan_t_last_error": (C.c_char_p, []),
     "seqpan_last_error": (C.c_char_p, []),
     "seqpan_device_ok": (_i, []),

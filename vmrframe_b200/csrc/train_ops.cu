@@ -14,8 +14,11 @@ namespace {
 // ---- strided batched SGEMM: C[b0,b1] = alpha * A.B + beta * C, every operand addressed by (row stride, column stride) ----
 constexpr int GT = 64, GK = 16;
 
+// PARTIAL (deterministic split-K): each K-split stores its raw tile to part[ks][M][N]; a template parameter, so that the default
+// instantiation is the kernel it was before (its register count, and so its occupancy, is unchanged)
+template <bool PARTIAL>
 __global__ void __launch_bounds__(256) t_gemm_kernel(const float* __restrict__ A, const float* __restrict__ B, float* __restrict__ C,
-                                                     const float* __restrict__ bias, SeqpanGemm g) {
+                                                     const float* __restrict__ bias, SeqpanGemm g, float* __restrict__ part) {
   __shared__ __align__(16) float As[GK][GT + 4];
   __shared__ __align__(16) float Bs[GK][GT + 4];
   const int split = g.splitk > 1 ? g.splitk : 1;
@@ -65,11 +68,38 @@ __global__ void __launch_bounds__(256) t_gemm_kernel(const float* __restrict__ A
     for (int j = 0; j < 4; ++j) {
       const long long gm = m0 + ty * 4 + i, gn = n0 + tx * 4 + j;
       if (gm >= g.M || gn >= g.N) continue;
+      if (PARTIAL) { part[(ks * g.M + gm) * g.N + gn] = acc[i][j]; continue; }
       float* c = C + gm * g.c_rs + gn * g.c_cs;
       const float v = g.alpha * acc[i][j] + ((bias && ks == 0) ? __ldg(bias + gn) : 0.f);     // bias[n]: added once (by K-split 0)
       if (split > 1) atomicAdd(c, v);                                           // C was pre-scaled by beta (0: zeroed) by the launcher
       else *c = v + (g.beta != 0.f ? g.beta * *c : 0.f);
     }
+}
+
+// ---- deterministic split-K: C = alpha * (((p0 + p1) + p2) + ...) + bias + beta * C, one thread per element ----
+__global__ void __launch_bounds__(256) t_splitk_reduce_kernel(float* __restrict__ C, const float* __restrict__ part,
+                                                              const float* __restrict__ bias, SeqpanGemm g, int split) {
+  const long long mn = g.M * g.N;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < mn; i += (long long)gridDim.x * blockDim.x) {
+    const long long m = i / g.N, n = i % g.N;
+    float s = part[i];
+    for (int k = 1; k < split; ++k) s += part[k * mn + i];
+    float* c = C + m * g.c_rs + n;                                   // split-K: c_cs == 1
+    const float v = g.alpha * s + (bias ? __ldg(bias + n) : 0.f);
+    *c = g.beta != 0.f ? v + g.beta * *c : v;
+  }
+}
+
+// ---- out[i] += part[0][i] + part[1][i] + ... in ascending partial order, one thread per element; elements i >= split_at
+// go to out1[i - split_at] (LayerNorm: dgamma | dbeta) ----
+__global__ void __launch_bounds__(256) t_ordered_sum_kernel(float* __restrict__ out0, float* __restrict__ out1, int split_at,
+                                                            const float* __restrict__ part, int parts, int width) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= width) return;
+  float s = part[i];
+  for (int p = 1; p < parts; ++p) s += part[(long long)p * width + i];
+  float* o = i < split_at ? out0 + i : out1 + (i - split_at);
+  *o += s;
 }
 
 // ---- 4-D broadcasting element-wise kernel ----
@@ -144,10 +174,11 @@ __global__ void __launch_bounds__(256) t_softmax_bwd_kernel(float* __restrict__ 
   }
 }
 
-// ---- LayerNorm backward over 128-wide rows: dx, and dgamma / dbeta accumulated with atomics ----
+// ---- LayerNorm backward over 128-wide rows: dx, and dgamma / dbeta accumulated with atomics (or written as per-CTA partials) ----
 __global__ void __launch_bounds__(256) t_layernorm_bwd_kernel(float* __restrict__ dx, float* __restrict__ dgamma, float* __restrict__ dbeta,
                                                               const float* __restrict__ x, const float* __restrict__ dy,
-                                                              const float* __restrict__ gamma, float eps, long long M) {
+                                                              const float* __restrict__ gamma, float eps, long long M,
+                                                              float* __restrict__ part) {
   __shared__ float sg[8][128], sb[8][128];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const float4 g = sq::ldg4(gamma + lane * 4);
@@ -172,8 +203,13 @@ __global__ void __launch_bounds__(256) t_layernorm_bwd_kernel(float* __restrict_
     float a = 0.f, b = 0.f;
 #pragma unroll
     for (int w = 0; w < 8; ++w) { a += sg[w][threadIdx.x]; b += sb[w][threadIdx.x]; }
-    atomicAdd(dgamma + threadIdx.x, a);
-    atomicAdd(dbeta + threadIdx.x, b);
+    if (part) {                                   // deterministic: this CTA's [dgamma | dbeta] partial row
+      part[blockIdx.x * 256 + threadIdx.x] = a;
+      part[blockIdx.x * 256 + 128 + threadIdx.x] = b;
+    } else {
+      atomicAdd(dgamma + threadIdx.x, a);
+      atomicAdd(dbeta + threadIdx.x, b);
+    }
   }
 }
 
@@ -193,7 +229,7 @@ __global__ void __launch_bounds__(128) t_dwconv_kernel(float* __restrict__ y, co
 }
 // dw[c, j] += sum over rows of dy[r, c] * x[r + j - 3, c] (inside the row's segment)
 __global__ void __launch_bounds__(128) t_dwconv_bwd_w_kernel(float* __restrict__ dw, const float* __restrict__ x, const float* __restrict__ dy,
-                                                             long long rows, int len) {
+                                                             long long rows, int len, float* __restrict__ part) {
   const int c = threadIdx.x;
   float acc[7] = {};
   for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
@@ -206,7 +242,10 @@ __global__ void __launch_bounds__(128) t_dwconv_bwd_w_kernel(float* __restrict__
     }
   }
 #pragma unroll
-  for (int j = 0; j < 7; ++j) atomicAdd(dw + c * 7 + j, acc[j]);
+  for (int j = 0; j < 7; ++j) {
+    if (part) part[blockIdx.x * (128 * 7) + c * 7 + j] = acc[j];   // deterministic: this CTA's [128 x 7] partial
+    else atomicAdd(dw + c * 7 + j, acc[j]);
+  }
 }
 
 // ---- row gather / scatter-add (embeddings) ----
@@ -223,6 +262,52 @@ __global__ void __launch_bounds__(128) t_scatter_add_rows_kernel(float* __restri
   long long id = ids[n];
   id = id < 0 ? 0 : (id >= nrows_table ? nrows_table - 1 : id);
   for (int d = threadIdx.x; d < dim; d += blockDim.x) atomicAdd(dtable + id * dim + d, dout[n * dim + d]);
+}
+
+// Deterministic adjoint: CTAs own table rows (grid-stride over rows); a CTA scans all ids 128 at a time and adds the matching
+// dout rows in ascending n into registers, then adds the sum once into dtable.  Columns: thread t owns t, t + 128, ...
+constexpr int SC_COLS = 4;   // columns per thread per pass: dim <= 512 in one scan of the ids
+__global__ void __launch_bounds__(128) t_scatter_add_rows_det_kernel(float* __restrict__ dtable, const float* __restrict__ dout,
+                                                                     const int64_t* __restrict__ ids, long long n, int dim,
+                                                                     long long nrows_table) {
+  __shared__ unsigned hits[4];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (long long row = blockIdx.x; row < nrows_table; row += gridDim.x) {
+    for (int d0 = 0; d0 < dim; d0 += 128 * SC_COLS) {
+      float acc[SC_COLS] = {};
+      bool any = false;
+      for (long long n0 = 0; n0 < n; n0 += 128) {
+        const long long nn = n0 + threadIdx.x;
+        bool hit = false;
+        if (nn < n) {
+          long long id = __ldg(ids + nn);
+          id = id < 0 ? 0 : (id >= nrows_table ? nrows_table - 1 : id);
+          hit = id == row;
+        }
+        const unsigned b = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) hits[warp] = b;
+        __syncthreads();
+        for (int w = 0; w < 4; ++w) {
+          for (unsigned m = hits[w]; m; m &= m - 1) {
+            const float* src = dout + (n0 + w * 32 + __ffs(m) - 1) * dim;
+            any = true;
+#pragma unroll
+            for (int k = 0; k < SC_COLS; ++k) {
+              const int d = d0 + k * 128 + threadIdx.x;
+              if (d < dim) acc[k] += src[d];
+            }
+          }
+        }
+        __syncthreads();
+      }
+      if (!any) continue;                       // no id hits this row: dtable's row is left untouched
+#pragma unroll
+      for (int k = 0; k < SC_COLS; ++k) {
+        const int d = d0 + k * 128 + threadIdx.x;
+        if (d < dim) dtable[row * dim + d] += acc[k];
+      }
+    }
+  }
 }
 
 // ---- max over the middle dim of [N, P, C] with indices (torch.max(dim): first maximum wins), and its scatter ----
@@ -246,7 +331,8 @@ __global__ void __launch_bounds__(128) t_maxpool_bwd_kernel(float* __restrict__ 
 }
 
 // ---- optimizer: sum of squares (clip_grad_norm_) and fused AdamW (torch.optim.AdamW semantics, utils/utils.py:87-97) ----
-__global__ void __launch_bounds__(256) t_sumsq_kernel(const float* __restrict__ x, long long n, double* __restrict__ out) {
+__global__ void __launch_bounds__(256) t_sumsq_kernel(const float* __restrict__ x, long long n, double* __restrict__ out,
+                                                      double* __restrict__ part) {
   float acc = 0.f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) acc = fmaf(x[i], x[i], acc);
   acc = sq::warp_sum(acc);
@@ -256,8 +342,14 @@ __global__ void __launch_bounds__(256) t_sumsq_kernel(const float* __restrict__ 
   if (threadIdx.x == 0) {
     double s = 0.0;
     for (int i = 0; i < 8; ++i) s += red[i];
-    atomicAdd(out, s);
+    if (part) part[blockIdx.x] = s;               // deterministic: this CTA's partial
+    else atomicAdd(out, s);
   }
+}
+__global__ void t_sumsq_reduce_kernel(double* __restrict__ out, const double* __restrict__ part, int parts) {
+  double s = 0.0;
+  for (int p = 0; p < parts; ++p) s += part[p];
+  *out += s;
 }
 __global__ void __launch_bounds__(256) t_adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                       float* __restrict__ v, long long n, SeqpanAdamW a, const double* __restrict__ sumsq,
@@ -286,6 +378,10 @@ unsigned grid_for(long long n, int per_block, long long cap = 148 * 16) {
   long long b = (n + per_block - 1) / per_block;
   return (unsigned)(b < 1 ? 1 : (b > cap ? cap : b));
 }
+// grids of the reductions: functions of the shape only (the deterministic entry points size their scratch from them)
+unsigned ln_bwd_grid(long long M) { return grid_for(M, 8, 148 * 4); }
+unsigned dwconv_bwd_w_grid(long long rows) { return grid_for(rows, 64, 148 * 8); }
+unsigned sumsq_grid(long long n) { return grid_for(n, 1024, 148 * 4); }
 
 }  // namespace
 
@@ -296,7 +392,8 @@ int tcheck() {
   return SEQPAN_OK;
 }
 
-int t_gemm_prepare(const float* A, const float* B, float* C, const SeqpanGemm* gp, cudaStream_t st, int& split, long long& gz) {
+int t_gemm_prepare(const float* A, const float* B, float* C, const SeqpanGemm* gp, cudaStream_t st, int& split, long long& gz,
+                   bool zero_c) {
   gz = 0;
   if (!A || !B || !C || !gp) return tfail("gemm: NULL argument");
   const SeqpanGemm& g = *gp;
@@ -306,7 +403,7 @@ int t_gemm_prepare(const float* A, const float* B, float* C, const SeqpanGemm* g
   if (split > 1) {
     if (g.beta != 0.f && g.beta != 1.f) return tfail("gemm: split-K needs beta 0 or 1");
     if (g.batch0 * g.batch1 != 1 || g.c_cs != 1) return tfail("gemm: split-K needs one batch and a row-major C");
-    if (g.beta == 0.f) {
+    if (g.beta == 0.f && zero_c) {
       if (cudaMemset2DAsync(C, (size_t)g.c_rs * sizeof(float), 0, (size_t)g.N * sizeof(float), (size_t)g.M, st) != cudaSuccess) return tcheck();
     }
   }
@@ -314,6 +411,21 @@ int t_gemm_prepare(const float* A, const float* B, float* C, const SeqpanGemm* g
   if (z > 65535) return tfail("gemm: too many batches");
   gz = z;
   return SEQPAN_OK;
+}
+
+size_t t_gemm_det_scratch(const SeqpanGemm& g) {
+  return g.splitk > 1 && g.M > 0 && g.N > 0 ? (size_t)g.splitk * g.M * g.N * sizeof(float) : 0;
+}
+int t_gemm_det_check(const SeqpanGemm& g, const void* scratch, size_t scratch_bytes) {
+  if (!scratch || scratch_bytes < t_gemm_det_scratch(g)) {
+    snprintf(g_terr, sizeof(g_terr), "gemm: split-K scratch needs %zu bytes", t_gemm_det_scratch(g));
+    return SEQPAN_E_WORKSPACE;
+  }
+  return SEQPAN_OK;
+}
+int t_gemm_splitk_reduce(float* C, const float* part, const float* bias, const SeqpanGemm& g, int split, cudaStream_t st) {
+  t_splitk_reduce_kernel<<<grid_for(g.M * g.N, 256), 256, 0, st>>>(C, part, bias, g, split);
+  return tcheck();
 }
 
 extern "C" const char* seqpan_t_last_error(void) { return g_terr; }
@@ -326,8 +438,27 @@ extern "C" int seqpan_t_gemm(const float* A, const float* B, float* C, const flo
   if (rc != SEQPAN_OK || gz == 0) return rc;
   const SeqpanGemm g = *gp;
   dim3 grid((unsigned)((g.N + GT - 1) / GT), (unsigned)((g.M + GT - 1) / GT), (unsigned)gz);
-  t_gemm_kernel<<<grid, 256, 0, st>>>(A, B, C, bias, g);
+  t_gemm_kernel<false><<<grid, 256, 0, st>>>(A, B, C, bias, g, nullptr);
   return tcheck();
+}
+extern "C" size_t seqpan_t_gemm_det_scratch_bytes(const SeqpanGemm* g) { return g ? t_gemm_det_scratch(*g) : 0; }
+extern "C" int seqpan_t_gemm_det(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, void* scratch,
+                                 size_t scratch_bytes, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  int split = 1;
+  long long gz = 0;
+  int rc = t_gemm_prepare(A, B, C, gp, st, split, gz, false);
+  if (rc != SEQPAN_OK || gz == 0) return rc;
+  const SeqpanGemm g = *gp;
+  dim3 grid((unsigned)((g.N + GT - 1) / GT), (unsigned)((g.M + GT - 1) / GT), (unsigned)gz);
+  if (split == 1) {                             // no K-split: every element is already written by one thread
+    t_gemm_kernel<false><<<grid, 256, 0, st>>>(A, B, C, bias, g, nullptr);
+    return tcheck();
+  }
+  if ((rc = t_gemm_det_check(g, scratch, scratch_bytes)) != SEQPAN_OK) return rc;
+  t_gemm_kernel<true><<<grid, 256, 0, st>>>(A, B, C, nullptr, g, (float*)scratch);
+  if ((rc = tcheck()) != SEQPAN_OK) return rc;
+  return t_gemm_splitk_reduce(C, (const float*)scratch, bias, g, split, st);
 }
 
 extern "C" int seqpan_t_ewise(float* out, const float* a, const float* b, const float* c, const SeqpanEwise* ep, void* stream) {
@@ -359,7 +490,24 @@ extern "C" int seqpan_t_layernorm_bwd(float* dx, float* dgamma, float* dbeta, co
                                       float eps, int64_t M, void* stream) {
   if (!dx || !dgamma || !dbeta || !x || !dy || !gamma) return tfail("layernorm_bwd: NULL argument");
   if (M <= 0) return SEQPAN_OK;
-  t_layernorm_bwd_kernel<<<grid_for(M, 8, 148 * 4), 256, 0, (cudaStream_t)stream>>>(dx, dgamma, dbeta, x, dy, gamma, eps, M);
+  t_layernorm_bwd_kernel<<<ln_bwd_grid(M), 256, 0, (cudaStream_t)stream>>>(dx, dgamma, dbeta, x, dy, gamma, eps, M, nullptr);
+  return tcheck();
+}
+extern "C" size_t seqpan_t_layernorm_bwd_det_scratch_bytes(int64_t M) {
+  return M > 0 ? (size_t)ln_bwd_grid(M) * 256 * sizeof(float) : 0;
+}
+extern "C" int seqpan_t_layernorm_bwd_det(float* dx, float* dgamma, float* dbeta, const float* x, const float* dy, const float* gamma,
+                                          float eps, int64_t M, void* scratch, size_t scratch_bytes, void* stream) {
+  if (!dx || !dgamma || !dbeta || !x || !dy || !gamma) return tfail("layernorm_bwd: NULL argument");
+  if (M <= 0) return SEQPAN_OK;
+  if (!scratch || scratch_bytes < seqpan_t_layernorm_bwd_det_scratch_bytes(M)) {
+    tfail("layernorm_bwd: scratch too small");
+    return SEQPAN_E_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned nb = ln_bwd_grid(M);
+  t_layernorm_bwd_kernel<<<nb, 256, 0, st>>>(dx, dgamma, dbeta, x, dy, gamma, eps, M, (float*)scratch);
+  t_ordered_sum_kernel<<<1, 256, 0, st>>>(dgamma, dbeta, 128, (const float*)scratch, (int)nb, 256);
   return tcheck();
 }
 
@@ -372,7 +520,24 @@ extern "C" int seqpan_t_dwconv(float* y, const float* x, const float* w, int64_t
 extern "C" int seqpan_t_dwconv_bwd_w(float* dw, const float* x, const float* dy, int64_t rows, int len, void* stream) {
   if (!dw || !x || !dy || len < 1 || rows % len) return tfail("dwconv_bwd_w: bad argument");
   if (rows <= 0) return SEQPAN_OK;
-  t_dwconv_bwd_w_kernel<<<grid_for(rows, 64, 148 * 8), 128, 0, (cudaStream_t)stream>>>(dw, x, dy, rows, len);
+  t_dwconv_bwd_w_kernel<<<dwconv_bwd_w_grid(rows), 128, 0, (cudaStream_t)stream>>>(dw, x, dy, rows, len, nullptr);
+  return tcheck();
+}
+extern "C" size_t seqpan_t_dwconv_bwd_w_det_scratch_bytes(int64_t rows) {
+  return rows > 0 ? (size_t)dwconv_bwd_w_grid(rows) * 128 * 7 * sizeof(float) : 0;
+}
+extern "C" int seqpan_t_dwconv_bwd_w_det(float* dw, const float* x, const float* dy, int64_t rows, int len, void* scratch,
+                                         size_t scratch_bytes, void* stream) {
+  if (!dw || !x || !dy || len < 1 || rows % len) return tfail("dwconv_bwd_w: bad argument");
+  if (rows <= 0) return SEQPAN_OK;
+  if (!scratch || scratch_bytes < seqpan_t_dwconv_bwd_w_det_scratch_bytes(rows)) {
+    tfail("dwconv_bwd_w: scratch too small");
+    return SEQPAN_E_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned nb = dwconv_bwd_w_grid(rows);
+  t_dwconv_bwd_w_kernel<<<nb, 128, 0, st>>>(dw, x, dy, rows, len, (float*)scratch);
+  t_ordered_sum_kernel<<<(128 * 7 + 255) / 256, 256, 0, st>>>(dw, dw, 128 * 7, (const float*)scratch, (int)nb, 128 * 7);
   return tcheck();
 }
 
@@ -387,6 +552,13 @@ extern "C" int seqpan_t_scatter_add_rows(float* dtable, const float* dout, const
   if (!dtable || !dout || !ids || dim < 1 || table_rows < 1) return tfail("scatter_add_rows: bad argument");
   if (n <= 0) return SEQPAN_OK;
   t_scatter_add_rows_kernel<<<(unsigned)n, 128, 0, (cudaStream_t)stream>>>(dtable, dout, ids, dim, table_rows);
+  return tcheck();
+}
+extern "C" int seqpan_t_scatter_add_rows_det(float* dtable, const float* dout, const int64_t* ids, int64_t n, int dim,
+                                             int64_t table_rows, void* stream) {
+  if (!dtable || !dout || !ids || dim < 1 || table_rows < 1) return tfail("scatter_add_rows: bad argument");
+  if (n <= 0) return SEQPAN_OK;
+  t_scatter_add_rows_det_kernel<<<grid_for(table_rows, 1), 128, 0, (cudaStream_t)stream>>>(dtable, dout, ids, n, dim, table_rows);
   return tcheck();
 }
 
@@ -407,7 +579,21 @@ extern "C" int seqpan_t_maxpool_bwd(float* dx, const float* dout, const int32_t*
 extern "C" int seqpan_t_sumsq(const float* x, int64_t n, double* out_accum, void* stream) {
   if (!x || !out_accum) return tfail("sumsq: NULL argument");
   if (n <= 0) return SEQPAN_OK;
-  t_sumsq_kernel<<<grid_for(n, 1024, 148 * 4), 256, 0, (cudaStream_t)stream>>>(x, n, out_accum);
+  t_sumsq_kernel<<<sumsq_grid(n), 256, 0, (cudaStream_t)stream>>>(x, n, out_accum, nullptr);
+  return tcheck();
+}
+extern "C" size_t seqpan_t_sumsq_det_scratch_bytes(int64_t n) { return n > 0 ? (size_t)sumsq_grid(n) * sizeof(double) : 0; }
+extern "C" int seqpan_t_sumsq_det(const float* x, int64_t n, double* out_accum, void* scratch, size_t scratch_bytes, void* stream) {
+  if (!x || !out_accum) return tfail("sumsq: NULL argument");
+  if (n <= 0) return SEQPAN_OK;
+  if (!scratch || scratch_bytes < seqpan_t_sumsq_det_scratch_bytes(n) || ((uintptr_t)scratch & 7)) {
+    tfail("sumsq: scratch too small or not 8-byte aligned");
+    return SEQPAN_E_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned nb = sumsq_grid(n);
+  t_sumsq_kernel<<<nb, 256, 0, st>>>(x, n, out_accum, (double*)scratch);
+  t_sumsq_reduce_kernel<<<1, 1, 0, st>>>(out_accum, (const double*)scratch, (int)nb);
   return tcheck();
 }
 extern "C" int seqpan_t_adamw(float* p, const float* g, float* m, float* v, int64_t n, const SeqpanAdamW* a, const double* sumsq,

@@ -12,7 +12,9 @@
 //   * thread 0 issues UMMA 128xBNx16 (kind::f16) on the staged k-block and commits to that stage's barrier; two stages, so
 //     the staging of k-block kb + 1 overlaps the MMAs of kb.  Edges (M, N, K) are zero-padded in shared memory.
 //   * epilogue: tcgen05.ld (one TMEM lane = one output row per thread), transposed through shared memory so that each warp
-//     stores 32 consecutive columns of a row at once; alpha, bias (K-split 0 only), beta; atomicAdd when split-K.
+//     stores 32 consecutive columns of a row at once; alpha, bias (K-split 0 only), beta; atomicAdd when split-K.  The
+//     deterministic entry point (seqpan_t_gemm_bf16_det) instead stores each K-split's raw tile to scratch [split][M][N] and
+//     leaves alpha, bias and beta to the ordered reduction of train_ops.cu.
 // No synchronisation and no allocation on the host side: TrainStep(graph=True) captures it like the fp32 kernel.
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -40,6 +42,7 @@ struct TbParams {
   long long kchunk;    // K range of one split: multiple of TB_K
   int a_kmaj, b_kmaj;  // the operand has unit stride along K
   int a_vec, b_vec;    // ... and every row start is 16-byte aligned: 8 k-values = two float4 loads
+  float* part;         // deterministic split-K: raw partial tiles [split][M][N] instead of C (NULL: write / add into C)
 };
 
 // One k-block [k0, min(k0 + 64, kend)) of an operand with `rows` tile rows (rows_valid of them inside the matrix): element
@@ -89,7 +92,7 @@ __global__ void __launch_bounds__(TB_THREADS) t_gemm_bf16_kernel(const float* __
   const long long kbeg = ks * p.kchunk, kend = min((long long)g.K, kbeg + p.kchunk);
   const int nkb = kbeg < kend ? (int)((kend - kbeg + TB_K - 1) / TB_K) : 0;
   const bool add_bias = bias && ks == 0;
-  if (nkb == 0 && p.split > 1 && !add_bias) return;   // an empty K-split adds nothing
+  if (nkb == 0 && p.split > 1 && !add_bias && !p.part) return;   // an empty K-split adds nothing (its partial tile is zeros)
   A += b0 * g.a_b0 + b1 * g.a_b1;
   B += b0 * g.b_b0 + b1 * g.b_b1;
   C += b0 * g.c_b0 + b1 * g.c_b1;
@@ -170,6 +173,7 @@ __global__ void __launch_bounds__(TB_THREADS) t_gemm_bf16_kernel(const float* __
     for (int i = 0; i < 32; ++i) {
       const long long m = mrow + i;
       if (!nok || m >= g.M) continue;
+      if (p.part) { p.part[(ks * g.M + m) * g.N + n] = stg[i * 33 + lane]; continue; }
       float* cp = C + m * g.c_rs + n * g.c_cs;
       const float v = g.alpha * stg[i * 33 + lane] + bv;
       if (p.split > 1) atomicAdd(cp, v);                         // C was pre-scaled by beta (0: zeroed) by the launcher
@@ -191,18 +195,16 @@ bool aligned16(const float* base, long long rs, long long s0, long long s1) {
 
 }  // namespace
 
-extern "C" int seqpan_t_gemm_bf16(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  int split = 1;
-  long long gz = 0;
-  const int rc = t_gemm_prepare(A, B, C, gp, st, split, gz);
-  if (rc != SEQPAN_OK || gz == 0) return rc;
+// part == NULL: seqpan_t_gemm_bf16; otherwise the K-splits of a split-K product store their raw tiles to `part`
+static int t_gemm_bf16_launch(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, int split, long long gz,
+                       float* part, cudaStream_t st) {
   static SqSmemOptIn optin;
   if (optin.ensure((const void*)t_gemm_bf16_kernel, TB_SMEM) != cudaSuccess) return tcheck();
   TbParams p;
   p.g = *gp;
   const SeqpanGemm& g = p.g;
   p.split = split;
+  p.part = part;
   p.kchunk = ((g.K + split - 1) / split + TB_K - 1) / TB_K * TB_K;
   // N tile: the smallest legal UMMA N that covers N, at most 128; halved to 64 when 128-wide tiles leave most SMs idle
   const long long mt = (g.M + TB_M - 1) / TB_M;
@@ -215,4 +217,26 @@ extern "C" int seqpan_t_gemm_bf16(const float* A, const float* B, float* C, cons
   dim3 grid((unsigned)((g.N + p.bn - 1) / p.bn), (unsigned)mt, (unsigned)gz);
   t_gemm_bf16_kernel<<<grid, TB_THREADS, TB_SMEM, st>>>(A, B, C, bias, p);
   return tcheck();
+}
+
+extern "C" int seqpan_t_gemm_bf16(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  int split = 1;
+  long long gz = 0;
+  const int rc = t_gemm_prepare(A, B, C, gp, st, split, gz);
+  if (rc != SEQPAN_OK || gz == 0) return rc;
+  return t_gemm_bf16_launch(A, B, C, bias, gp, split, gz, nullptr, st);
+}
+
+extern "C" int seqpan_t_gemm_bf16_det(const float* A, const float* B, float* C, const float* bias, const SeqpanGemm* gp,
+                                      void* scratch, size_t scratch_bytes, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  int split = 1;
+  long long gz = 0;
+  int rc = t_gemm_prepare(A, B, C, gp, st, split, gz, false);
+  if (rc != SEQPAN_OK || gz == 0) return rc;
+  if (split == 1) return t_gemm_bf16_launch(A, B, C, bias, gp, split, gz, nullptr, st);   // already one writer per element
+  if ((rc = t_gemm_det_check(*gp, scratch, scratch_bytes)) != SEQPAN_OK) return rc;
+  if ((rc = t_gemm_bf16_launch(A, B, C, nullptr, gp, split, gz, (float*)scratch, st)) != SEQPAN_OK) return rc;
+  return t_gemm_splitk_reduce(C, (const float*)scratch, bias, *gp, split, st);
 }

@@ -52,6 +52,14 @@ def train_precision(model, precision=None):
     return _check_precision(precision)
 
 
+def deterministic_mode():
+    """True while ``torch.use_deterministic_algorithms(True)`` is in force (``warn_only=True`` included: the deterministic
+    kernels exist, so there is nothing to warn about).  Then every tape reduces with the fixed-order ``seqpan_t_*_det`` kernels
+    instead of float atomics, and two runs of a step on the same inputs and draws are bit-identical (DESIGN.md section 10).
+    ``cudnn.deterministic`` is deliberately not consulted."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # kernel backend: torch tensors in, library kernels underneath
 # ---------------------------------------------------------------------------------------------------------------------
@@ -87,6 +95,10 @@ class CudaBackend:
     def empty(self, shape):
         return torch.empty(tuple(shape), dtype=torch.float32, device=self.device)
 
+    def _scratch(self, nbytes):
+        """Device scratch of a deterministic kernel (fp32 elements; torch's allocator, so the graph's pool under capture)."""
+        return self.empty(((nbytes + 7) // 8 * 2,))
+
     def zeros(self, shape):
         return torch.zeros(tuple(shape), dtype=torch.float32, device=self.device)
 
@@ -111,9 +123,10 @@ class CudaBackend:
         return -torch.empty(tuple(shape), dtype=torch.float32, device=self.device).exponential_().log()
 
     # -- C[..., M, N] = alpha * A[..., M, K] @ B[..., K, N] + beta * C --
-    def gemm(self, A, B, out=None, alpha=1.0, beta=0.0, splitk=1, bias=None, mixed=False):
+    def gemm(self, A, B, out=None, alpha=1.0, beta=0.0, splitk=1, bias=None, mixed=False, deterministic=False):
         """``mixed=True``: bf16 operands (rounded to nearest even), fp32 accumulation, on the tensor cores
-        (``seqpan_t_gemm_bf16``); otherwise the fp32 kernel."""
+        (``seqpan_t_gemm_bf16``); otherwise the fp32 kernel.  ``deterministic=True``: a split-K product reduces its partial
+        tiles in a fixed order (``seqpan_t_gemm_det`` / ``_bf16_det``) instead of with atomics."""
         self._req(A, B, out, bias)
         nb = A.dim() - 2
         assert B.dim() == A.dim() and 0 <= nb <= 2 and A.shape[-1] == B.shape[-2] and A.shape[:nb] == B.shape[:nb]
@@ -130,8 +143,15 @@ class CudaBackend:
         sa, sb, sc = (_pad4(t.stride()[:nb], 0)[2:] for t in (A, B, out))
         g.a_b0, g.a_b1, g.b_b0, g.b_b1, g.c_b0, g.c_b1 = sa[0], sa[1], sb[0], sb[1], sc[0], sc[1]
         g.alpha, g.beta, g.splitk = alpha, beta, splitk if nb == 0 and out.stride(-1) == 1 else 1
-        fn = self.L.seqpan_t_gemm_bf16 if mixed else self.L.seqpan_t_gemm
-        self._chk(fn(A.data_ptr(), B.data_ptr(), out.data_ptr(), bias.data_ptr() if bias is not None else None, C.byref(g), self._st()))
+        args = (A.data_ptr(), B.data_ptr(), out.data_ptr(), bias.data_ptr() if bias is not None else None, C.byref(g))
+        if deterministic and g.splitk > 1:
+            nbytes = self.L.seqpan_t_gemm_det_scratch_bytes(C.byref(g))
+            fn = self.L.seqpan_t_gemm_bf16_det if mixed else self.L.seqpan_t_gemm_det
+            scratch = self._scratch(nbytes)
+            self._chk(fn(*args, scratch.data_ptr(), nbytes, self._st()))
+        else:
+            fn = self.L.seqpan_t_gemm_bf16 if mixed else self.L.seqpan_t_gemm
+            self._chk(fn(*args, self._st()))
         return out
 
     # -- element-wise with broadcasting over <= 4 dims --
@@ -189,12 +209,17 @@ class CudaBackend:
                                                x.numel() // D, self._st()))
         return y
 
-    def layernorm_bwd(self, x, dy, g, eps):
+    def layernorm_bwd(self, x, dy, g, eps, deterministic=False):
         self._req(x, dy, g)
         dy = dy if dy.is_contiguous() else self.ewise("COPY", dy)
         dx, dg, db = torch.empty_like(x), self.zeros((D,)), self.zeros((D,))
-        self._chk(self.L.seqpan_t_layernorm_bwd(dx.data_ptr(), dg.data_ptr(), db.data_ptr(), x.data_ptr(), dy.data_ptr(),
-                                                g.data_ptr(), C.c_float(eps), x.numel() // D, self._st()))
+        args = (dx.data_ptr(), dg.data_ptr(), db.data_ptr(), x.data_ptr(), dy.data_ptr(), g.data_ptr(), C.c_float(eps), x.numel() // D)
+        if deterministic:
+            nb = self.L.seqpan_t_layernorm_bwd_det_scratch_bytes(x.numel() // D)
+            scratch = self._scratch(nb)
+            self._chk(self.L.seqpan_t_layernorm_bwd_det(*args, scratch.data_ptr(), nb, self._st()))
+        else:
+            self._chk(self.L.seqpan_t_layernorm_bwd(*args, self._st()))
         return dx, dg, db
 
     def dwconv(self, x, w, seg_len, flip=False):
@@ -204,11 +229,17 @@ class CudaBackend:
         self._chk(self.L.seqpan_t_dwconv(y.data_ptr(), x.data_ptr(), w.data_ptr(), x.numel() // D, seg_len, int(flip), self._st()))
         return y
 
-    def dwconv_bwd_w(self, x, dy, seg_len):
+    def dwconv_bwd_w(self, x, dy, seg_len, deterministic=False):
         self._req(x, dy)
         dy = dy if dy.is_contiguous() else self.ewise("COPY", dy)
         dw = self.zeros((D, 1, 7))
-        self._chk(self.L.seqpan_t_dwconv_bwd_w(dw.data_ptr(), x.data_ptr(), dy.data_ptr(), x.numel() // D, seg_len, self._st()))
+        args = (dw.data_ptr(), x.data_ptr(), dy.data_ptr(), x.numel() // D, seg_len)
+        if deterministic:
+            nb = self.L.seqpan_t_dwconv_bwd_w_det_scratch_bytes(x.numel() // D)
+            scratch = self._scratch(nb)
+            self._chk(self.L.seqpan_t_dwconv_bwd_w_det(*args, scratch.data_ptr(), nb, self._st()))
+        else:
+            self._chk(self.L.seqpan_t_dwconv_bwd_w(*args, self._st()))
         return dw
 
     def gather_rows(self, table, ids):
@@ -219,12 +250,12 @@ class CudaBackend:
                                               table.shape[0], self._st()))
         return out
 
-    def scatter_add_rows(self, dout, ids, rows):
+    def scatter_add_rows(self, dout, ids, rows, deterministic=False):
         self._req(dout)
         dout = dout if dout.is_contiguous() else self.ewise("COPY", dout)
         dt = self.zeros((rows, dout.shape[-1]))
-        self._chk(self.L.seqpan_t_scatter_add_rows(dt.data_ptr(), dout.data_ptr(), ids.data_ptr(), ids.numel(), dout.shape[-1],
-                                                   rows, self._st()))
+        fn = self.L.seqpan_t_scatter_add_rows_det if deterministic else self.L.seqpan_t_scatter_add_rows
+        self._chk(fn(dt.data_ptr(), dout.data_ptr(), ids.data_ptr(), ids.numel(), dout.shape[-1], rows, self._st()))
         return dt
 
     def maxpool(self, x):
@@ -244,8 +275,13 @@ class CudaBackend:
         self._chk(self.L.seqpan_t_maxpool_bwd(dx.data_ptr(), dout.data_ptr(), idx.data_ptr(), N, P, Cc, self._st()))
         return dx
 
-    def sumsq(self, x, accum):
-        self._chk(self.L.seqpan_t_sumsq(x.data_ptr(), x.numel(), accum.data_ptr(), self._st()))
+    def sumsq(self, x, accum, deterministic=False):
+        if deterministic:
+            nb = self.L.seqpan_t_sumsq_det_scratch_bytes(x.numel())
+            scratch = self._scratch(nb)
+            self._chk(self.L.seqpan_t_sumsq_det(x.data_ptr(), x.numel(), accum.data_ptr(), scratch.data_ptr(), nb, self._st()))
+        else:
+            self._chk(self.L.seqpan_t_sumsq(x.data_ptr(), x.numel(), accum.data_ptr(), self._st()))
 
     def adamw(self, p, g, m, v, hp, sumsq, dyn=None):
         self._chk(self.L.seqpan_t_adamw(p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(), C.byref(hp),
@@ -269,14 +305,19 @@ class SeqpanTape:
     ``precision="bf16"``: the model's matrix products (``linear`` y / dx / dW, the forward ``bmm``, the six products of
     ``attention``, the char-CNN window products) and their adjoints run with bf16 operands and fp32 accumulation; ones-vector
     reductions, bias gradients, the loss functions, LayerNorm, softmax, element-wise ops and the optimizer stay fp32 -- the
-    autocast policy.  ``"fp32"`` calls ``backend.gemm`` exactly as before the mode existed (no ``mixed`` keyword)."""
+    autocast policy.  ``"fp32"`` calls ``backend.gemm`` exactly as before the mode existed (no ``mixed`` keyword).
 
-    def __init__(self, backend, droprate=0.0, training=True, mask_fn=None, precision="fp32"):
+    ``deterministic=True``: every reduction of the backward that the default kernels combine with float atomics (split-K
+    products, LayerNorm dgamma / dbeta, depthwise-conv dw, embedding scatter-add) gets ``deterministic=True`` and runs on the
+    fixed-order kernels; ``False`` passes no such keyword."""
+
+    def __init__(self, backend, droprate=0.0, training=True, mask_fn=None, precision="fp32", deterministic=False):
         self.be = backend
         self.p = float(droprate) if training else 0.0
         self.mask_fn = mask_fn          # optional: (shape) -> keep-mask tensor of 0/1 (parity tests inject the oracle's draws)
         self.nodes = []
         self.mm = {"mixed": True} if _check_precision(precision) == "bf16" else {}    # keywords of a model product's be.gemm
+        self.det = {"deterministic": True} if deterministic else {}                    # keywords of a reduction's backend call
 
     # -- bookkeeping --
     def leaf(self, t, needs=False):
@@ -328,8 +369,8 @@ class SeqpanTape:
         def bwd(g):
             g2 = g.reshape(M, N)
             dx = be.gemm(g2, W2, **self.mm).reshape(x.v.shape) if x.needs else None
-            dW = be.gemm(g2.t(), x2, splitk=sk, **self.mm).reshape(W.v.shape) if W.needs else None
-            db = be.gemm(be.ones(M).reshape(1, M), g2, splitk=sk).reshape(b.v.shape) if (b is not None and b.needs) else None
+            dW = be.gemm(g2.t(), x2, splitk=sk, **self.mm, **self.det).reshape(W.v.shape) if W.needs else None
+            db = be.gemm(be.ones(M).reshape(1, M), g2, splitk=sk, **self.det).reshape(b.v.shape) if (b is not None and b.needs) else None
             return (dx, dW, db) if b is not None else (dx, dW)
         return self._rec(y.reshape(tuple(x.v.shape[:-1]) + (N,)), [x, W] + ([b] if b is not None else []), bwd)
 
@@ -339,7 +380,7 @@ class SeqpanTape:
         y = be.layernorm(xc, g.v, b.v, eps)
 
         def bwd(gy):
-            dx, dg, db = be.layernorm_bwd(xc, gy, g.v, eps)
+            dx, dg, db = be.layernorm_bwd(xc, gy, g.v, eps, **self.det)
             return dx, dg, db
         return self._rec(y, [x, g, b], bwd)
 
@@ -365,7 +406,8 @@ class SeqpanTape:
             for s in g.shape[:lead]:
                 outer *= s
             inner = g.numel() // outer
-            g = be.gemm(be.ones(outer).reshape(1, outer), g.reshape(outer, inner), splitk=min(64, max(1, outer // 128))).reshape(g.shape[lead:])
+            g = be.gemm(be.ones(outer).reshape(1, outer), g.reshape(outer, inner), splitk=min(64, max(1, outer // 128)),
+                        **self.det).reshape(g.shape[lead:])
         for d, (gs, ss) in enumerate(zip(g.shape, shape)):
             if ss == 1 and gs != 1:                    # reduce dim d, keep it
                 outer = 1
@@ -477,7 +519,8 @@ class SeqpanTape:
 
         def bwd(g):
             gc = g if g.is_contiguous() else be.ewise("COPY", g)
-            return (be.dwconv(gc, w.v, seg_len, True) if a.needs else None, be.dwconv_bwd_w(ac, gc, seg_len) if w.needs else None)
+            return (be.dwconv(gc, w.v, seg_len, True) if a.needs else None,
+                    be.dwconv_bwd_w(ac, gc, seg_len, **self.det) if w.needs else None)
         return self._rec(y, [a, w], bwd)
 
     def cat_last(self, parts):
@@ -500,7 +543,7 @@ class SeqpanTape:
     def embedding(self, table, ids):
         be = self.be
         y = be.gather_rows(table.v, ids)
-        return self._rec(y, [table], lambda g: (be.scatter_add_rows(g.reshape(-1, g.shape[-1]), ids, table.v.shape[0]),))
+        return self._rec(y, [table], lambda g: (be.scatter_add_rows(g.reshape(-1, g.shape[-1]), ids, table.v.shape[0], **self.det),))
 
     def maxpool_mid(self, a):
         be = self.be
@@ -520,7 +563,7 @@ class SeqpanTape:
         be = self.be
         ac = a.v if a.v.is_contiguous() else be.ewise("COPY", a.v)
         n = ac.numel()
-        y = be.gemm(be.ones(n).reshape(1, n), ac.reshape(n, 1), splitk=min(64, max(1, n // 2048))).reshape(())
+        y = be.gemm(be.ones(n).reshape(1, n), ac.reshape(n, 1), splitk=min(64, max(1, n // 2048)), **self.det).reshape(())
         return self._rec(y, [a], lambda g: (g.reshape((1,) * a.v.dim()).expand(a.v.shape),))
 
     def log(self, a):
@@ -667,9 +710,9 @@ def _text_embedding(tp, P, word_ids, char_ids):
                 dce = be.zeros((R, 100))
                 for j in range(k):                       # overlapping windows add up: k shifted accumulations
                     be.ewise("AXPBY", dce[j:j + Rk], dwin[:, j * 100:(j + 1) * 100], out=dce[j:j + Rk], alpha=1.0, beta=1.0)
-            dWp = be.gemm(g2[:Rk].t(), win, splitk=min(64, max(1, Rk // 128)), **tp.mm)             # [ch, k*100]
+            dWp = be.gemm(g2[:Rk].t(), win, splitk=min(64, max(1, Rk // 128)), **tp.mm, **tp.det)   # [ch, k*100]
             dW = be.ewise("COPY", dWp.reshape(ch, k, 100).permute(0, 2, 1)).reshape(Wk.v.shape)
-            db = be.gemm(be.ones(R).reshape(1, R), g2, splitk=min(64, max(1, R // 128))).reshape(ch)
+            db = be.gemm(be.ones(R).reshape(1, R), g2, splitk=min(64, max(1, R // 128)), **tp.det).reshape(ch)
             return dce, dW, db
         yk = tp._rec(y, [ce, Wk, bk], bwd)
         outs.append(tp.maxpool_mid(tp.relu(yk)))                       # [B*T, ch]
@@ -1005,7 +1048,7 @@ class TrainStep:
         self.dyn = None                      # device float[3]: lr, 1 - beta1^t, sqrt(1 - beta2^t) of the current step
         self._graphs = {}
         self.max_graphs = 8                  # input shapes replayed as CUDA graphs (each holds its activations' memory pool)
-        self._g2, self._g2_seen, self._g2_out = None, 0, None
+        self._g2 = {}                        # deterministic mode -> the clip + AdamW half: {"seen", "graph", "out"}
         self.views = {}
 
     def _lr_now(self):
@@ -1022,7 +1065,8 @@ class TrainStep:
         """Forward + both losses + backward.  Returns ``(loss tensor (device scalar), {name: grad}, outputs)``."""
         be = self.be
         m = self.model
-        tp = SeqpanTape(be, droprate=m.configs.model.droprate, training=m.training, mask_fn=self.mask_fn, precision=self.precision)
+        tp = SeqpanTape(be, droprate=m.configs.model.droprate, training=m.training, mask_fn=self.mask_fn, precision=self.precision,
+                        deterministic=deterministic_mode())
         P = _Params(tp, self.named)
         vmask, tmask = data["vmasks"].to(torch.float32), data["tmasks"].to(torch.float32)
         spec = train_spec(m)
@@ -1072,13 +1116,13 @@ class TrainStep:
             return dist.get_world_size()
         return 1
 
-    def _part2(self, world):
+    def _part2(self, world, det):
         """Mean over the ranks, squared norm for clip_grad_norm_, AdamW on every live tensor (scalars of the step from ``self.dyn``)."""
         be = self.be
         if world > 1:
             be.ewise("AFFINE", self.flat, out=self.flat, alpha=1.0 / world, beta=0.0)
         ss = torch.zeros((), dtype=torch.float64, device=self.flat.device)
-        be.sumsq(self.flat, ss)
+        be.sumsq(self.flat, ss, **({"deterministic": True} if det else {}))
         for k in self.live:
             p = self.named[k]
             if k not in self.m:
@@ -1097,8 +1141,10 @@ class TrainStep:
         clip + AdamW) as CUDA graphs after two eager steps per input shape: the tape issues ~1200 small launches from Python,
         which is host-bound; the graphs keep the same kernels and remove the host.  Inputs are copied into static buffers, the
         dropout / Gumbel draws stay fresh (torch's graph-safe generator), the gradient all-reduce stays an eager call between
-        the two graphs."""
+        the two graphs.  Graphs are kept per deterministic mode (:func:`deterministic_mode`): a graph captured in one mode never
+        replays in the other."""
         be = self.be
+        det = deterministic_mode()
         self.t += 1
         sc = self._scalars()
         if self.dyn is None:
@@ -1112,9 +1158,9 @@ class TrainStep:
         if not graph:
             loss, out = self._part1(data, gumbel)
             world = self._allreduce()
-            ss = self._part2(world)
+            ss = self._part2(world, det)
         else:
-            key = tuple((k, tuple(v.shape)) for k, v in sorted(data.items())) + (gumbel is not None,)
+            key = tuple((k, tuple(v.shape)) for k, v in sorted(data.items())) + (gumbel is not None, det)
             ent = self._graphs.setdefault(key, {"seen": 0})
             # every captured shape keeps its own pool of intermediates alive: at most `max_graphs` shapes are captured (the most
             # frequent ones arrive first in practice), the rest run from the tape
@@ -1138,18 +1184,19 @@ class TrainStep:
                 ent["graph"].replay()
                 loss, out = ent["out"]
             world = self._allreduce()
-            if self._g2 is None and self._g2_seen < 2:
-                self._g2_seen += 1
-                ss = self._part2(world)
+            e2 = self._g2.setdefault(det, {"seen": 0})
+            if "graph" not in e2 and e2["seen"] < 2:
+                e2["seen"] += 1
+                ss = self._part2(world, det)
             else:
-                if self._g2 is None:
+                if "graph" not in e2:
                     torch.cuda.synchronize()
                     g2 = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g2):
-                        self._g2_out = self._part2(world)
-                    self._g2 = g2
-                self._g2.replay()
-                ss = self._g2_out
+                        e2["out"] = self._part2(world, det)
+                    e2["graph"] = g2
+                e2["graph"].replay()
+                ss = e2["out"]
         if hasattr(self.model, "repack"):
             self.model.repack()           # the inference handle's packed weights follow the update (p.data edits bump no version)
         return loss, out, ss              # ss: squared gradient norm before clipping (device fp64 scalar)
@@ -1215,7 +1262,8 @@ class _TapeForward(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, be, word_ids, char_ids, vmask, tmask, gumbel, vfeat_in, names, *params):
         ctx.set_materialize_grads(False)          # an output nobody used arrives as None and costs nothing
-        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model))
+        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model),
+                        deterministic=deterministic_mode())
         P = _Params(tp, dict(zip(names, params)))
         xv = tp.leaf(vfeat_in, needs=ctx.needs_input_grad[7])
         outs = [o for o in forward_train(tp, P, word_ids, char_ids, xv, vmask, tmask, gumbel, **train_spec(model)["fwd"])
