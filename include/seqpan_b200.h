@@ -147,6 +147,21 @@ int seqpan_span_decode(const float* slogits, const float* elogits, const float* 
 /* counters[0..4] (fp64, device) += {n, sum IoU, #IoU>=0.3, #IoU>=0.5, #IoU>=0.7} of fracs vs gt [B,2]. */
 int seqpan_iou_counters(const float* fracs, const float* gt_fracs, int B, double* counters, void* stream);
 
+/* Top-k spans per sample with greedy temporal NMS (infer_basic's probabilities; DESIGN.md section 11).  Candidates are the
+ * spans i <= j with score sp[i]*ep[j] > 0, best first, exact ties to the lower i, then the lower j.  Each of k rounds keeps
+ * the best candidate not yet kept and not suppressed: a kept (a,b) suppresses (i,j) when union > 0 and
+ * (float)inter >= nms_thresh * (float)union on the integer indices (nms_thresh = 1: plain top-k).
+ * Outputs in selection order: start_idx/end_idx [B,k] int64, scores [B,k] fp32, fracs [B,k,2] fp32 (nullable; indices
+ * divided by vmask.sum(1), or by L when vmask is NULL).  Slots beyond the last surviving candidate are -1, -1, 0, -1.
+ * 1 <= k <= SEQPAN_TOPK_MAX, 0 < nms_thresh <= 1, 1 <= L <= SEQPAN_MAX_VLEN.  No allocation, no host synchronisation. */
+#define SEQPAN_TOPK_MAX 32
+int seqpan_span_topk(const float* slogits, const float* elogits, const float* vmask, int B, int L, int k, float nms_thresh,
+                     int64_t* start_idx, int64_t* end_idx, float* scores, float* fracs, void* stream);
+
+/* counters[0..3] (fp64, device) += {n, #>=0.3, #>=0.5, #>=0.7} of the best IoU over each sample's filled top-k slots
+ * (fracs [B,k,2] from seqpan_span_topk, empty slots -1) against gt [B,2]: R@k as counters that add exactly across shards. */
+int seqpan_topk_counters(const float* fracs, const float* gt_fracs, int B, int k, double* counters, void* stream);
+
 /* Host -> device copy of BaseCollate's zero-padded clip features [B,L,row_floats] (utils/BaseDataset.py:201-234 pads
  * every clip to vlen rows) that moves only the first valid_rows[b] rows of each sample over PCIe and writes the
  * padding rows as zeros on the device.  src_host must be PINNED host memory (cudaHostAlloc / torch pin_memory).

@@ -73,6 +73,8 @@ SIGNATURES = {
     "seqpan_forward_shared_video": (_i, [_vp] + [_vp] * 4 + [_i] + [_vp] * 3 + [_i, _i, _i] + [_vp] * 3 + [_vp, _sz, _vp]),
     "seqpan_span_decode": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "seqpan_iou_counters": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "seqpan_span_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, C.c_float, _vp, _vp, _vp, _vp, _vp]),
+    "seqpan_topk_counters": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "seqpan_h2d_ragged": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "seqpan_collate_clips": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "seqpan_collate_text": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),

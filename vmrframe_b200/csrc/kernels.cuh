@@ -92,6 +92,9 @@ cudaError_t launch_build_rowmask(const float* vmask, long long nv, const float* 
 cudaError_t launch_span_decode(const float* s, const float* e, const float* vmask, int B, int L, int64_t* si,
                                int64_t* ei, float* fracs, cudaStream_t st);
 cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, double* counters, cudaStream_t st);
+cudaError_t launch_span_topk(const float* s, const float* e, const float* vmask, int B, int L, int k, float thr,
+                             int64_t* si, int64_t* ei, float* scores, float* fracs, cudaStream_t st);
+cudaError_t launch_topk_counters(const float* fracs, const float* gt, int B, int k, double* counters, cudaStream_t st);
 cudaError_t launch_h2d_ragged(float* dst, const float* src_host, const int32_t* valid_dev, int B, int L, int row_floats,
                               int ctas, cudaStream_t st);
 cudaError_t launch_zero_tail_rows(float* dst, const int32_t* valid_dev, int B, int L, int row_floats, cudaStream_t st);

@@ -935,14 +935,11 @@ cudaError_t launch_build_rowmask(const float* vmask, long long nv, const float* 
 // exactly: the decode is O(L) with a suffix max of ep and a prefix max of sp (SURVEY.md A.7).  Ties resolve to
 // the lowest index like torch.max on CPU.  One warp per sample.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) span_decode_kernel(const float* __restrict__ s, const float* __restrict__ e,
-                                                          const float* __restrict__ vmask, int B, int L,
-                                                          int64_t* __restrict__ si, int64_t* __restrict__ ei,
-                                                          float* __restrict__ fracs) {
-  __shared__ float sp[4][SEQPAN_MAX_VLEN], ep[4][SEQPAN_MAX_VLEN], aux[4][SEQPAN_MAX_VLEN];
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int b = blockIdx.x * 4 + w;
-  if (b >= B) return;
+// sp/ep = softmax(mask_logits(logits, vmask)) of sample b, computed by one warp into shared memory; returns vmask.sum()
+// (0 without a mask).  span_decode_kernel and span_topk_kernel both call it, so their probabilities are the same bits.
+__device__ __forceinline__ float span_probs_warp(const float* __restrict__ s, const float* __restrict__ e,
+                                                 const float* __restrict__ vmask, int b, int L, float* sp, float* ep,
+                                                 int lane) {
   float ms = -INFINITY, me = -INFINITY, nvalid = 0.f;
   for (int i = lane; i < L; i += 32) {
     float a = s[(long long)b * L + i], c = e[(long long)b * L + i];
@@ -952,19 +949,31 @@ __global__ void __launch_bounds__(128) span_decode_kernel(const float* __restric
       c = c + SQ_MASK * (1.0f - m);
       nvalid += m;
     }
-    sp[w][i] = a; ep[w][i] = c;
+    sp[i] = a; ep[i] = c;
     ms = fmaxf(ms, a); me = fmaxf(me, c);
   }
   ms = warp_max(ms); me = warp_max(me); nvalid = warp_sum(nvalid);
   float ss = 0.f, se = 0.f;
   for (int i = lane; i < L; i += 32) {
-    const float a = expf(sp[w][i] - ms), c = expf(ep[w][i] - me);
-    sp[w][i] = a; ep[w][i] = c;
+    const float a = expf(sp[i] - ms), c = expf(ep[i] - me);
+    sp[i] = a; ep[i] = c;
     ss += a; se += c;
   }
   ss = warp_sum(ss); se = warp_sum(se);
-  for (int i = lane; i < L; i += 32) { sp[w][i] = sp[w][i] / ss; ep[w][i] = ep[w][i] / se; }
+  for (int i = lane; i < L; i += 32) { sp[i] = sp[i] / ss; ep[i] = ep[i] / se; }
   __syncwarp();
+  return nvalid;
+}
+
+__global__ void __launch_bounds__(128) span_decode_kernel(const float* __restrict__ s, const float* __restrict__ e,
+                                                          const float* __restrict__ vmask, int B, int L,
+                                                          int64_t* __restrict__ si, int64_t* __restrict__ ei,
+                                                          float* __restrict__ fracs) {
+  __shared__ float sp[4][SEQPAN_MAX_VLEN], ep[4][SEQPAN_MAX_VLEN], aux[4][SEQPAN_MAX_VLEN];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * 4 + w;
+  if (b >= B) return;
+  const float nvalid = span_probs_warp(s, e, vmask, b, L, sp[w], ep[w], lane);
   // start index: argmax_i sp[i] * max_{j>=i} ep[j]
   {   // suffix max of ep, 32 positions per step: warp scan + carry from the chunk behind
     float carry = 0.f;
@@ -1030,15 +1039,20 @@ cudaError_t launch_span_decode(const float* s, const float* e, const float* vmas
 // IoU counters (utils/utils.py:161-185, models/loss.py:83-109): temporal IoU of [s,e] fractions against
 // ground truth, accumulated as {n, sum, #>=0.3, #>=0.5, #>=0.7} in fp64 so shards add exactly.
 // ------------------------------------------------------------------------------------------------
+// calculate_iou of [p0,p1] against [g0,g1]: fp32 min/max, fp64 division, clamped at 0 (shared with topk_counters_kernel)
+__device__ __forceinline__ double span_iou(float g0, float g1, float p0, float p1) {
+  const float u0 = fminf(g0, p0), u1 = fmaxf(g1, p1), i0 = fmaxf(g0, p0), i1 = fminf(g1, p1);
+  double iou = 0.0;
+  if ((u1 - u0) != 0.0f) iou = (double)(i1 - i0) / (double)(u1 - u0);
+  if (iou < 0.0) iou = 0.0;
+  return iou;
+}
+
 __global__ void iou_counters_kernel(const float* __restrict__ fracs, const float* __restrict__ gt, int B,
                                     double* __restrict__ counters) {
   double c[5] = {0, 0, 0, 0, 0};
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
-    const float g0 = gt[b * 2], g1 = gt[b * 2 + 1], p0 = fracs[b * 2], p1 = fracs[b * 2 + 1];
-    const float u0 = fminf(g0, p0), u1 = fmaxf(g1, p1), i0 = fmaxf(g0, p0), i1 = fminf(g1, p1);
-    double iou = 0.0;
-    if ((u1 - u0) != 0.0f) iou = (double)(i1 - i0) / (double)(u1 - u0);
-    if (iou < 0.0) iou = 0.0;
+    const double iou = span_iou(gt[b * 2], gt[b * 2 + 1], fracs[b * 2], fracs[b * 2 + 1]);
     c[0] += 1.0; c[1] += iou; c[2] += iou >= 0.3; c[3] += iou >= 0.5; c[4] += iou >= 0.7;
   }
 #pragma unroll
@@ -1053,6 +1067,123 @@ cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, doub
   int blocks = (B + 255) / 256;
   if (blocks > 148) blocks = 148;
   iou_counters_kernel<<<blocks, 256, 0, st>>>(fracs, gt, B, counters);
+  return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
+// Top-k span retrieval with greedy temporal NMS (DESIGN.md section 11).  Candidates are all spans i <= j with score
+// sp[i]*ep[j] > 0, ordered by (score desc, i asc, j asc).  Each of k rounds keeps the best candidate that no kept span
+// removes; a kept (a,b) removes itself and every (i,j) with union > 0 and inter >= thr * union on the integer indices.
+// One CTA per sample, thread j owns the column of spans ending at j and caches the best of its column: a column is
+// rescanned only when the newly kept span removes that best, so a round usually costs one block-wide argmax.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ bool span_removed(int i, int j, int a, int b, float thr) {
+  if (i == a && j == b) return true;         // explicit: a zero-length span has IoU 0, even with itself
+  const int uni = max(j, b) - min(i, a);
+  const int inter = max(0, min(j, b) - max(i, a));
+  return uni > 0 && (float)inter >= __fmul_rn(thr, (float)uni);
+}
+__device__ __forceinline__ bool span_before(float s, int i, int j, float s2, int i2, int j2) {
+  return s > s2 || (s == s2 && (i < i2 || (i == i2 && j < j2)));
+}
+
+constexpr int kTopkThreads = SEQPAN_MAX_VLEN;   // one thread per end index
+
+__global__ void __launch_bounds__(kTopkThreads) span_topk_kernel(const float* __restrict__ s, const float* __restrict__ e,
+                                                                 const float* __restrict__ vmask, int L, int k, float thr,
+                                                                 int64_t* __restrict__ si, int64_t* __restrict__ ei,
+                                                                 float* __restrict__ scores, float* __restrict__ fracs) {
+  __shared__ float sp[SEQPAN_MAX_VLEN], ep[SEQPAN_MAX_VLEN];
+  __shared__ int ka[SEQPAN_TOPK_MAX], kb[SEQPAN_TOPK_MAX];
+  __shared__ float ws[kTopkThreads / 32];
+  __shared__ int wi[kTopkThreads / 32], wj[kTopkThreads / 32];
+  __shared__ float n_sh;
+  const int b = blockIdx.x, j = threadIdx.x, lane = j & 31, w = j >> 5;
+  if (w == 0) {
+    const float nvalid = span_probs_warp(s, e, vmask, b, L, sp, ep, lane);
+    if (lane == 0) n_sh = vmask ? nvalid : (float)L;
+  }
+  __syncthreads();
+  const float ej = j < L ? ep[j] : 0.f;
+  float bs = 0.f;                            // best of the column: score 0 = none left
+  int bi = INT_MAX;
+  bool stale = j < L;
+  int r = 0;
+  for (; r < k; ++r) {
+    if (stale) {
+      bs = 0.f; bi = INT_MAX;
+      for (int i = 0; i <= j; ++i) {
+        const float sc = sp[i] * ej;
+        if (sc > bs) {                         // strict: the lowest i wins a tie inside the column
+          bool ok = true;
+          for (int q = 0; q < r; ++q) ok = ok && !span_removed(i, j, ka[q], kb[q], thr);
+          if (ok) { bs = sc; bi = i; }
+        }
+      }
+      stale = false;
+    }
+    float S = bs;
+    int I = bi, J = bi == INT_MAX ? INT_MAX : j;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float os = __shfl_xor_sync(0xffffffffu, S, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, I, o), oj = __shfl_xor_sync(0xffffffffu, J, o);
+      if (span_before(os, oi, oj, S, I, J)) { S = os; I = oi; J = oj; }
+    }
+    if (lane == 0) { ws[w] = S; wi[w] = I; wj[w] = J; }
+    __syncthreads();
+    S = ws[0]; I = wi[0]; J = wj[0];
+#pragma unroll
+    for (int q = 1; q < kTopkThreads / 32; ++q)
+      if (span_before(ws[q], wi[q], wj[q], S, I, J)) { S = ws[q]; I = wi[q]; J = wj[q]; }
+    if (S <= 0.f) break;                       // uniform: every thread reduced the same values
+    if (j == 0) {
+      ka[r] = I; kb[r] = J;
+      const long long o = (long long)b * k + r;
+      si[o] = I; ei[o] = J; scores[o] = S;
+      if (fracs) { fracs[o * 2] = (float)I / n_sh; fracs[o * 2 + 1] = (float)J / n_sh; }
+    }
+    __syncthreads();                           // ka/kb visible; ws/wi/wj free for the next round
+    if (bi != INT_MAX && span_removed(bi, j, I, J, thr)) stale = true;
+  }
+  for (int q = r + j; q < k; q += kTopkThreads) {
+    const long long o = (long long)b * k + q;
+    si[o] = -1; ei[o] = -1; scores[o] = 0.f;
+    if (fracs) { fracs[o * 2] = -1.f; fracs[o * 2 + 1] = -1.f; }
+  }
+}
+cudaError_t launch_span_topk(const float* s, const float* e, const float* vmask, int B, int L, int k, float thr,
+                             int64_t* si, int64_t* ei, float* scores, float* fracs, cudaStream_t st) {
+  if (B <= 0) return cudaSuccess;
+  span_topk_kernel<<<B, kTopkThreads, 0, st>>>(s, e, vmask, L, k, thr, si, ei, scores, fracs);
+  return cudaGetLastError();
+}
+
+// R@k counters {n, #>=0.3, #>=0.5, #>=0.7} of the best IoU over each sample's filled top-k slots (start fraction >= 0).
+__global__ void topk_counters_kernel(const float* __restrict__ fracs, const float* __restrict__ gt, int B, int k,
+                                     double* __restrict__ counters) {
+  double c[4] = {0, 0, 0, 0};
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
+    const float g0 = gt[b * 2], g1 = gt[b * 2 + 1];
+    double best = 0.0;
+    for (int q = 0; q < k; ++q) {
+      const float p0 = fracs[((long long)b * k + q) * 2], p1 = fracs[((long long)b * k + q) * 2 + 1];
+      if (p0 >= 0.f) best = fmax(best, span_iou(g0, g1, p0, p1));
+    }
+    c[0] += 1.0; c[1] += best >= 0.3; c[2] += best >= 0.5; c[3] += best >= 0.7;
+  }
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) c[q] += __shfl_xor_sync(0xffffffffu, c[q], o);
+    if ((threadIdx.x & 31) == 0 && c[0] > 0) atomicAdd(counters + q, c[q]);   // integer counts: exact in any order
+  }
+}
+cudaError_t launch_topk_counters(const float* fracs, const float* gt, int B, int k, double* counters, cudaStream_t st) {
+  if (B <= 0) return cudaSuccess;
+  int blocks = (B + 255) / 256;
+  if (blocks > 148) blocks = 148;
+  topk_counters_kernel<<<blocks, 256, 0, st>>>(fracs, gt, B, k, counters);
   return cudaGetLastError();
 }
 

@@ -1005,6 +1005,27 @@ extern "C" int seqpan_iou_counters(const float* fracs, const float* gt_fracs, in
   return SEQPAN_OK;
 }
 
+extern "C" int seqpan_span_topk(const float* slogits, const float* elogits, const float* vmask, int B, int L, int k,
+                                float nms_thresh, int64_t* start_idx, int64_t* end_idx, float* scores, float* fracs,
+                                void* stream) {
+  if (!slogits || !elogits) return fail(SEQPAN_E_INVALID, "NULL logits");
+  if (!start_idx || !end_idx || !scores) return fail(SEQPAN_E_INVALID, "NULL output");
+  if (B < 0) return fail(SEQPAN_E_INVALID, "B=%d < 0", B);
+  if (L < 1 || L > SEQPAN_MAX_VLEN) return fail(SEQPAN_E_INVALID, "L=%d outside [1,%d]", L, SEQPAN_MAX_VLEN);
+  if (k < 1 || k > SEQPAN_TOPK_MAX) return fail(SEQPAN_E_INVALID, "k=%d outside [1,%d]", k, SEQPAN_TOPK_MAX);
+  if (!(nms_thresh > 0.f && nms_thresh <= 1.f)) return fail(SEQPAN_E_INVALID, "nms_thresh=%g outside (0,1]", nms_thresh);
+  CK(launch_span_topk(slogits, elogits, vmask, B, L, k, nms_thresh, start_idx, end_idx, scores, fracs, (cudaStream_t)stream));
+  return SEQPAN_OK;
+}
+
+extern "C" int seqpan_topk_counters(const float* fracs, const float* gt_fracs, int B, int k, double* counters, void* stream) {
+  if (!fracs || !gt_fracs || !counters) return fail(SEQPAN_E_INVALID, "NULL argument");
+  if (B < 0) return fail(SEQPAN_E_INVALID, "B=%d < 0", B);
+  if (k < 1 || k > SEQPAN_TOPK_MAX) return fail(SEQPAN_E_INVALID, "k=%d outside [1,%d]", k, SEQPAN_TOPK_MAX);
+  CK(launch_topk_counters(fracs, gt_fracs, B, k, counters, (cudaStream_t)stream));
+  return SEQPAN_OK;
+}
+
 // Host -> device copy of zero-padded clip features that only moves the valid prefix of every sample and writes the
 // padding rows as zeros on the device.  mode 0: one cudaMemcpyAsync per sample (copy engine) + a zero-fill kernel;
 // mode >= 1: one kernel that reads the pinned host buffer directly (zero-copy over PCIe) with `mode` CTAs.

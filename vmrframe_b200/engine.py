@@ -79,6 +79,65 @@ class IouCounters:
         return metrics_from_counters(self.buf.cpu().tolist())
 
 
+# ---- top-k retrieval metrics (R@k after temporal NMS) -------------------------------------------------------
+TOPK_THRESHOLDS = (0.3, 0.5, 0.7)
+
+
+def append_ious_topk(ious, se_gts, se_props):
+    """R@k analogue of ``append_ious``: for each sample, the best ``calculate_iou`` over its filled top-k proposals
+    (``se_props`` ``[B,k,2]`` as returned by ``infer_topk``; empty slots have a negative start) against its ground truth,
+    0 when no slot is filled."""
+    for gt, props in zip(se_gts, se_props):
+        ious.append(max((calculate_iou(gt, p) for p in props if p[0] >= 0), default=0.0))
+    return ious
+
+
+def recall_at_k(ious):
+    """``(R@k IoU>=0.3, >=0.5, >=0.7)`` in percent from the per-sample best IoUs of :func:`append_ious_topk`."""
+    return tuple(calculate_iou_accuracy(ious, t) for t in TOPK_THRESHOLDS)
+
+
+def metrics_topk_from_counters(counters):
+    """:func:`recall_at_k` from the summable counters ``[n, #>=0.3, #>=0.5, #>=0.7]``."""
+    c = [float(x) for x in counters]
+    n = max(c[0], 1.0)
+    return tuple(x / n * 100.0 for x in c[1:4])
+
+
+def _allreduce_sum(t: torch.Tensor) -> torch.Tensor:
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    return t
+
+
+class TopkCounters:
+    """Device-side R@k counters (seqpan_topk_counters) of top-``k`` spans retrieved with NMS threshold ``nms_thresh``:
+    ``[n, #>=0.3, #>=0.5, #>=0.7]`` in fp64, no sync until ``.result()``.  ``buf`` may be a caller's 4-element fp64 view."""
+
+    def __init__(self, device, k: int, nms_thresh: float = 0.5, buf: torch.Tensor | None = None):
+        self.k, self.nms_thresh = int(k), float(nms_thresh)
+        self.buf = torch.zeros(4, dtype=torch.float64, device=device) if buf is None else buf
+
+    def update(self, fracs: torch.Tensor, gt_fracs: torch.Tensor):
+        """``fracs`` ``[B,k,2]`` from :func:`infer_topk` / the top-k kernel, ``gt_fracs`` ``[B,2]``."""
+        dev = self.buf.device
+        fr = fracs.to(device=dev, dtype=torch.float32).contiguous()
+        gt = gt_fracs.to(device=dev, dtype=torch.float32).contiguous()
+        if fr.dim() != 3 or fr.shape[1] != self.k or fr.shape[2] != 2 or gt.shape != (fr.shape[0], 2):
+            raise ValueError(f"fracs must be [B,{self.k},2] and gt_fracs [B,2], got {tuple(fr.shape)} and {tuple(gt.shape)}")
+        with torch.cuda.device(dev):
+            _cabi.check(_cabi.lib().seqpan_topk_counters(fr.data_ptr(), gt.data_ptr(), fr.shape[0], self.k,
+                                                         self.buf.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
+
+    def allreduce(self):
+        _allreduce_sum(self.buf)
+        return self
+
+    def result(self):
+        return metrics_topk_from_counters(self.buf.cpu().tolist())
+
+
 # ---- sharding ---------------------------------------------------------------------------------------------
 def shard_batches(num_batches: int, rank: int, world_size: int) -> list[int]:
     """Whole reference batches, round-robin: batch k -> rank k mod world_size."""
@@ -129,7 +188,7 @@ def valid_rows_from_mask(vmask: torch.Tensor) -> torch.Tensor:
 class _Slot:
     """Device-side landing buffers of one in-flight batch (inputs, noise, outputs): allocated once per sweep."""
 
-    def __init__(self, device, B, L, V, T, C):
+    def __init__(self, device, B, L, V, T, C, topk=0):
         f32, i64 = torch.float32, torch.int64
         self.words = torch.empty(B * T, dtype=i64, device=device)
         self.chars = torch.empty(B * T * C, dtype=i64, device=device)
@@ -144,6 +203,11 @@ class _Slot:
         self.fracs = torch.empty(B * 2, dtype=f32, device=device)
         self.valid_dev = torch.empty(B, dtype=torch.int32, device=device)
         self.vindex = torch.empty(B, dtype=torch.int32, device=device)
+        if topk:
+            self.topk_si = torch.empty(B * topk, dtype=i64, device=device)
+            self.topk_ei = torch.empty(B * topk, dtype=i64, device=device)
+            self.topk_scores = torch.empty(B * topk, dtype=f32, device=device)
+            self.topk_fracs = torch.empty(B * topk * 2, dtype=f32, device=device)
         self.copied = torch.cuda.Event()      # recorded on the copy stream when the inputs have landed
         self.consumed = torch.cuda.Event()    # recorded on the compute lane when the batch is done with the slot
         self.used = False
@@ -151,7 +215,7 @@ class _Slot:
 
 def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: bool = False, streams: int = 2,
              ragged_h2d: bool = True, h2d_ctas: int = 32, profile: bool = False, check_padding: bool | None = None,
-             allreduce: bool = True):
+             allreduce: bool = True, topk: int | None = None, nms_thresh: float = 0.5):
     """Runs forward + span decode + IoU counters over an iterable of HOST batches (dicts in ``BaseCollate``'s key
     naming, ideally pinned) -- the eval loop of ``main.py:112-134`` as one pipelined call.
 
@@ -171,8 +235,17 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     ``allreduce=False`` leaves the counters rank-local (a caller that evaluates several chunks sums them and all-reduces once).
     Returns ``(metrics 5-tuple, counters tensor, info dict)``; with ``return_fracs`` the info holds all ``(B,2)``
     fractions.
+    ``topk=k`` additionally retrieves the k best spans of every sample after temporal NMS at ``nms_thresh`` (the kernel of
+    :func:`extract_topk`) on the batch's lane and accumulates R@k counters; ``info["topk"]`` then holds ``k``, ``nms_thresh``,
+    ``recall`` (R@k at IoU 0.3, 0.5, 0.7, percent) and ``counters`` (``[n, #>=0.3, #>=0.5, #>=0.7]``), and with
+    ``return_fracs`` ``info["topk_fracs"]`` holds all ``(B,k,2)`` fractions.  Both counter sets live in one fp64 buffer, so
+    the sweep still ends in a single all-reduce.
     """
     _cabi.require_device()
+    if topk is not None:
+        topk = int(topk)
+        if not (1 <= topk <= 32 and 0.0 < nms_thresh <= 1.0):
+            raise ValueError(f"topk={topk} must be in [1,32] and nms_thresh={nms_thresh} in (0,1]")
     device = torch.device(device or "cuda")
     L_ = _cabi.lib()
     import os
@@ -182,8 +255,20 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     main = torch.cuda.current_stream(device)
     nstreams = max(1, int(streams))
     counters = IouCounters(device)
+    tk = None
+    if topk is not None:   # one fp64 buffer [5 IoU counters | 4 R@k counters]: one all-reduce for both
+        joint = torch.zeros(9, dtype=torch.float64, device=device)
+        counters.buf = joint[:5]
+        tk = TopkCounters(device, topk, nms_thresh, buf=joint[5:])
+
+    def topk_info():
+        return {"k": tk.k, "nms_thresh": tk.nms_thresh, "recall": tk.result(), "counters": tk.buf}
+
     if not batches:
-        return counters.result(), counters.buf, {"h2d_bytes": 0, "d2h_bytes": 0, "wall_s": 0.0, "batches": 0}
+        info = {"h2d_bytes": 0, "d2h_bytes": 0, "wall_s": 0.0, "batches": 0}
+        if tk is not None:
+            info["topk"] = topk_info()
+        return counters.result(), counters.buf, info
     lanes = [main] + [torch.cuda.Stream(device) for _ in range(nstreams - 1)]
     copy_stream = torch.cuda.Stream(device)
     depth = max(1, int(depth))
@@ -195,7 +280,7 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     if hasattr(model, "set_side_stream"):
         model.set_side_stream(False)      # the sweep is bound by its own host->device copy kernel (include/seqpan_b200.h)
     with torch.cuda.device(device):
-        slots = [_Slot(device, Bm, Lv, V, Tm, Cm) for _ in range(min(depth + nstreams, len(batches)))]
+        slots = [_Slot(device, Bm, Lv, V, Tm, Cm, topk or 0) for _ in range(min(depth + nstreams, len(batches)))]
         # every kernel context is sized for the largest batch of the sweep up front (no handle re-creation / weight
         # re-packing in the middle of it)
         for k in range(nstreams):
@@ -207,6 +292,7 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
         copy_stream.wait_event(ready)
     host_fracs = torch.empty(len(batches), Bm, 2, dtype=torch.float32, pin_memory=True)
     valid_host = torch.empty(len(batches), Bm, dtype=torch.int32, pin_memory=True)   # one row per batch: never rewritten
+    host_topk = torch.empty(len(batches), Bm, topk, 2, dtype=torch.float32, pin_memory=True) if tk is not None and return_fracs else None
     h2d = d2h = 0
     views = {}
     prof = []   # profile=True: (copy start, copy end, compute start, compute end) events per batch
@@ -225,6 +311,9 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
              "gumbel": sl.gumbel[: B * Lv * 4].view(B, Lv, 4), "slogits": sl.slogits[: B * Lv].view(B, Lv),
              "elogits": sl.elogits[: B * Lv].view(B, Lv), "match": sl.match[: B * Lv * 4].view(B, Lv, 4),
              "fracs": sl.fracs[: B * 2].view(B, 2)}
+        if tk is not None:
+            v.update(topk_si=sl.topk_si[: B * topk], topk_ei=sl.topk_ei[: B * topk], topk_scores=sl.topk_scores[: B * topk],
+                     topk_fracs=sl.topk_fracs[: B * topk * 2].view(B, topk, 2))
         views[i] = v
         with torch.cuda.stream(copy_stream):
             if sl.used:
@@ -294,6 +383,17 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                                                            counters.buf.data_ptr(), st))
                     host_fracs[i, :B].copy_(v["fracs"], non_blocking=True)     # device -> host read of the step's result
                     d2h += B * 2 * 4
+                    if tk is not None:
+                        _cabi.check(L_.seqpan_span_topk(v["slogits"].data_ptr(), v["elogits"].data_ptr(), v["vmask"].data_ptr(),
+                                                        B, Lv, topk, tk.nms_thresh, v["topk_si"].data_ptr(),
+                                                        v["topk_ei"].data_ptr(), v["topk_scores"].data_ptr(),
+                                                        v["topk_fracs"].data_ptr(), st))
+                        if v["gt"] is not None:
+                            _cabi.check(L_.seqpan_topk_counters(v["topk_fracs"].data_ptr(), v["gt"].data_ptr(), B, topk,
+                                                                tk.buf.data_ptr(), st))
+                        if host_topk is not None:
+                            host_topk[i, :B].copy_(v["topk_fracs"], non_blocking=True)
+                            d2h += B * topk * 2 * 4
                     sl.consumed.record(lane)
                     if profile:
                         prof[i][3].record(lane)
@@ -304,20 +404,28 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                 e.record(ln)
                 main.wait_event(e)
             if allreduce:
-                counters.allreduce()
+                if tk is None:
+                    counters.allreduce()
+                else:
+                    _allreduce_sum(joint)
             metrics = counters.result()  # synchronises
     finally:
         model.use_context(was_ctx)
         model.sync_timing = was_sync
         if hasattr(model, "set_side_stream"):
             model.set_side_stream(was_side)
-    info = {"h2d_bytes": h2d, "d2h_bytes": d2h + 40, "wall_s": time.time() - t0, "batches": len(batches)}
+    info = {"h2d_bytes": h2d, "d2h_bytes": d2h + (40 if tk is None else 72), "wall_s": time.time() - t0,
+            "batches": len(batches)}
+    if tk is not None:
+        info["topk"] = topk_info()
     if profile:
         info["copy_ms"] = [p[0].elapsed_time(p[1]) for p in prof]
         info["compute_ms"] = [p[2].elapsed_time(p[3]) for p in prof]
         info["copy_to_compute_start_ms"] = [prof[0][0].elapsed_time(p[2]) for p in prof]
     if return_fracs:  # counters.result() above synchronised the device, so the pinned buffer is complete
         info["fracs"] = [host_fracs[i, : b["vmasks"].shape[0]].numpy().copy() for i, b in enumerate(batches)]
+        if host_topk is not None:
+            info["topk_fracs"] = [host_topk[i, : b["vmasks"].shape[0]].numpy().copy() for i, b in enumerate(batches)]
     return metrics, counters.buf, info
 
 

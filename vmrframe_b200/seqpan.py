@@ -618,6 +618,44 @@ def infer_basic_device(start_logits, end_logits, vmask):
     return _decode(start_logits, end_logits, vmask, False, True)[2]
 
 
+def _topk(start_logits, end_logits, vmask, k, nms_thresh, want_fracs):
+    _cabi.require_device()
+    if not start_logits.is_cuda:
+        raise _cabi.SeqpanError("top-k span retrieval needs CUDA tensors (no CPU path)")
+    s = start_logits.detach().to(torch.float32).contiguous()
+    e = end_logits.detach().to(torch.float32).contiguous()
+    B, L = s.shape
+    dev = s.device
+    vm = vmask.detach().to(device=dev, dtype=torch.float32).contiguous() if vmask is not None else None
+    k = int(k)
+    si = torch.empty(B, max(k, 0), dtype=torch.int64, device=dev)
+    ei = torch.empty_like(si)
+    sc = torch.empty(B, max(k, 0), dtype=torch.float32, device=dev)
+    fr = torch.empty(B, max(k, 0), 2, dtype=torch.float32, device=dev) if want_fracs else None
+    with torch.cuda.device(dev):
+        _cabi.check(_cabi.lib().seqpan_span_topk(
+            s.data_ptr(), e.data_ptr(), vm.data_ptr() if vm is not None else None, B, L, k, float(nms_thresh),
+            si.data_ptr(), ei.data_ptr(), sc.data_ptr(), fr.data_ptr() if fr is not None else None,
+            torch.cuda.current_stream(dev).cuda_stream))
+    return si, ei, sc, fr
+
+
+def extract_topk(start_logits, end_logits, vmask=None, k: int = 5, nms_thresh: float = 0.5):
+    """The ``k`` best spans of every sample after greedy temporal NMS, as device tensors ``(start_idx, end_idx, scores)`` of
+    shape ``[B,k]`` (int64, int64, fp32) in selection order.  Scores are ``sp[i] * ep[j]`` with ``infer_basic``'s
+    probabilities (``mask_logits`` first when ``vmask`` is given); a candidate whose IoU with a kept span is at least
+    ``nms_thresh`` is suppressed (``nms_thresh=1``: plain top-k).  Slots past the last surviving candidate hold ``-1, -1, 0``.
+    At ``k=1`` the start equals :func:`extract_index`'s; the end too unless the best score is attained by several spans."""
+    si, ei, sc, _ = _topk(start_logits, end_logits, vmask, k, nms_thresh, False)
+    return si, ei, sc
+
+
+def infer_topk(output, k: int = 5, nms_thresh: float = 0.5):
+    """Top-k counterpart of ``infer_SeqPAN`` for the output dict of any of the five models: ``np.ndarray float32 (B,k,2)`` of
+    span fractions (indices divided by ``vmask.sum(1)``) in selection order; empty slots are ``-1``."""
+    return _topk(output["slogits"], output["elogits"], output["vmask"], k, nms_thresh, True)[3].cpu().numpy()
+
+
 class BaseFast(SeqPAN):
     """Drop-in for the reference's ``models/BaseFast.py:10-97`` (SURVEY.md section 8 row f3): the same blocks as SeqPAN with a
     2-layer shared ``FeatureEncoder`` (``:27``) and without the two ``DualAttentionBlock`` passes (``:62-68`` are commented
