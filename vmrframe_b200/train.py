@@ -25,7 +25,10 @@ and fp32 accumulation, and keeps everything else fp32.
 """
 from __future__ import annotations
 
+import collections
+import contextlib
 import ctypes as C
+import gc
 import math
 
 import torch
@@ -35,6 +38,27 @@ from . import _cabi
 D, H, HD = 128, 4, 32
 MASKV = -1e30
 PRECISIONS = ("fp32", "bf16")      # training precision modes (see SeqpanTape)
+# Input shapes a TrainStep keeps as CUDA graphs, least recently used evicted first; shared by TrainStep.step, the train engines
+# and model(...) in train().  Each captured shape holds its activations in a graph pool (DESIGN.md section 10 gives the measured
+# size per shape).
+GRAPH_CACHE_SIZE = 16
+
+
+@contextlib.contextmanager
+def _capture(graph, pool=None):
+    """``torch.cuda.graph`` with the cyclic garbage collector off.  A collection during a capture may destroy the graphs of a
+    dead model (a model and its ``TrainStep`` form a cycle), a call that is illegal while a stream captures and that would
+    invalidate the capture; so pending garbage is collected first."""
+    was = gc.isenabled()
+    torch.cuda.synchronize()
+    gc.collect()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph, pool=pool):
+            yield
+    finally:
+        if was:
+            gc.enable()
 
 
 def _check_precision(precision):
@@ -71,6 +95,7 @@ def _pad4(vals, fill):
 class CudaBackend:
     """Thin tensor-level wrappers of the ``seqpan_t_*`` kernels.  Operands may be strided views (transposes, head splits
     and broadcasts are stride tricks, never copies)."""
+    graph_safe = True       # every call is a stream-ordered launch with no host synchronisation: a tape on it can be captured
 
     def __init__(self, device):
         _cabi.require_device()
@@ -1046,8 +1071,8 @@ class TrainStep:
         self.runtype = "train"                # MultiTeacher: the teacher terms enter the loss for runtype "train" only
         self.flat = None
         self.dyn = None                      # device float[3]: lr, 1 - beta1^t, sqrt(1 - beta2^t) of the current step
-        self._graphs = {}
-        self.max_graphs = 8                  # input shapes replayed as CUDA graphs (each holds its activations' memory pool)
+        self._graphs = collections.OrderedDict()     # graph key -> entry, least recently used first
+        self.max_graphs = GRAPH_CACHE_SIZE           # captured entries kept (each holds its activations' memory pool)
         self._g2 = {}                        # deterministic mode -> the clip + AdamW half: {"seen", "graph", "out"}
         self.views = {}
 
@@ -1087,13 +1112,15 @@ class TrainStep:
         lr = self._lr_now() if self.total > 1 else self.lr
         return [lr, 1.0 - 0.9 ** self.t, math.sqrt(1.0 - 0.999 ** self.t)]
 
-    def _part1(self, data, gumbel):
-        """Forward + losses + backward; the live gradients land in ONE flat bucket (``self.flat``)."""
+    def _part1(self, data, gumbel, relayout=False):
+        """Forward + losses + backward; the live gradients land in ONE flat bucket (``self.flat``).  ``relayout``: a changed set
+        of live gradients gets a new bucket instead of an error (the train engines, where parameters may be frozen between
+        steps; every captured graph keeps the bucket it writes in its entry)."""
         be = self.be
         loss, grads, out = self.loss_and_grads(data, gumbel)
         names = sorted(grads)
-        if self.live is None:
-            self.live = names
+        if self.live is None or (relayout and names != self.live):
+            self.live, self.views = names, {}
             self.flat = be.zeros((sum(grads[k].numel() for k in names),))
             off = 0
             for k in names:
@@ -1136,13 +1163,80 @@ class TrainStep:
             be.adamw(p.data, self.views[k], self.m[k], self.v[k], hp, ss, self.dyn)
         return ss
 
+    # -- CUDA graphs of forward + losses + backward, one per graph key, least recently used evicted first --
+    def _graph_key(self, route, data, gumbel, precision, *extra):
+        """Everything a captured forward + backward bakes in: the route, the input shapes and dtypes, whether a Gumbel draw is
+        given, the deterministic mode, the precision, ``model.training`` and its droprate, and for every parameter whether it
+        requires grad and where its storage is (a re-created parameter must not replay a graph that reads the old one)."""
+        m = self.model
+        return ((route,) + tuple((k, tuple(v.shape), v.dtype) for k, v in sorted(data.items()))
+                + (gumbel is not None, deterministic_mode(), precision, m.training, float(m.configs.model.droprate))
+                + tuple((k, p.requires_grad, p.data_ptr()) for k, p in self.named.items()) + extra)
+
+    def _entry(self, key):
+        """The cache entry of ``key`` (``{"seen": eager runs}`` at first), moved to the most recently used end."""
+        ent = self._graphs.pop(key, None)
+        self._graphs[key] = ent = ent if ent is not None else {"seen": 0}
+        return ent
+
+    def _use_graph(self, ent):
+        """Whether ``ent`` replays (and is captured first if need be): after two eager runs, and when a capture fits.  At most
+        ``max_graphs`` entries hold graphs; the least recently used one without a forward in flight gives its graphs and pool
+        up (its eager count stays).  When every capture holds a forward in flight the call runs eagerly."""
+        if "graph" in ent:
+            return True
+        if ent["seen"] < 2:
+            return False
+        captured = [e for e in self._graphs.values() if "graph" in e]
+        while len(captured) >= self.max_graphs:
+            old = next((e for e in captured if not e.get("busy")), None)
+            if old is None:
+                return False
+            captured.remove(old)
+            for k in [k for k in old if k != "seen"]:
+                del old[k]
+        return True
+
+    def _replay_part1(self, ent, data, gumbel, relayout=False):
+        """``_part1`` from the entry's graph, captured on first use.  Inputs are copied into static buffers; the dropout / Gumbel
+        draws stay fresh (torch's graph-safe generator).  The entry keeps the bucket its graph writes."""
+        if "graph" not in ent:
+            ent["in"] = {k: v.clone() for k, v in data.items()}
+            ent["gum"] = gumbel.clone() if gumbel is not None else None
+            g = torch.cuda.CUDAGraph()
+            with _capture(g):
+                ent["out"] = self._part1(ent["in"], ent["gum"], relayout)
+            ent["bucket"] = (self.flat, self.live)
+            ent["graph"] = g
+        for k, v in data.items():
+            ent["in"][k].copy_(v, non_blocking=True)
+        if gumbel is not None:
+            ent["gum"].copy_(gumbel, non_blocking=True)
+        ent["graph"].replay()
+        return ent["out"]
+
+    def _engine_loss_and_grads(self, data, gumbel):
+        """``loss_and_grads`` of the train engines, replayed from a CUDA graph from the third call with the same key on.  A
+        replay hands out views of a fresh copy of the entry's bucket and fresh copies of the outputs: they outlive the next
+        replay, so gradients of two calls can be accumulated before one backward."""
+        ent = self._entry(self._graph_key("loss", data, gumbel, self.precision, self.runtype))
+        if not self._use_graph(ent):
+            ent["seen"] += 1
+            return self.loss_and_grads(data, gumbel)
+        loss, out = self._replay_part1(ent, data, gumbel, relayout=True)
+        flat, live = ent["bucket"]
+        grads = dict(zip(live, flat.clone().split([self.named[k].numel() for k in live])))
+        out = {k: (v.clone() if k in ("slogits", "elogits", "match_score") else v) for k, v in out.items()}
+        out["vmask"] = data["vmasks"]
+        return loss, grads, out
+
     def step(self, data, gumbel=None, graph=False):
         """One optimisation step.  ``graph=True`` replays the two device halves of the step (forward + backward into the bucket;
         clip + AdamW) as CUDA graphs after two eager steps per input shape: the tape issues ~1200 small launches from Python,
         which is host-bound; the graphs keep the same kernels and remove the host.  Inputs are copied into static buffers, the
         dropout / Gumbel draws stay fresh (torch's graph-safe generator), the gradient all-reduce stays an eager call between
-        the two graphs.  Graphs are kept per deterministic mode (:func:`deterministic_mode`): a graph captured in one mode never
-        replays in the other."""
+        the two graphs.  Graphs are kept per key (:meth:`_graph_key`: shapes, deterministic mode, precision, parameters), at
+        most ``max_graphs`` of them, least recently used evicted first."""
         be = self.be
         det = deterministic_mode()
         self.t += 1
@@ -1160,29 +1254,12 @@ class TrainStep:
             world = self._allreduce()
             ss = self._part2(world, det)
         else:
-            key = tuple((k, tuple(v.shape)) for k, v in sorted(data.items())) + (gumbel is not None, det)
-            ent = self._graphs.setdefault(key, {"seen": 0})
-            # every captured shape keeps its own pool of intermediates alive: at most `max_graphs` shapes are captured (the most
-            # frequent ones arrive first in practice), the rest run from the tape
-            full = "graph" not in ent and sum("graph" in e for e in self._graphs.values()) >= self.max_graphs
-            if ent["seen"] < 2 or full:                    # two eager steps first: lazy state (Adam moments, bucket, caches) exists
+            ent = self._entry(self._graph_key("step", data, gumbel, self.precision, self.runtype))
+            if not self._use_graph(ent):                   # two eager steps first: lazy state (Adam moments, bucket, caches) exists
                 ent["seen"] += 1
                 loss, out = self._part1(data, gumbel)
             else:
-                if "graph" not in ent:
-                    ent["in"] = {k: v.clone() for k, v in data.items()}
-                    ent["gum"] = gumbel.clone() if gumbel is not None else None
-                    torch.cuda.synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        ent["out"] = self._part1(ent["in"], ent["gum"])
-                    ent["graph"] = g
-                for k, v in data.items():
-                    ent["in"][k].copy_(v, non_blocking=True)
-                if gumbel is not None:
-                    ent["gum"].copy_(gumbel, non_blocking=True)
-                ent["graph"].replay()
-                loss, out = ent["out"]
+                loss, out = self._replay_part1(ent, data, gumbel)
             world = self._allreduce()
             e2 = self._g2.setdefault(det, {"seen": 0})
             if "graph" not in e2 and e2["seen"] < 2:
@@ -1190,9 +1267,8 @@ class TrainStep:
                 ss = self._part2(world, det)
             else:
                 if "graph" not in e2:
-                    torch.cuda.synchronize()
                     g2 = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g2):
+                    with _capture(g2):
                         e2["out"] = self._part2(world, det)
                     e2["graph"] = g2
                 e2["graph"].replay()
@@ -1221,16 +1297,35 @@ class _TapeLoss(torch.autograd.Function):
 def tape_loss(model, data, gumbel=None, mask_fn=None, runtype="train"):
     """Training forward + the model's loss terms + backward on the kernels; returns ``(loss, output)`` where ``loss`` is a scalar
     tensor attached to the module's parameters (``loss.backward()`` fills ``p.grad``).  ``runtype`` is the train engines' fourth
-    argument (only MultiTeacher reads it: its teacher terms exist for "train")."""
+    argument (only MultiTeacher reads it: its teacher terms exist for "train").
+
+    From the third call with the same key (:meth:`TrainStep._graph_key`) on, forward, losses and backward replay as one CUDA
+    graph from the model's ``TrainStep`` cache; never with ``mask_fn`` or off the CUDA kernels."""
+    ts = _train_step_of(model)
+    named = dict(model.named_parameters())
+    ts.named, ts.mask_fn, ts.runtype = named, mask_fn, runtype
+    if _can_capture(ts.be, data["vfeats"], mask_fn):
+        value, grads, out = ts._engine_loss_and_grads(data, gumbel)
+    else:
+        value, grads, out = ts.loss_and_grads(data, gumbel)
+    params = [p for p in named.values() if p.requires_grad]
+    glist = [grads[k].reshape(p.shape) if k in grads else None for k, p in named.items() if p.requires_grad]
+    return _TapeLoss.apply(value, glist, *params), out
+
+
+def _train_step_of(model):
+    """The ``TrainStep`` the drop-in routes share per model: its graph cache and bound serve both."""
     ts = getattr(model, "_train_step", None)
     if ts is None:
         ts = model._train_step = TrainStep(model)
-    ts.mask_fn, ts.runtype = mask_fn, runtype
-    value, grads, out = ts.loss_and_grads(data, gumbel)
-    names = [k for k, p in model.named_parameters() if p.requires_grad]
-    params = [dict(model.named_parameters())[k] for k in names]
-    glist = [grads[k].reshape(p.shape) if k in grads else None for k, p in zip(names, params)]
-    return _TapeLoss.apply(value, glist, *params), out
+    return ts
+
+
+def _can_capture(be, x, mask_fn=None):
+    """Whether a drop-in route may capture and replay: the CUDA kernels on a CUDA tensor, no injected dropout masks (a
+    ``mask_fn`` hands in host-made draws) and no capture of the caller's already under way."""
+    return (getattr(be, "graph_safe", False) and x.is_cuda and mask_fn is None
+            and not torch.cuda.is_current_stream_capturing())
 
 
 # ---- the training forward as one torch autograd node: any torch loss on its outputs backpropagates through the tape ----------
@@ -1250,6 +1345,63 @@ class _Recording:
         self.tp.nodes = []
 
 
+class _InFlight:
+    """Marks a graph entry's forward as in flight while the node that replayed it can still be backpropagated: a forward of
+    the same key meanwhile runs on the eager tape, since a replay would overwrite the activations this backward reads."""
+    __slots__ = ("ent",)
+
+    def __init__(self, ent):
+        self.ent = ent
+        ent["busy"] = True
+
+    def __del__(self):
+        self.ent["busy"] = False
+
+
+def _capture_node_forward(ent, model, be, inputs, gumbel, named, needs_x):
+    """Record the training forward of the node inside a CUDA graph; the tape, its nodes and the static inputs stay with
+    the entry, so that backward graphs can be captured from the same recording."""
+    ent["in"] = [t.detach().clone() for t in inputs]
+    ent["gum"] = gumbel.clone() if gumbel is not None else None
+    g = torch.cuda.CUDAGraph()
+    with _capture(g):
+        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model),
+                        deterministic=deterministic_mode())
+        P = _Params(tp, named)
+        w, c, vm, tm, x = ent["in"]
+        xv = tp.leaf(x, needs=needs_x)
+        outs = [o for o in forward_train(tp, P, w, c, xv, vm, tm, ent["gum"], **train_spec(model)["fwd"]) if o is not None]
+    ent.update(graph=g, rec=_Recording(tp, outs, xv, P), nodes=list(tp.nodes), bwd={})
+
+
+def _graphed_node_backward(ent, gouts, names):
+    """The node's backward from a graph per pattern of cotangents (which are None): the backward issues different kernels for
+    each.  A graph is captured from the entry's recording on first use, in the forward graph's pool.  Cotangents are copied
+    into static buffers (which makes expanded views contiguous); the gradients handed back are fresh copies."""
+    bkey = tuple(g is not None for g in gouts)
+    if bkey not in ent["bwd"]:
+        rec = ent["rec"]
+        static = [None if g is None else torch.empty(g.shape, dtype=torch.float32, device=g.device) for g in gouts]
+        for o, inputs, _ in ent["nodes"]:            # the gradient state an earlier capture left on the tape's Vars
+            for v in (o, *inputs):
+                v.g, v.own = None, False
+        rec.tp.nodes = list(ent["nodes"])
+        gb = torch.cuda.CUDAGraph()
+        with _capture(gb, pool=ent["graph"].pool()):
+            rec.tp.backward(list(zip(rec.outs, static)))
+            grads = [rec.xv.g] + [rec.P[k].g for k in names]
+            for k in _EMB_PAD_ROW:
+                if k in rec.P.vars and rec.P[k].g is not None:
+                    rec.P[k].g[0].zero_()
+        ent["bwd"][bkey] = (gb, static, grads)
+    gb, static, grads = ent["bwd"][bkey]
+    for s, g in zip(static, gouts):
+        if s is not None:
+            s.copy_(g)
+    gb.replay()
+    return [g.clone() if g is not None else None for g in grads]
+
+
 class _TapeForward(torch.autograd.Function):
     """Forward: the training forward recorded on a ``SeqpanTape`` (kept on ``ctx``).  Backward: the tape's adjoints from the
     cotangents of ``slogits`` / ``elogits`` / ``match_score`` that autograd hands in, one gradient per parameter and for
@@ -1257,18 +1409,36 @@ class _TapeForward(torch.autograd.Function):
 
     The outputs are fresh views of the tape's tensors, never the tensors the tape (and so ``ctx``) holds: a returned tensor
     reachable from ``ctx`` would close the cycle output -> grad_fn -> ctx -> output, and a forward dropped without a backward
-    would keep its whole tape alive until a full garbage collection."""
+    would keep its whole tape alive until a full garbage collection.
+
+    ``slot``: None, or ``(entry, graphed)`` of the model's graph cache.  Graphed, the forward replays the entry's graph and
+    returns copies of its outputs, and the backward replays a backward graph; eager, a completed backward counts towards the
+    entry's capture."""
 
     @staticmethod
-    def forward(ctx, model, be, word_ids, char_ids, vmask, tmask, gumbel, vfeat_in, names, *params):
+    def forward(ctx, model, be, slot, word_ids, char_ids, vmask, tmask, gumbel, vfeat_in, names, *params):
         ctx.set_materialize_grads(False)          # an output nobody used arrives as None and costs nothing
+        ctx.names, ctx.shapes = names, [p.shape for p in params]
+        ent, graphed = slot if slot is not None else (None, False)
+        ctx.ent = ent
+        if graphed:
+            if "graph" not in ent:
+                _capture_node_forward(ent, model, be, (word_ids, char_ids, vmask, tmask, vfeat_in), gumbel,
+                                      dict(zip(names, params)), ctx.needs_input_grad[8])
+            for s, t in zip(ent["in"], (word_ids, char_ids, vmask, tmask, vfeat_in)):
+                s.copy_(t, non_blocking=True)
+            if gumbel is not None:
+                ent["gum"].copy_(gumbel, non_blocking=True)
+            ent["graph"].replay()
+            ctx.rec = _InFlight(ent)
+            return tuple(o.v.clone() for o in ent["rec"].outs)
         tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model),
                         deterministic=deterministic_mode())
         P = _Params(tp, dict(zip(names, params)))
-        xv = tp.leaf(vfeat_in, needs=ctx.needs_input_grad[7])
+        xv = tp.leaf(vfeat_in, needs=ctx.needs_input_grad[8])
         outs = [o for o in forward_train(tp, P, word_ids, char_ids, xv, vmask, tmask, gumbel, **train_spec(model)["fwd"])
                 if o is not None]
-        ctx.rec, ctx.names, ctx.shapes = _Recording(tp, outs, xv, P), names, [p.shape for p in params]
+        ctx.rec = _Recording(tp, outs, xv, P)
         return tuple(o.v.view_as(o.v) for o in outs)
 
     @staticmethod
@@ -1279,6 +1449,10 @@ class _TapeForward(torch.autograd.Function):
             raise RuntimeError("backward through the SeqPAN training forward a second time: the tape is freed by the first "
                                "backward (retain_graph is not supported); run the forward again")
         ctx.rec = None
+        if isinstance(rec, _InFlight):
+            grads = _graphed_node_backward(rec.ent, gouts, ctx.names)
+            res = [g.reshape(shape) if g is not None else None for g, shape in zip(grads, [rec.ent["in"][4].shape] + ctx.shapes)]
+            return (None,) * 8 + tuple(res[:1]) + (None,) + tuple(res[1:])
         be = rec.tp.be
         gouts = [g if g is None or g.is_contiguous() else be.ewise("COPY", g) for g in gouts]   # e.g. .sum()'s expanded views
         rec.tp.backward(list(zip(rec.outs, gouts)))
@@ -1299,7 +1473,9 @@ class _TapeForward(torch.autograd.Function):
                 taken.add(g.untyped_storage().data_ptr())
                 g = g.reshape(shape)
             res.append(g)
-        return (None,) * 7 + tuple(res[:1]) + (None,) + tuple(res[1:])
+        if ctx.ent is not None:
+            ctx.ent["seen"] += 1                  # one more eager forward + backward of this key
+        return (None,) * 8 + tuple(res[:1]) + (None,) + tuple(res[1:])
 
 
 def forward_differentiable(model, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel=None, backend=None):
@@ -1307,11 +1483,22 @@ def forward_differentiable(model, word_ids, char_ids, vfeat_in, vmask, tmask, gu
     None)`` attached to every parameter that requires grad and to ``vfeat_in`` when it does, so that ``loss.backward()`` of any
     torch loss on them fills ``p.grad`` / ``vfeat_in.grad`` through the training kernels.  The same kernels, in the same order,
     with the same dropout and Gumbel draws as :func:`forward_only`: the values are bit-identical.  ``backend`` defaults to the
-    CUDA kernels of ``vfeat_in``'s device."""
+    CUDA kernels of ``vfeat_in``'s device.
+
+    With the default backend the node replays CUDA graphs from the model's ``TrainStep`` cache once its key (shapes, modes,
+    parameters, whether ``vfeat_in`` requires grad) has completed forward and backward eagerly twice: one forward graph, and a
+    backward graph per pattern of unused outputs.  While a replayed forward awaits its backward, the same key runs eagerly."""
     be = backend if backend is not None else CudaBackend(vfeat_in.device)
-    names, params = zip(*model.named_parameters())
-    outs = _TapeForward.apply(model, be, word_ids, char_ids, vmask.to(torch.float32), tmask.to(torch.float32), gumbel,
-                              vfeat_in.to(torch.float32), names, *params)
+    named = dict(model.named_parameters())
+    vm, tm, x = vmask.to(torch.float32), tmask.to(torch.float32), vfeat_in.to(torch.float32)
+    slot = None
+    if backend is None and _can_capture(be, x):
+        ts = _train_step_of(model)
+        ts.named = named
+        data = {"words_ids": word_ids, "char_ids": char_ids, "vmasks": vm, "tmasks": tm, "vfeats": x}
+        ent = ts._entry(ts._graph_key("node", data, gumbel, train_precision(model), x.requires_grad and torch.is_grad_enabled()))
+        slot = (ent, not ent.get("busy") and ts._use_graph(ent))
+    outs = _TapeForward.apply(model, be, slot, word_ids, char_ids, vm, tm, gumbel, x, tuple(named), *named.values())
     return outs if len(outs) == 3 else (outs[0], outs[1], None)
 
 
