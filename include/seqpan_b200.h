@@ -138,6 +138,23 @@ int seqpan_forward_shared_video(SeqpanHandle* h, const int64_t* word_ids, const 
                                 float* elogits, float* match_score, void* workspace, size_t workspace_bytes,
                                 void* stream);
 
+/* The query-independent video branch on its own (DESIGN.md section 12): VisualProjection + the video half of the shared
+ * FeatureEncoder (2 layers for BaseFast / MultiTeacher, 4 otherwise) of U clips vfeat [U,vlen,vdim] fp32 -> venc
+ * [U,vlen,128] fp32, the caller's buffer.  1 <= U <= max_batch (the workspace holds max_batch*vlen rows).  vfeat and venc
+ * must be 16-byte aligned (TMA and float4 access; every cudaMalloc'ed or torch tensor start is).  A clip's rows do
+ * not depend on the other clips of the call.  The encodings stay valid for this handle's weights and precision. */
+int seqpan_encode_videos(SeqpanHandle* h, const float* vfeat, int U, float* venc, void* workspace, size_t workspace_bytes,
+                         void* stream);
+
+/* seqpan_forward_shared_video on stored encodings: venc [U,vlen,128] from seqpan_encode_videos, video_index [B] int32
+ * (device) names the clip of pair b; out-of-range indices are clamped.  venc must be 16-byte aligned (float4 reads).  U is the size of the caller's encoding library and
+ * is not bounded by B; video_index == NULL pairs b with row block b (requires U >= B).  The outputs are bit-identical to
+ * seqpan_forward_shared_video on the raw clips.  Debug tap "video_affine" does not exist on this path. */
+int seqpan_forward_encoded(SeqpanHandle* h, const int64_t* word_ids, const int64_t* char_ids, const float* venc,
+                           const int32_t* video_index, int U, const float* vmask, const float* tmask, const float* gumbel,
+                           int B, int T, int C, float* slogits, float* elogits, float* match_score, void* workspace,
+                           size_t workspace_bytes, void* stream);
+
 /* Span decode.  vmask != NULL: infer_basic (mask_logits, softmax, triu outer-product argmax, indices
  * divided by vmask.sum(1)) -> fracs [B,2] fp32.  vmask == NULL: extract_index.  start_idx/end_idx
  * [B] int64 and fracs may each be NULL.  Ties resolve to the lowest index (torch CPU behaviour). */

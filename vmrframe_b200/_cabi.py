@@ -71,6 +71,8 @@ SIGNATURES = {
     "seqpan_destroy": (None, [_vp]),
     "seqpan_forward": (_i, [_vp] + [_vp] * 6 + [_i, _i, _i] + [_vp] * 3 + [_vp, _sz, _vp]),
     "seqpan_forward_shared_video": (_i, [_vp] + [_vp] * 4 + [_i] + [_vp] * 3 + [_i, _i, _i] + [_vp] * 3 + [_vp, _sz, _vp]),
+    "seqpan_encode_videos": (_i, [_vp, _vp, _i, _vp, _vp, _sz, _vp]),
+    "seqpan_forward_encoded": (_i, [_vp] + [_vp] * 4 + [_i] + [_vp] * 3 + [_i, _i, _i] + [_vp] * 3 + [_vp, _sz, _vp]),
     "seqpan_span_decode": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "seqpan_iou_counters": (_i, [_vp, _vp, _i, _vp, _vp]),
     "seqpan_span_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, C.c_float, _vp, _vp, _vp, _vp, _vp]),

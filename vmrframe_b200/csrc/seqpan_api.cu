@@ -167,7 +167,7 @@ static void carve_workspace(Carver& c, const SeqpanShapes& s, int B, int T, Work
 // One captured forward: every argument that is baked into the kernel nodes (pointers, shapes) is part of the key.
 struct GraphKey {
   const void* p[11];
-  int B, T, C, U, side;
+  int B, T, C, U, side, mode;   // mode: FWD_RAW / FWD_SHARED / FWD_ENCODED (the same pointers may serve two of them)
   bool operator<(const GraphKey& o) const { return memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 struct GraphEntry { cudaGraphExec_t exec; int launches; unsigned long long last_use; };
@@ -183,6 +183,7 @@ struct SeqpanHandle {
   std::vector<float> hostw[W_COUNT];
   float dab_fold_host[2][512];        // host mirror of DabPacked::fold_b
   int lastB = 0, lastT = 0;
+  bool last_encoded = false;          // the last forward read stored encodings (no "video_affine" tap)
   // CUDA graphs: a forward whose arguments (pointers + shapes) were seen before is replayed as ONE graph launch instead of
   // 18+ kernel launches and ~40 tensor-map encodes (static ring buffers of the eval sweep, bench.py's resident batches, and
   // in practice torch's caching allocator hand the same pointers back).  Captured on the handle's own stream (the caller's
@@ -288,13 +289,14 @@ __global__ void bil_bias_kernel(const float* __restrict__ b1, const float* __res
 }
 
 // dst[b*L + l][:] = src[index[b]*L + l][:] -- expands the encoded rows of U unique clips to the B pairs that share them
-// (SURVEY.md section 8 (f1): VisualProjection + FeatureEncoder(video) do not depend on the query, models/SeqPAN.py:57,59)
+// (SURVEY.md section 8 (f1): VisualProjection + FeatureEncoder(video) do not depend on the query, models/SeqPAN.py:57,59).
+// index == nullptr: pair b reads clip b (the caller guarantees B <= U).
 __global__ void __launch_bounds__(256) gather_clips_kernel(const float* __restrict__ src, const int32_t* __restrict__ index,
                                                            float* __restrict__ dst, int L, int U, long long rows) {
   const long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (r >= rows) return;
   const int b = (int)(r / L), l = (int)(r % L);
-  const int u = min(max(__ldg(index + b), 0), U - 1);
+  const int u = min(max(index ? __ldg(index + b) : b, 0), U - 1);
   const int lane = threadIdx.x & 31;
   reinterpret_cast<float4*>(dst + r * SQ_D)[lane] = __ldg(reinterpret_cast<const float4*>(src + ((long long)u * L + l) * SQ_D) + lane);
 }
@@ -506,6 +508,8 @@ extern "C" int seqpan_profile_summary(SeqpanHandle* h, char* buf, size_t cap) {
 }
 
 // ---- forward -----------------------------------------------------------------------------------------
+enum { FWD_RAW = 0, FWD_SHARED = 1, FWD_ENCODED = 2 };   // what `vfeat` of forward_impl holds: [B,L,V], [U,L,V] or [U,L,128]
+
 namespace {
 
 struct Fwd {
@@ -709,7 +713,8 @@ struct Fwd {
 
   const int64_t* word_ids; const int64_t* char_ids; const float* vfeat; const float* vmask; const float* tmask;
   const float* gumbel; float* slogits; float* elogits; float* match_score;
-  const int32_t* video_index = nullptr;   // != nullptr: vfeat holds U unique clips, video_index[b] = clip of pair b
+  const int32_t* video_index = nullptr;   // != nullptr: vfeat (or venc) holds U unique clips, video_index[b] = clip of pair b
+  const float* venc = nullptr;            // != nullptr: stored encodings [U,L,128] of seqpan_encode_videos instead of vfeat
   int U = 0;
 
   int run() {
@@ -720,7 +725,7 @@ struct Fwd {
       LAUNCH(h, launch_build_rowmask(vmask, Mv, tmask, Mt, ws.rowmask, st));
     // text embedding (models/layers.py:87-93) -> rows [Mv, M) of x; on the side stream, concurrently with the video affine
     cudaStream_t main_st = st;
-    const bool fork = h->side && h->use_side && !h->profile && !h->debug && !video_index;
+    const bool fork = h->side && h->use_side && !h->profile && !h->debug && !video_index && !venc;
     if (fork) {
       CK(cudaEventRecord(h->ev_fork, main_st));
       CK(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
@@ -746,6 +751,7 @@ struct Fwd {
       st = main_st;
     }
     if ((rc = tap(0, xt, SQ_D))) return rc;
+    if (venc) return run_encoded(venc, xt);
     if (video_index) return run_shared_video(xt);
     // video affine (models/layers.py:118-123) -> rows [0, Mv)
     if ((rc = video_affine(vfeat, Mv, ws.z, ws.x))) return rc;
@@ -775,27 +781,41 @@ struct Fwd {
     return run_after_encoder(tc_att0);
   }
 
-  // Query-independent video branch once per UNIQUE clip (SURVEY.md section 8 (f1)): VisualProjection + the video half of the
-  // shared FeatureEncoder run on U*L rows, the encoded rows are then expanded to the B pairs; the text half of the encoder
-  // runs on its own.  Same kernels, same per-row arithmetic as the plain path.
-  int run_shared_video(float* xt) {
-    const long long Mu = (long long)U * L;
+  // The query-independent video branch of `nclips` clips (models/SeqPAN.py:57,59): VisualProjection -> `aff`, then the video
+  // half of the shared FeatureEncoder -> `out` (`tmp`: pre-LayerNorm rows of the fp32 mode).  One segment per clip and
+  // row-local arithmetic: a clip's rows do not depend on the other clips of the call (seqpan_encode_videos relies on it).
+  int encode_clips(const float* vf, int nclips, float* tmp, float* aff, float* out) {
+    const long long Mu = (long long)nclips * L;
     int rc;
-    if ((rc = video_affine(vfeat, Mu, ws.o, ws.u))) return rc;
-    Segs clips{{0, 0}, {U, 0}, {L, 0}};
-    if ((rc = conv_block(ws.u, ws.s, W_ENC_POS, clips, Mu, TC_ENC_PW0))) return rc;
-    auto gather = [&](const float* src, float* dst) -> int {
-      h->begin("gather_clips", st);
-      gather_clips_kernel<<<(unsigned)((Mv + 7) / 8), 256, 0, st>>>(src, video_index, dst, L, U, Mv);
-      h->end(st);
-      ++h->launches;
-      CK(cudaGetLastError());
-      return SEQPAN_OK;
-    };
-    if ((rc = gather(ws.s, ws.xb))) return rc;
+    if ((rc = video_affine(vf, Mu, tmp, aff))) return rc;
+    Segs clips{{0, 0}, {nclips, 0}, {L, 0}};
+    return conv_block(aff, out, W_ENC_POS, clips, Mu, TC_ENC_PW0);
+  }
+  int gather(const float* src, float* dst) {
+    h->begin("gather_clips", st);
+    gather_clips_kernel<<<(unsigned)((Mv + 7) / 8), 256, 0, st>>>(src, video_index, dst, L, U, Mv);
+    h->end(st);
+    ++h->launches;
+    CK(cudaGetLastError());
+    return SEQPAN_OK;
+  }
+
+  // Query-independent video branch once per UNIQUE clip (SURVEY.md section 8 (f1)): the U clips are encoded into the
+  // workspace, then the query half runs as on stored encodings.  Same kernels, same per-row arithmetic as the plain path.
+  int run_shared_video(float* xt) {
+    int rc;
+    if ((rc = encode_clips(vfeat, U, ws.o, ws.u, ws.s))) return rc;
     if (h->debug) {
       if ((rc = gather(ws.u, ws.x)) || (rc = tap(1, ws.x, SQ_D))) return rc;
     }
+    return run_encoded(ws.s, xt);
+  }
+
+  // The query half on encoded clip rows `enc` [U,L,128]: expand them to the B pairs, run the text half of the encoder
+  // (BackBone: its own tfeat_encoder), then everything behind the encoder.
+  int run_encoded(const float* enc, float* xt) {
+    int rc;
+    if ((rc = gather(enc, ws.xb))) return rc;
     Segs text{{0, 0}, {B, 0}, {T, 0}};
     const bool own_text = h->s.variant == SEQPAN_VARIANT_BACKBONE;
     if ((rc = conv_block(xt, ws.xb + Mv * SQ_D, own_text ? W_TENC_POS : W_ENC_POS, text, Mt, own_text ? TC_TENC_PW0 : TC_ENC_PW0))) return rc;
@@ -872,7 +892,7 @@ struct Fwd {
 
 }  // namespace
 
-static int forward_impl(SeqpanHandle* h, const int64_t* word_ids, const int64_t* char_ids, const float* vfeat,
+static int forward_impl(SeqpanHandle* h, int mode, const int64_t* word_ids, const int64_t* char_ids, const float* vfeat,
                         const int32_t* video_index, int U, const float* vmask, const float* tmask, const float* gumbel, int B,
                         int T, int C, float* slogits, float* elogits, float* match_score, void* workspace,
                         size_t workspace_bytes, void* stream) {
@@ -897,18 +917,19 @@ static int forward_impl(SeqpanHandle* h, const int64_t* word_ids, const int64_t*
     return fail(SEQPAN_E_INVALID, "L=%d, T=%d: CQAttention score tiles (%zu B) exceed 227 KB of shared memory", s.vlen, T, cq_attention_smem(s.vlen, T));
   if (dual_attention_smem(s.vlen, T) > 227 * 1024 || batch_attention_smem(B) > 227 * 1024)
     return fail(SEQPAN_E_INVALID, "attention tiles exceed 227 KB of shared memory (B=%d, L=%d, T=%d)", B, s.vlen, T);
-  f.word_ids = word_ids; f.char_ids = char_ids; f.vfeat = vfeat; f.vmask = vmask; f.tmask = tmask; f.gumbel = gumbel;
+  f.word_ids = word_ids; f.char_ids = char_ids; f.vmask = vmask; f.tmask = tmask; f.gumbel = gumbel;
+  (mode == FWD_ENCODED ? f.venc : f.vfeat) = vfeat;
   f.slogits = slogits; f.elogits = elogits; f.match_score = match_score;
   f.video_index = video_index; f.U = U;
   h->launches = 0;
-  h->lastB = B; h->lastT = T;
+  h->lastB = B; h->lastT = T; h->last_encoded = mode == FWD_ENCODED;
   if (h->profile && h->recs.size() > 200000) { h->recs.clear(); h->pool_used = 0; }
   if (!h->use_graph || h->debug || h->profile || (h->use_graph == 2 && f.Mv > 8192)) return f.run();
   GraphKey key;
   memset(&key, 0, sizeof(key));
   const void* ptrs[11] = {word_ids, char_ids, vfeat, video_index, vmask, tmask, gumbel, slogits, elogits, match_score, workspace};
   memcpy(key.p, ptrs, sizeof(ptrs));
-  key.B = B; key.T = T; key.C = C; key.U = U; key.side = h->use_side;
+  key.B = B; key.T = T; key.C = C; key.U = U; key.side = h->use_side; key.mode = mode;
   ++h->tick;
   auto it = h->graphs.find(key);
   if (it != h->graphs.end()) {
@@ -958,7 +979,7 @@ extern "C" int seqpan_forward(SeqpanHandle* h, const int64_t* word_ids, const in
                               const float* vmask, const float* tmask, const float* gumbel, int B, int T, int C,
                               float* slogits, float* elogits, float* match_score, void* workspace,
                               size_t workspace_bytes, void* stream) {
-  return forward_impl(h, word_ids, char_ids, vfeat, nullptr, 0, vmask, tmask, gumbel, B, T, C, slogits, elogits, match_score,
+  return forward_impl(h, FWD_RAW, word_ids, char_ids, vfeat, nullptr, 0, vmask, tmask, gumbel, B, T, C, slogits, elogits, match_score,
                       workspace, workspace_bytes, stream);
 }
 
@@ -969,7 +990,43 @@ extern "C" int seqpan_forward_shared_video(SeqpanHandle* h, const int64_t* word_
                                            void* stream) {
   if (!video_index) return fail(SEQPAN_E_INVALID, "video_index is NULL");
   if (U < 1 || U > B) return fail(SEQPAN_E_INVALID, "U=%d outside [1,B=%d]", U, B);
-  return forward_impl(h, word_ids, char_ids, vfeat_unique, video_index, U, vmask, tmask, gumbel, B, T, C, slogits, elogits,
+  return forward_impl(h, FWD_SHARED, word_ids, char_ids, vfeat_unique, video_index, U, vmask, tmask, gumbel, B, T, C, slogits,
+                      elogits, match_score, workspace, workspace_bytes, stream);
+}
+
+// The argument checks that need no handle come first, so they answer the same with or without a device.
+extern "C" int seqpan_encode_videos(SeqpanHandle* h, const float* vfeat, int U, float* venc, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  if (!vfeat || !venc) return fail(SEQPAN_E_INVALID, "NULL tensor argument");
+  if (((uintptr_t)vfeat | (uintptr_t)venc) & 15) return fail(SEQPAN_E_INVALID, "vfeat and venc must be 16-byte aligned (vector and TMA access)");
+  if (U < 1) return fail(SEQPAN_E_INVALID, "U=%d < 1", U);
+  if (!h) return fail(SEQPAN_E_INVALID, "handle is NULL");
+  const SeqpanShapes& s = h->s;
+  if (U > s.max_batch) return fail(SEQPAN_E_INVALID, "U=%d > max_batch=%d (the workspace holds max_batch*vlen rows)", U, s.max_batch);
+  if (!workspace || ((uintptr_t)workspace & 255)) return fail(SEQPAN_E_WORKSPACE, "workspace must be a 256-byte aligned device pointer");
+  Fwd f{};
+  f.h = h; f.st = (cudaStream_t)stream; f.B = U; f.L = s.vlen; f.T = 1; f.C = 4;
+  f.Mv = (long long)U * s.vlen; f.Mt = U; f.M = f.Mv + f.Mt;
+  f.tc = s.precision == SEQPAN_PREC_BF16;
+  f.tf32 = s.precision == SEQPAN_PREC_TF32;
+  Carver c(workspace);
+  carve_workspace(c, s, U, 1, f.ws);
+  if (c.off > workspace_bytes) return fail(SEQPAN_E_WORKSPACE, "workspace too small: need %zu, have %zu", c.off, workspace_bytes);
+  h->launches = 0;
+  h->lastB = 0;   // the workspace no longer holds a forward's taps
+  if (h->profile && h->recs.size() > 200000) { h->recs.clear(); h->pool_used = 0; }
+  return f.encode_clips(vfeat, U, f.ws.o, f.ws.u, venc);
+}
+
+extern "C" int seqpan_forward_encoded(SeqpanHandle* h, const int64_t* word_ids, const int64_t* char_ids, const float* venc,
+                                      const int32_t* video_index, int U, const float* vmask, const float* tmask,
+                                      const float* gumbel, int B, int T, int C, float* slogits, float* elogits,
+                                      float* match_score, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!venc) return fail(SEQPAN_E_INVALID, "venc is NULL");
+  if ((uintptr_t)venc & 15) return fail(SEQPAN_E_INVALID, "venc must be 16-byte aligned (the clip gather reads float4)");
+  if (U < 1) return fail(SEQPAN_E_INVALID, "U=%d < 1", U);
+  if (!video_index && U < B) return fail(SEQPAN_E_INVALID, "video_index is NULL and U=%d < B=%d: pair b needs clip b", U, B);
+  return forward_impl(h, FWD_ENCODED, word_ids, char_ids, venc, video_index, U, vmask, tmask, gumbel, B, T, C, slogits, elogits,
                       match_score, workspace, workspace_bytes, stream);
 }
 
@@ -982,6 +1039,7 @@ extern "C" int64_t seqpan_debug_tap(SeqpanHandle* h, const char* name, const voi
   carve_workspace(c, h->s, h->lastB, h->lastT, ws);
   for (int i = 0; i < NUM_TAPS; ++i) {
     if (strcmp(name, kTapNames[i]) != 0) continue;
+    if (i == 1 && h->last_encoded) return fail(SEQPAN_E_INVALID, "tap 'video_affine' does not exist on a forward from stored encodings");
     const int64_t rows = kTapIsText[i] ? (int64_t)h->lastB * h->lastT : (int64_t)h->lastB * h->s.vlen;
     if (rows * SQ_D > out_capacity_floats) return fail(SEQPAN_E_WORKSPACE, "tap '%s' needs %lld floats", name, (long long)rows * SQ_D);
     CK(cudaMemcpyAsync(out, ws.taps[i], sizeof(float) * rows * SQ_D, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));

@@ -215,7 +215,7 @@ class _Slot:
 
 def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: bool = False, streams: int = 2,
              ragged_h2d: bool = True, h2d_ctas: int = 32, profile: bool = False, check_padding: bool | None = None,
-             allreduce: bool = True, topk: int | None = None, nms_thresh: float = 0.5):
+             allreduce: bool = True, topk: int | None = None, nms_thresh: float = 0.5, video_encodings=None):
     """Runs forward + span decode + IoU counters over an iterable of HOST batches (dicts in ``BaseCollate``'s key
     naming, ideally pinned) -- the eval loop of ``main.py:112-134`` as one pipelined call.
 
@@ -240,6 +240,11 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     ``recall`` (R@k at IoU 0.3, 0.5, 0.7, percent) and ``counters`` (``[n, #>=0.3, #>=0.5, #>=0.7]``), and with
     ``return_fracs`` ``info["topk_fracs"]`` holds all ``(B,k,2)`` fractions.  Both counter sets live in one fp64 buffer, so
     the sweep still ends in a single all-reduce.
+    ``video_encodings`` (from ``model.encode_videos``, on ``device``; DESIGN.md section 12): the batches carry no ``vfeats``,
+    their ``video_index`` names clips of the encodings (without it, pair b reads clip b), and no video byte crosses PCIe --
+    ``info["h2d_bytes"]`` counts ids, masks, ground truth and indices only.  Results equal the sweep over the raw clips with the
+    same ``video_index``.  Under ``torchrun`` every rank encodes the clips its batches use onto its own device (encodings are
+    device memory and are not shared between ranks).
     """
     _cabi.require_device()
     if topk is not None:
@@ -247,11 +252,28 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
         if not (1 <= topk <= 32 and 0.0 < nms_thresh <= 1.0):
             raise ValueError(f"topk={topk} must be in [1,32] and nms_thresh={nms_thresh} in (0,1]")
     device = torch.device(device or "cuda")
+    if device.index is None:     # "cuda" = the current device; the handles and the parameters compare full device names
+        device = torch.device("cuda", torch.cuda.current_device())
     L_ = _cabi.lib()
     import os
     if check_padding is None:
         check_padding = os.environ.get("SEQPAN_CHECK_PADDING") == "1"
     batches = list(host_batches)
+    enc = video_encodings
+    if enc is not None:
+        model._check_encoded_call(enc, None, None)
+        if enc.device != device:
+            raise _cabi.SeqpanError(f"the encodings live on {enc.device}, the sweep runs on {device}: encode on every rank's device")
+        for i, b in enumerate(batches):
+            B = b["vmasks"].shape[0]
+            if "vfeats" in b:
+                raise _cabi.SeqpanError(f"batch {i} carries vfeats: with video_encodings the clips come from the encodings")
+            if "video_index" in b:
+                idx = b["video_index"]
+                if idx.shape != (B,) or (B and (int(idx.min()) < 0 or int(idx.max()) >= len(enc))):
+                    raise _cabi.SeqpanError(f"batch {i}: video_index must be [{B}] with values in [0,{len(enc)})")
+            elif B > len(enc):
+                raise _cabi.SeqpanError(f"batch {i} has no video_index and {B} pairs > {len(enc)} encoded clips")
     main = torch.cuda.current_stream(device)
     nstreams = max(1, int(streams))
     counters = IouCounters(device)
@@ -275,7 +297,7 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     Bm = max(b["vmasks"].shape[0] for b in batches)
     Tm = max(b["words_ids"].shape[1] for b in batches)
     Cm = max(b["char_ids"].shape[2] for b in batches)
-    Lv, V = batches[0]["vfeats"].shape[1], batches[0]["vfeats"].shape[2]
+    Lv, V = (batches[0]["vfeats"].shape[1], batches[0]["vfeats"].shape[2]) if enc is None else (enc.rows.shape[1], 0)
     was_sync, was_ctx, was_side = model.sync_timing, model._ctx_key, getattr(model, "_side_stream", True)
     if hasattr(model, "set_side_stream"):
         model.set_side_stream(False)      # the sweep is bound by its own host->device copy kernel (include/seqpan_b200.h)
@@ -285,6 +307,8 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
         # re-packing in the middle of it)
         for k in range(nstreams):
             model.use_context(k)._ensure_handle(device, Bm, Tm, Cm)
+            if enc is not None:
+                model._check_encoding_weights(enc)
         model.use_context(was_ctx)
         # the slots and contexts were allocated / packed on the caller's stream: the copy stream and the lanes start after it
         ready = torch.cuda.Event()
@@ -303,7 +327,7 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
         nonlocal h2d
         b, sl = batches[i], slots[i % len(slots)]
         B, T, Cc = b["words_ids"].shape[0], b["words_ids"].shape[1], b["char_ids"].shape[2]
-        U = b["vfeats"].shape[0]          # == B unless the batch shares clips through video_index
+        U = b["vfeats"].shape[0] if enc is None else 0   # == B unless the batch shares clips through video_index
         v = {"words": sl.words[: B * T].view(B, T), "chars": sl.chars[: B * T * Cc].view(B, T, Cc),
              "vfeats": sl.vfeats[: U * Lv * V].view(U, Lv, V), "vmask": sl.vmask[: B * Lv].view(B, Lv),
              "vindex": sl.vindex[:B] if "video_index" in b else None,
@@ -329,11 +353,13 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
             if v["gt"] is not None:
                 v["gt"].copy_(b["se_fracs"], non_blocking=True)
                 h2d += b["se_fracs"].numel() * 4
-            vf = b["vfeats"]
+            vf = b.get("vfeats")
             if v["vindex"] is not None:
                 v["vindex"].copy_(b["video_index"].to(torch.int32), non_blocking=True)
                 h2d += B * 4
-            if (ragged_h2d and v["vindex"] is None and vf.is_pinned() and vf.dtype == torch.float32 and vf.is_contiguous()
+            if enc is not None:
+                pass                                      # the clips are resident as encodings
+            elif (ragged_h2d and v["vindex"] is None and vf.is_pinned() and vf.dtype == torch.float32 and vf.is_contiguous()
                     and V % 4 == 0):
                 valid_host[i, :B].copy_(valid_rows_from_mask(b["vmasks"]))
                 if check_padding:
@@ -373,7 +399,7 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                     # == F.gumbel_softmax's draw (models/SeqPAN.py:79): -empty_like(logits).exponential_().log()
                     v["gumbel"].exponential_().log_().neg_()
                     model.forward_into(v["words"], v["chars"], v["vfeats"], v["vmask"], v["tmask"], v["gumbel"],
-                                       v["slogits"], v["elogits"], v["match"], v["vindex"])
+                                       v["slogits"], v["elogits"], v["match"], v["vindex"], video_encodings=enc)
                     B = v["vmask"].shape[0]
                     st = lane.cuda_stream
                     _cabi.check(L_.seqpan_span_decode(v["slogits"].data_ptr(), v["elogits"].data_ptr(), v["vmask"].data_ptr(),

@@ -191,6 +191,26 @@ class _SeqPANPredictor(_Holder):  # models/layers.py:642-657
         self.end_dense = _Conv1D(dim, 1)
 
 
+class VideoEncodings:
+    """Encoded clips of :meth:`SeqPAN.encode_videos`: ``rows`` is the ``[U,vlen,128]`` fp32 CUDA tensor of VisualProjection +
+    the video half of the shared FeatureEncoder (DESIGN.md section 12), owned by the caller.  ``precision``, ``variant`` and
+    ``signature`` (the weights' ``(data_ptr, _version)`` signature when they were packed, with the count of explicit
+    ``repack()`` calls) record what made them: a forward refuses encodings of another precision, another model variant or
+    weights that changed since."""
+
+    __slots__ = ("rows", "precision", "variant", "signature")
+
+    def __init__(self, rows: torch.Tensor, precision: str, variant: int, signature):
+        self.rows, self.precision, self.variant, self.signature = rows, precision, variant, signature
+
+    def __len__(self):
+        return self.rows.shape[0]
+
+    @property
+    def device(self):
+        return self.rows.device
+
+
 class SeqPAN(nn.Module):
     """B200-native SeqPAN.  Extra, optional knobs beyond the reference constructor:
 
@@ -247,6 +267,7 @@ class SeqPAN(nn.Module):
         self._ctx_key = 0
         self._frozen = False
         self._debug = False
+        self._repacks = 0            # explicit repack() calls: part of what VideoEncodings are checked against
         self._register_load_state_dict_pre_hook(self._strip_module_prefix)
 
     # ---- checkpoint compatibility ----------------------------------------------------------------------
@@ -322,7 +343,9 @@ class SeqPAN(nn.Module):
         """Re-derives the packed weights (bf16 copies, folded products, host mirrors of the small vectors) from the current
         parameter values.  Needed only after edits the version counters cannot see -- ``p.data.copy_(...)`` /
         ``p.data.mul_(...)`` (EMA swaps) do not bump ``Tensor._version`` -- or while :meth:`freeze` is on; ordinary optimizer
-        steps, ``load_state_dict`` and ``.to()`` are detected automatically."""
+        steps, ``load_state_dict`` and ``.to()`` are detected automatically.  Encodings of :meth:`encode_videos` made before
+        the call are stale afterwards: the edits it exists for leave the weights' signature unchanged."""
+        self._repacks += 1
         for key in [self._ctx_key] + list(self._ctxs):
             self.use_context(key)
             if self._handle is not None:
@@ -414,7 +437,7 @@ class SeqPAN(nn.Module):
                 raise _cabi.SeqpanError(f"parameter {name} has {t.numel()} elements, the configured shapes need {want} "
                                         f"(configs.num_words / num_chars / vlen / vdim must match the tensors)")
 
-    def _check_inputs(self, word_ids, char_ids, vfeat_in, vmask, tmask, video_index):
+    def _check_inputs(self, word_ids, char_ids, vfeat_in, vmask, tmask, video_index, encoded=False):
         if not vfeat_in.is_cuda:
             raise _cabi.SeqpanError("inputs must be CUDA tensors (the reference moves them in train_engine_SeqPAN, "
                                     "models/SeqPAN.py:173); there is no CPU path")
@@ -429,8 +452,12 @@ class SeqPAN(nn.Module):
         if word_ids.shape != (B, T) or char_ids.shape != (B, T, Cc) or tmask.shape != (B, T):
             raise _cabi.SeqpanError(f"batch / length mismatch: word_ids {tuple(word_ids.shape)}, char_ids {tuple(char_ids.shape)}, "
                                     f"tmask {tuple(tmask.shape)} against vmask {tuple(vmask.shape)}")
-        U = B if video_index is None else vfeat_in.shape[0]
-        if Lv != self.configs.model.vlen or vfeat_in.shape != (U, Lv, self.configs.model.vdim) or not 1 <= U <= B:
+        U = B if video_index is None and not encoded else vfeat_in.shape[0]
+        if encoded:   # vfeat_in = the rows of VideoEncodings: any number of clips, at least B without video_index
+            if Lv != self.configs.model.vlen or vfeat_in.shape != (U, Lv, 128) or U < (B if video_index is None else 1):
+                raise _cabi.SeqpanError(f"video_encodings.rows must be [U,{self.configs.model.vlen},128] with U >= 1 (U >= B={B} "
+                                        f"without video_index), got {tuple(vfeat_in.shape)} with vmask {tuple(vmask.shape)}")
+        elif Lv != self.configs.model.vlen or vfeat_in.shape != (U, Lv, self.configs.model.vdim) or not 1 <= U <= B:
             raise _cabi.SeqpanError(f"vfeat_in must be [B,{self.configs.model.vlen},{self.configs.model.vdim}] (or [U<=B,...] "
                                     f"with video_index), got {tuple(vfeat_in.shape)} with vmask {tuple(vmask.shape)}")
         if video_index is not None and video_index.shape != (B,):
@@ -438,7 +465,7 @@ class SeqPAN(nn.Module):
         return device, B, Lv, T, Cc, U
 
     # ---- the hot path ----------------------------------------------------------------------------------
-    def forward(self, word_ids, char_ids, vfeat_in, vmask, tmask, *, gumbel=None, video_index=None):
+    def forward(self, word_ids, char_ids, vfeat_in, vmask, tmask, *, gumbel=None, video_index=None, video_encodings=None):
         """models/SeqPAN.py:50-95.  ``gumbel`` (keyword-only, optional) injects the ``[B,L,4]`` noise that
         ``F.gumbel_softmax`` would draw (parity tests against a CPU run); by default it is drawn on the device by
         the same torch call the reference makes, so a seeded reference on the same GPU sees the same noise.
@@ -448,10 +475,18 @@ class SeqPAN(nn.Module):
         (VisualProjection + the video half of the shared encoder, models/SeqPAN.py:57,59) runs once per clip; the
         outputs equal the plain call on ``vfeat_in[video_index]``.
 
+        ``video_encodings`` (keyword-only, optional; DESIGN.md section 12): clips stored by :meth:`encode_videos`, in place of
+        ``vfeat_in`` (pass ``None`` for it).  ``video_index[b]`` names the clip of pair ``b`` among them (``None``: clip ``b``);
+        only the query half of the forward runs, and the outputs are bit-identical to ``forward(vfeats, video_index=...)`` on the
+        raw clips.  Eval mode only; encodings of another precision or model variant, or of weights that changed since they
+        were made (optimizer step, ``load_state_dict``, :meth:`repack`; not checked under :meth:`freeze`), raise.
+
         In ``train()`` mode (no ``video_index``) the forward runs with dropout on the training kernels.  When grad mode is on
         and some parameter or ``vfeat_in`` requires grad, the outputs carry an autograd graph: ``loss.backward()`` of any torch
         loss on them fills ``p.grad`` (and ``vfeat_in.grad``) through the training kernels' backward, once per forward (no
         double backward, no ``retain_graph``).  ``eval()`` mode never records one."""
+        if video_encodings is not None:
+            self._check_encoded_call(video_encodings, vfeat_in, video_index)
         _cabi.require_device()
         if self.training:
             # training mode (dropout active, models/layers.py nn.Dropout sites): the primitive-by-primitive forward of
@@ -481,12 +516,14 @@ class SeqPAN(nn.Module):
                 return {"slogits": sl, "elogits": el, "vmask": vmask, "consume_time": consume_time}
             return {"slogits": sl, "elogits": el, "vmask": vmask, "match_score": ms, "label_embs": self.label_embs,
                     "consume_time": consume_time}
-        device, B, Lv, T, Cc, U = self._check_inputs(word_ids, char_ids, vfeat_in, vmask, tmask, video_index)
+        enc = video_encodings
+        device, B, Lv, T, Cc, U = self._check_inputs(word_ids, char_ids, vfeat_in if enc is None else enc.rows, vmask, tmask,
+                                                     video_index, encoded=enc is not None)
         if video_index is not None:
-            video_index = video_index.to(device=vfeat_in.device, dtype=torch.int32).contiguous()
+            video_index = video_index.to(device=device, dtype=torch.int32).contiguous()
         word_ids = word_ids.to(torch.int64).contiguous()
         char_ids = char_ids.to(torch.int64).contiguous()
-        vfeat = vfeat_in.to(torch.float32).contiguous()
+        vfeat = vfeat_in.to(torch.float32).contiguous() if enc is None else enc.rows
         vm = vmask.to(torch.float32).contiguous()
         tm = tmask.to(torch.float32).contiguous()
         if not self._MATCH_HEAD:      # BackBone: no Gumbel softmax, nothing drawn (the library ignores the pointer)
@@ -498,6 +535,8 @@ class SeqPAN(nn.Module):
             gumbel = gumbel.to(device=device, dtype=torch.float32).contiguous()
         with torch.cuda.device(device):
             self._ensure_handle(device, B, T, Cc)
+            if enc is not None:
+                self._check_encoding_weights(enc)
             slogits = torch.empty(B, Lv, dtype=torch.float32, device=device)
             elogits = torch.empty(B, Lv, dtype=torch.float32, device=device)
             match_score = torch.empty(B, Lv, 4, dtype=torch.float32, device=device)
@@ -505,7 +544,13 @@ class SeqPAN(nn.Module):
                 torch.cuda.synchronize()
             start = time.time()
             stream = torch.cuda.current_stream(device).cuda_stream
-            if video_index is None:
+            if enc is not None:
+                _cabi.check(_cabi.lib().seqpan_forward_encoded(
+                    self._handle, word_ids.data_ptr(), char_ids.data_ptr(), vfeat.data_ptr(),
+                    video_index.data_ptr() if video_index is not None else None, U, vm.data_ptr(), tm.data_ptr(),
+                    gumbel.data_ptr(), B, T, Cc, slogits.data_ptr(), elogits.data_ptr(), match_score.data_ptr(),
+                    self._workspace.data_ptr(), self._workspace.numel(), stream))
+            elif video_index is None:
                 _cabi.check(_cabi.lib().seqpan_forward(
                     self._handle, word_ids.data_ptr(), char_ids.data_ptr(), vfeat.data_ptr(), vm.data_ptr(), tm.data_ptr(),
                     gumbel.data_ptr(), B, T, Cc, slogits.data_ptr(), elogits.data_ptr(), match_score.data_ptr(),
@@ -524,15 +569,26 @@ class SeqPAN(nn.Module):
         return {"slogits": slogits, "elogits": elogits, "vmask": vmask, "match_score": match_score,
                 "label_embs": self.label_embs, "consume_time": consume_time}
 
-    def forward_into(self, word_ids, char_ids, vfeat, vmask, tmask, gumbel, slogits, elogits, match_score, video_index=None):
+    def forward_into(self, word_ids, char_ids, vfeat, vmask, tmask, gumbel, slogits, elogits, match_score, video_index=None,
+                     video_encodings=None):
         """The raw call behind :meth:`forward` for callers that own every buffer (the engine's static ring): all
         arguments are contiguous CUDA tensors of the C ABI's dtypes (int64 ids, float32 everything else; int32
         ``video_index`` with ``vfeat`` = the ``[U,L,V]`` unique clips) on one device; nothing is allocated, converted or
-        checked here beyond what the library checks."""
-        device = vfeat.device
+        checked here beyond what the library checks.  With ``video_encodings`` (see :meth:`forward`) ``vfeat`` is ignored
+        and ``video_index`` indexes the encodings' rows (out-of-range indices are clamped by the library, not reported)."""
+        device = (vfeat if video_encodings is None else video_encodings.rows).device
         B, T, Cc = word_ids.shape[0], word_ids.shape[1], char_ids.shape[2]
         with torch.cuda.device(device):
             self._ensure_handle(device, B, T, Cc)
+            if video_encodings is not None:
+                rows = video_encodings.rows
+                _cabi.check(_cabi.lib().seqpan_forward_encoded(
+                    self._handle, word_ids.data_ptr(), char_ids.data_ptr(), rows.data_ptr(),
+                    video_index.data_ptr() if video_index is not None else None, rows.shape[0], vmask.data_ptr(),
+                    tmask.data_ptr(), gumbel.data_ptr(), B, T, Cc, slogits.data_ptr(), elogits.data_ptr(),
+                    match_score.data_ptr(), self._workspace.data_ptr(), self._workspace.numel(),
+                    torch.cuda.current_stream(device).cuda_stream))
+                return
             if video_index is not None:
                 _cabi.check(_cabi.lib().seqpan_forward_shared_video(
                     self._handle, word_ids.data_ptr(), char_ids.data_ptr(), vfeat.data_ptr(), video_index.data_ptr(),
@@ -545,6 +601,69 @@ class SeqPAN(nn.Module):
                 tmask.data_ptr(), gumbel.data_ptr(), B, T, Cc, slogits.data_ptr(), elogits.data_ptr(),
                 match_score.data_ptr(), self._workspace.data_ptr(), self._workspace.numel(),
                 torch.cuda.current_stream(device).cuda_stream))
+
+    # ---- stored video encodings (DESIGN.md section 12) ---------------------------------------------------------
+    def encode_videos(self, vfeats, chunk: int = 256) -> VideoEncodings:
+        """Runs the query-independent video branch -- VisualProjection + the video half of the shared FeatureEncoder
+        (models/SeqPAN.py:57,59) -- once over ``vfeats`` ``[U,vlen,vdim]`` and returns its ``[U,vlen,128]`` fp32 rows as
+        :class:`VideoEncodings` for ``forward(..., None, ..., video_encodings=, video_index=)`` and
+        ``evaluate(video_encodings=)``: later queries of these clips move no video bytes and skip that branch.  ``vfeats`` is a
+        CUDA tensor; the encodings land on its device.  At most ``chunk`` clips go through the library per call, which bounds
+        the workspace (``chunk`` above the library's batch limit of 768 is lowered to it); a clip's encoding does not depend on
+        the chunking.  Eval mode only: in ``train()``
+        dropout acts on the video branch of every pair, so there is nothing to store."""
+        if self.training:
+            raise _cabi.SeqpanError("encode_videos needs eval(): in train() dropout acts on the video branch of every pair")
+        m = self.configs.model
+        if vfeats.dim() != 3 or tuple(vfeats.shape[1:]) != (m.vlen, m.vdim):
+            raise _cabi.SeqpanError(f"vfeats must be [U,{m.vlen},{m.vdim}], got {tuple(vfeats.shape)}")
+        if int(chunk) < 1:
+            raise ValueError(f"chunk={chunk} must be >= 1")
+        _cabi.require_device()
+        if not vfeats.is_cuda:
+            raise _cabi.SeqpanError("vfeats must be a CUDA tensor (there is no CPU path)")
+        device, U = vfeats.device, vfeats.shape[0]
+        n = max(1, min(int(chunk), U, _MAX_BATCH))
+        rows = torch.empty(U, m.vlen, 128, dtype=torch.float32, device=device)
+        with torch.cuda.device(device):
+            self._ensure_handle(device, n, 1, 4)
+            stream = torch.cuda.current_stream(device).cuda_stream
+            for lo in range(0, U, n):
+                vf = vfeats[lo:lo + n].to(torch.float32).contiguous()
+                _cabi.check(_cabi.lib().seqpan_encode_videos(self._handle, vf.data_ptr(), vf.shape[0], rows[lo:lo + n].data_ptr(),
+                                                             self._workspace.data_ptr(), self._workspace.numel(), stream))
+        return VideoEncodings(rows, self.precision, self._VARIANT, self._packed_weights_key())
+
+    def _check_encoded_call(self, enc, vfeat_in, video_index):
+        """The checks of a forward on stored encodings that need neither the device nor the library handle."""
+        if vfeat_in is not None:
+            raise _cabi.SeqpanError("pass vfeat_in=None with video_encodings: the clips come from the encodings")
+        if self.training:
+            raise _cabi.SeqpanError("video_encodings need eval(): in train() dropout acts on the video branch of every pair")
+        if not isinstance(enc, VideoEncodings):
+            raise _cabi.SeqpanError(f"video_encodings must come from encode_videos, got {type(enc).__name__}")
+        if enc.precision != self.precision or enc.variant != self._VARIANT:
+            raise _cabi.SeqpanError(f"the encodings were made by a {enc.precision} model of variant {enc.variant}, this is a "
+                                    f"{self.precision} model of variant {self._VARIANT}")
+        rows, vlen = enc.rows, self.configs.model.vlen
+        if rows.dim() != 3 or tuple(rows.shape[1:]) != (vlen, 128) or rows.dtype != torch.float32 or not rows.is_contiguous():
+            raise _cabi.SeqpanError(f"video_encodings.rows must be a contiguous float32 [U,{vlen},128] tensor, got "
+                                    f"{rows.dtype} {tuple(rows.shape)}")
+        if video_index is not None and video_index.numel() > 0:
+            lo, hi = int(video_index.min()), int(video_index.max())
+            if lo < 0 or hi >= rows.shape[0]:
+                raise _cabi.SeqpanError(f"video_index values [{lo},{hi}] outside [0,{rows.shape[0]}) of the encodings")
+
+    def _packed_weights_key(self):
+        """What the current kernel context packed: the weights' signature at packing time (under :meth:`freeze` it can lag the
+        parameters) and the count of explicit :meth:`repack` calls (which follow edits the signature cannot see)."""
+        return self._repacks, self._wsig
+
+    def _check_encoding_weights(self, enc):
+        """Encodings made with other weights are stale (the current kernel context's signature is fresh after _ensure_handle)."""
+        if not self._frozen and enc.signature != self._packed_weights_key():
+            raise _cabi.SeqpanError("the weights changed since these encodings were made (optimizer step, load_state_dict, "
+                                    "repack): call encode_videos again")
 
     def set_profile(self, on: bool = True):
         """Per-launch CUDA-event timing inside the library (bench.py's per-kernel roofline)."""
@@ -579,6 +698,9 @@ class SeqPAN(nn.Module):
 
 def _cabi_max_tlen() -> int:
     return 128  # SEQPAN_MAX_TLEN in include/seqpan_b200.h
+
+
+_MAX_BATCH = 768   # largest SeqpanShapes.max_batch the library accepts (check_shapes in csrc/seqpan_api.cu)
 
 
 def _decode(start_logits, end_logits, vmask, want_idx, want_fracs):
@@ -697,7 +819,7 @@ def _runner(cls, configs, modules, precision, sync_timing):
         setattr(r, k, v)
     r.precision, r.sync_timing = precision, sync_timing
     r._handle = r._limits = r._arena = r._workspace = r._wsig = r._wptrs = None
-    r._ctxs, r._ctx_key, r._frozen, r._debug = {}, 0, False, False
+    r._ctxs, r._ctx_key, r._frozen, r._debug, r._repacks = {}, 0, False, False, 0
     r.eval()
     return r
 
@@ -754,8 +876,10 @@ class OneTeacher(nn.Module):
             label_embs=self.label_embs_t0, predictor=self.predictor_t0), prec, False)
         object.__setattr__(self, "_runners", (teacher, student))
 
-    def forward(self, word_ids, char_ids, vfeat_in, vmask, tmask, *, gumbel=None, gumbel_t0=None):
+    def forward(self, word_ids, char_ids, vfeat_in, vmask, tmask, *, gumbel=None, gumbel_t0=None, video_encodings=None):
         """models/OneTeacher.py:54-128.  ``gumbel_t0`` / ``gumbel`` inject the teacher's / student's noise (parity tests)."""
+        if video_encodings is not None:
+            raise NotImplementedError("OneTeacher has two video branches (teacher and student): no stored encodings")
         _cabi.require_device()
         if self.training:
             raise NotImplementedError("OneTeacher ships the inference forward; call model.eval()")
@@ -772,6 +896,11 @@ class OneTeacher(nn.Module):
         return {"slogits_t0": t["slogits"], "elogits_t0": t["elogits"], "match_score_t0": t["match_score"],
                 "label_embs_t0": self.label_embs_t0, "slogits": s["slogits"], "elogits": s["elogits"],
                 "match_score": s["match_score"], "label_embs": self.label_embs, "vmask": vmask, "consume_time": consume_time}
+
+
+    def encode_videos(self, vfeats, chunk: int = 256):
+        raise NotImplementedError("OneTeacher has two video branches (teacher and student); stored encodings exist for SeqPAN, "
+                                  "BaseFast, MultiTeacher and BackBone")
 
 
 def infer_OneTeacher(output, configs=None):
