@@ -164,6 +164,18 @@ int seqpan_span_decode(const float* slogits, const float* elogits, const float* 
 /* counters[0..4] (fp64, device) += {n, sum IoU, #IoU>=0.3, #IoU>=0.5, #IoU>=0.7} of fracs vs gt [B,2]. */
 int seqpan_iou_counters(const float* fracs, const float* gt_fracs, int B, double* counters, void* stream);
 
+/* Reproducible evaluation sweeps (DESIGN.md section 13).
+ * seqpan_gumbel_noise: out [B,L,4] fp32 (16-byte aligned) = Gumbel(0,1) noise of batch `batch_id` of a sweep seeded with `seed`,
+ * a function of (seed, batch_id, B, L) alone.  Philox4x32-10 with key = (seed & 0xffffffff, seed >> 32) and counter =
+ * (b * L + l, batch_id, 0, 0); its four output words x are the labels c = 0..3 of row (b, l).  u = ((x >> 9) + 0.5f) * 2^-23
+ * (exact in fp32, never 0 or 1) and out = -logf(-logf(u)) with IEEE logf.  0 <= B, B * L < 2^32, 1 <= L <= SEQPAN_MAX_VLEN.
+ * seqpan_iou_counters_exact: seqpan_iou_counters with each sample's fp64 IoU rounded to rint(iou * 2^28) * 2^-28 before it is
+ * added to the sum (the thresholds test the unrounded IoU).  Every partial sum is then an integer multiple of 2^-28, so the
+ * adds, and any later sum of such buffers, are exact in any order while the sample count stays <= 2^25; the mean IoU moves by
+ * less than 2^-29 per sample.  Both: no allocation, no host synchronisation, shape-only work split (graph-capturable). */
+int seqpan_gumbel_noise(uint64_t seed, uint32_t batch_id, int B, int L, float* out, void* stream);
+int seqpan_iou_counters_exact(const float* fracs, const float* gt_fracs, int B, double* counters, void* stream);
+
 /* Top-k spans per sample with greedy temporal NMS (infer_basic's probabilities; DESIGN.md section 11).  Candidates are the
  * spans i <= j with score sp[i]*ep[j] > 0, best first, exact ties to the lower i, then the lower j.  Each of k rounds keeps
  * the best candidate not yet kept and not suppressed: a kept (a,b) suppresses (i,j) when union > 0 and

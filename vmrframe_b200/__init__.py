@@ -7,10 +7,11 @@ from .seqpan import (BackBone, BaseFast, MultiTeacher, OneTeacher, infer_OneTeac
                      infer_BackBone, infer_MultiTeacher, infer_SeqPAN, train_engine_BackBone, train_engine_BaseFast, train_engine_MultiTeacher,
                      infer_topk, train_engine_SeqPAN, VideoEncodings)
 from .engine import (IouCounters, TopkCounters, append_ious, append_ious_topk, calculate_iou, calculate_iou_accuracy,  # noqa: F401
-                     evaluate, draw_chunks, get_i345_mi, metrics_from_counters, metrics_topk_from_counters, recall_at_k,
-                     shard_batches)
+                     evaluate, draw_chunks, get_i345_mi, gumbel_noise, metrics_from_counters, metrics_topk_from_counters,
+                     recall_at_k, shard_batches)
 
 from . import data_utils  # noqa: F401  (device versions of utils/data_utils.py's clip resampling / padding, SURVEY.md section 8 f2)
 
 __all__ = ["data_utils", "SeqPAN", "infer_SeqPAN", "train_engine_SeqPAN", "BaseFast", "infer_BaseFast", "train_engine_BaseFast", "MultiTeacher", "infer_MultiTeacher", "train_engine_MultiTeacher", "BackBone", "infer_BackBone", "train_engine_BackBone", "OneTeacher", "infer_OneTeacher", "extract_index", "infer_basic", "extract_topk", "infer_topk", "VideoEncodings", "evaluate",
-           "append_ious", "get_i345_mi", "IouCounters", "TopkCounters", "append_ious_topk", "recall_at_k", "metrics_topk_from_counters", "shard_batches", "draw_chunks"]
+           "append_ious", "get_i345_mi", "IouCounters", "TopkCounters", "append_ious_topk", "recall_at_k", "metrics_topk_from_counters", "shard_batches", "draw_chunks",
+           "gumbel_noise"]

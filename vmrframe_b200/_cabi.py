@@ -75,6 +75,8 @@ SIGNATURES = {
     "seqpan_forward_encoded": (_i, [_vp] + [_vp] * 4 + [_i] + [_vp] * 3 + [_i, _i, _i] + [_vp] * 3 + [_vp, _sz, _vp]),
     "seqpan_span_decode": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "seqpan_iou_counters": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "seqpan_iou_counters_exact": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "seqpan_gumbel_noise": (_i, [C.c_uint64, C.c_uint32, _i, _i, _vp, _vp]),
     "seqpan_span_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, C.c_float, _vp, _vp, _vp, _vp, _vp]),
     "seqpan_topk_counters": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "seqpan_h2d_ragged": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),

@@ -91,7 +91,10 @@ cudaError_t launch_build_rowmask(const float* vmask, long long nv, const float* 
                                  cudaStream_t st);
 cudaError_t launch_span_decode(const float* s, const float* e, const float* vmask, int B, int L, int64_t* si,
                                int64_t* ei, float* fracs, cudaStream_t st);
-cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, double* counters, cudaStream_t st);
+// exact: the IoU sum adds multiples of 2^-28 (order-independent, DESIGN.md section 13)
+cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, double* counters, bool exact, cudaStream_t st);
+// rows = B * L rows of 4 labels, out 16-byte aligned
+cudaError_t launch_gumbel_noise(uint64_t seed, uint32_t batch_id, uint32_t rows, float* out, cudaStream_t st);
 cudaError_t launch_span_topk(const float* s, const float* e, const float* vmask, int B, int L, int k, float thr,
                              int64_t* si, int64_t* ei, float* scores, float* fracs, cudaStream_t st);
 cudaError_t launch_topk_counters(const float* fracs, const float* gt, int B, int k, double* counters, cudaStream_t st);

@@ -3,6 +3,7 @@
 // Reference formulas: SURVEY.md Appendix A; each kernel cites the reference lines it replaces.
 #include <cstdlib>
 #include "kernels.cuh"
+#include "gumbel.cuh"
 
 #include <cuda_bf16.h>
 
@@ -1048,12 +1049,16 @@ __device__ __forceinline__ double span_iou(float g0, float g1, float p0, float p
   return iou;
 }
 
+// kExact (DESIGN.md section 13): the IoU added to the sum is rounded to a multiple of 2^-28, so every partial sum is an
+// integer multiple of 2^-28 below 2^25 and every fp64 add is exact, in any order.  The thresholds test the unrounded IoU.
+template <bool kExact>
 __global__ void iou_counters_kernel(const float* __restrict__ fracs, const float* __restrict__ gt, int B,
                                     double* __restrict__ counters) {
   double c[5] = {0, 0, 0, 0, 0};
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
     const double iou = span_iou(gt[b * 2], gt[b * 2 + 1], fracs[b * 2], fracs[b * 2 + 1]);
-    c[0] += 1.0; c[1] += iou; c[2] += iou >= 0.3; c[3] += iou >= 0.5; c[4] += iou >= 0.7;
+    c[0] += 1.0; c[1] += kExact ? rint(iou * 0x1p28) * 0x1p-28 : iou;
+    c[2] += iou >= 0.3; c[3] += iou >= 0.5; c[4] += iou >= 0.7;
   }
 #pragma unroll
   for (int k = 0; k < 5; ++k) {
@@ -1062,11 +1067,28 @@ __global__ void iou_counters_kernel(const float* __restrict__ fracs, const float
     if ((threadIdx.x & 31) == 0 && c[0] > 0) atomicAdd(counters + k, c[k]);
   }
 }
-cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, double* counters, cudaStream_t st) {
+cudaError_t launch_iou_counters(const float* fracs, const float* gt, int B, double* counters, bool exact, cudaStream_t st) {
   if (B <= 0) return cudaSuccess;
   int blocks = (B + 255) / 256;
   if (blocks > 148) blocks = 148;
-  iou_counters_kernel<<<blocks, 256, 0, st>>>(fracs, gt, B, counters);
+  if (exact)
+    iou_counters_kernel<true><<<blocks, 256, 0, st>>>(fracs, gt, B, counters);
+  else
+    iou_counters_kernel<false><<<blocks, 256, 0, st>>>(fracs, gt, B, counters);
+  return cudaGetLastError();
+}
+
+// Seeded Gumbel noise of one batch (seqpan_gumbel_noise): one thread per row (b, l) writes its four labels as one float4.
+__global__ void __launch_bounds__(256) gumbel_noise_kernel(uint64_t seed, uint32_t batch_id, uint32_t rows,
+                                                           float4* __restrict__ out) {
+  const uint32_t r = blockIdx.x * 256u + threadIdx.x;
+  if (r >= rows) return;
+  const uint4 x = gumbel_words(seed, batch_id, r);
+  out[r] = make_float4(gumbel_of(x.x), gumbel_of(x.y), gumbel_of(x.z), gumbel_of(x.w));
+}
+cudaError_t launch_gumbel_noise(uint64_t seed, uint32_t batch_id, uint32_t rows, float* out, cudaStream_t st) {
+  if (rows == 0) return cudaSuccess;
+  gumbel_noise_kernel<<<(unsigned)(((uint64_t)rows + 255) / 256), 256, 0, st>>>(seed, batch_id, rows, reinterpret_cast<float4*>(out));
   return cudaGetLastError();
 }
 

@@ -1059,7 +1059,26 @@ extern "C" int seqpan_span_decode(const float* slogits, const float* elogits, co
 
 extern "C" int seqpan_iou_counters(const float* fracs, const float* gt_fracs, int B, double* counters, void* stream) {
   if (!fracs || !gt_fracs || !counters) return fail(SEQPAN_E_INVALID, "NULL argument");
-  CK(launch_iou_counters(fracs, gt_fracs, B, counters, (cudaStream_t)stream));
+  CK(launch_iou_counters(fracs, gt_fracs, B, counters, false, (cudaStream_t)stream));
+  return SEQPAN_OK;
+}
+
+extern "C" int seqpan_iou_counters_exact(const float* fracs, const float* gt_fracs, int B, double* counters, void* stream) {
+  if (!fracs) return fail(SEQPAN_E_INVALID, "fracs is NULL");
+  if (!gt_fracs) return fail(SEQPAN_E_INVALID, "gt_fracs is NULL");
+  if (!counters) return fail(SEQPAN_E_INVALID, "counters is NULL");
+  if (B < 0) return fail(SEQPAN_E_INVALID, "B=%d < 0", B);
+  CK(launch_iou_counters(fracs, gt_fracs, B, counters, true, (cudaStream_t)stream));
+  return SEQPAN_OK;
+}
+
+extern "C" int seqpan_gumbel_noise(uint64_t seed, uint32_t batch_id, int B, int L, float* out, void* stream) {
+  if (!out) return fail(SEQPAN_E_INVALID, "out is NULL");
+  if ((uintptr_t)out & 15) return fail(SEQPAN_E_INVALID, "out must be 16-byte aligned (one float4 per row)");
+  if (B < 0) return fail(SEQPAN_E_INVALID, "B=%d < 0", B);
+  if (L < 1 || L > SEQPAN_MAX_VLEN) return fail(SEQPAN_E_INVALID, "L=%d outside [1,%d]", L, SEQPAN_MAX_VLEN);
+  if ((int64_t)B * L > (int64_t)UINT32_MAX) return fail(SEQPAN_E_INVALID, "B=%d: B*L rows exceed the 32-bit counter word", B);
+  CK(launch_gumbel_noise(seed, batch_id, (uint32_t)((int64_t)B * L), out, (cudaStream_t)stream));
   return SEQPAN_OK;
 }
 

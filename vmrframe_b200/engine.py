@@ -13,6 +13,7 @@ replicated, there is no collective in the forward, and one all-reduce(sum) of th
 """
 from __future__ import annotations
 
+import operator
 import time
 
 import numpy as np
@@ -55,18 +56,21 @@ def metrics_from_counters(counters):
 
 
 class IouCounters:
-    """Device-side IoU counters (seqpan_iou_counters): no host loop, no sync until ``.result()``."""
+    """Device-side IoU counters (seqpan_iou_counters): no host loop, no sync until ``.result()``.  ``exact=True``
+    (seqpan_iou_counters_exact, DESIGN.md section 13) adds each IoU rounded to a multiple of 2^-28, so the sum is the same
+    bits in any order of samples, calls, streams and ranks (up to 2^25 samples in all)."""
 
-    def __init__(self, device):
+    def __init__(self, device, exact: bool = False):
+        self.exact = bool(exact)
         self.buf = torch.zeros(5, dtype=torch.float64, device=device)
 
     def update(self, fracs: torch.Tensor, gt_fracs: torch.Tensor):
         dev = self.buf.device
         fr = fracs.to(device=dev, dtype=torch.float32).contiguous()
         gt = gt_fracs.to(device=dev, dtype=torch.float32).contiguous()
+        fn = _cabi.lib().seqpan_iou_counters_exact if self.exact else _cabi.lib().seqpan_iou_counters
         with torch.cuda.device(dev):
-            _cabi.check(_cabi.lib().seqpan_iou_counters(fr.data_ptr(), gt.data_ptr(), fr.shape[0], self.buf.data_ptr(),
-                                                        torch.cuda.current_stream(dev).cuda_stream))
+            _cabi.check(fn(fr.data_ptr(), gt.data_ptr(), fr.shape[0], self.buf.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
 
     def allreduce(self):
         """Sum over ranks: the only collective of the sharded sweep (NCCL on GPUs)."""
@@ -174,6 +178,75 @@ def allreduce_counters_cpu(counters: torch.Tensor) -> torch.Tensor:
     return counters
 
 
+# ---- seeded sweeps (DESIGN.md section 13) ----------------------------------------------------------------------
+EXACT_MAX_SAMPLES = 1 << 25   # the exact IoU sums stay exact up to this many samples
+
+
+def _check_seed(seed) -> int:
+    if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)):
+        raise ValueError(f"seed must be an int in [0, 2^64), got {seed!r}")
+    if not 0 <= int(seed) < 1 << 64:
+        raise ValueError(f"seed={seed} outside [0, 2^64)")
+    return int(seed)
+
+
+def _check_batch_id(i) -> int:
+    try:
+        if isinstance(i, bool):
+            raise TypeError
+        i = operator.index(i)
+    except TypeError:
+        raise ValueError(f"batch ids must be integers, got {i!r}") from None
+    if not 0 <= i < 1 << 32:
+        raise ValueError(f"batch id {i} outside [0, 2^32)")
+    return i
+
+
+def _resolve_device(device) -> torch.device:
+    device = torch.device(device or "cuda")
+    if device.index is None:     # "cuda" = the current device; the handles and the parameters compare full device names
+        device = torch.device("cuda", torch.cuda.current_device())
+    return device
+
+
+def _sweep_ids(batches, seed, batch_ids):
+    """``(seed, one id per batch)`` of a seeded sweep after the argument checks of :func:`evaluate`; ``(None, None)`` without
+    a seed."""
+    if seed is None:
+        if batch_ids is not None:
+            raise ValueError("batch_ids name the noise of a seeded sweep: pass seed= too")
+        return None, None
+    seed = _check_seed(seed)
+    ids = list(range(len(batches))) if batch_ids is None else [_check_batch_id(i) for i in batch_ids]
+    if len(ids) != len(batches):
+        raise ValueError(f"{len(ids)} batch ids for {len(batches)} batches")
+    if len(set(ids)) != len(ids):
+        raise ValueError("duplicate batch ids: two batches would get the same noise")
+    n = sum(int(b["vmasks"].shape[0]) for b in batches)
+    if n > EXACT_MAX_SAMPLES:
+        raise ValueError(f"{n} samples in one seeded call: the exact IoU sum holds up to 2^25")
+    return seed, ids
+
+
+def gumbel_noise(B: int, L: int, seed: int, batch_id: int, device=None) -> torch.Tensor:
+    """The Gumbel noise ``[B, L, 4]`` fp32 that ``evaluate(seed=seed)`` uses for the batch with id ``batch_id``
+    (seqpan_gumbel_noise, DESIGN.md section 13): a function of ``(seed, batch_id, B, L)`` alone.  Pass it as
+    ``forward(..., gumbel=)`` to reproduce one batch of a seeded sweep.  ``device`` defaults to the current CUDA device."""
+    seed, batch_id = _check_seed(seed), _check_batch_id(batch_id)
+    B, L = int(B), int(L)
+    if B < 0:
+        raise ValueError(f"B={B} < 0")
+    _cabi.require_device()
+    device = _resolve_device(device)
+    out = torch.empty(B, L, 4, dtype=torch.float32, device=device)
+    if B == 0:
+        return out
+    with torch.cuda.device(device):
+        _cabi.check(_cabi.lib().seqpan_gumbel_noise(seed, batch_id, B, L, out.data_ptr(),
+                                                    torch.cuda.current_stream(device).cuda_stream))
+    return out
+
+
 # ---- pipelined evaluation sweep (the public e2e call) -----------------------------------------------------
 _INPUT_KEYS = ("words_ids", "char_ids", "vfeats", "vmasks", "tmasks", "se_fracs")
 
@@ -215,7 +288,8 @@ class _Slot:
 
 def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: bool = False, streams: int = 2,
              ragged_h2d: bool = True, h2d_ctas: int = 32, profile: bool = False, check_padding: bool | None = None,
-             allreduce: bool = True, topk: int | None = None, nms_thresh: float = 0.5, video_encodings=None):
+             allreduce: bool = True, topk: int | None = None, nms_thresh: float = 0.5, video_encodings=None,
+             seed: int | None = None, batch_ids=None):
     """Runs forward + span decode + IoU counters over an iterable of HOST batches (dicts in ``BaseCollate``'s key
     naming, ideally pinned) -- the eval loop of ``main.py:112-134`` as one pipelined call.
 
@@ -245,20 +319,26 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
     ``info["h2d_bytes"]`` counts ids, masks, ground truth and indices only.  Results equal the sweep over the raw clips with the
     same ``video_index``.  Under ``torchrun`` every rank encodes the clips its batches use onto its own device (encodings are
     device memory and are not shared between ranks).
+    ``seed`` (an int in ``[0, 2^64)``; DESIGN.md section 13) makes the sweep reproducible: batch ``i`` gets the Gumbel noise
+    :func:`gumbel_noise` ``(B, L, seed, batch_ids[i])`` instead of a draw from torch's generator, and the IoU counters add
+    exactly (``IouCounters(exact=True)``), so counters, metrics and spans are the same bits however the batches are split
+    over streams, calls, ranks and work-queue schedules.  ``batch_ids`` (default ``range(len(batches))``) are the batches'
+    global ids: a caller that shards passes ``shard_batches(...)`` or the ranges ``draw_chunks`` yields.  Ids must be distinct
+    and in ``[0, 2^32)``, and one call (and, after the all-reduce, the whole sweep) holds at most 2^25 samples.
+    ``info["seed"]`` records the seed.  Without a seed the sweep makes exactly the calls it always made.
     """
+    batches = list(host_batches)
+    seed, batch_ids = _sweep_ids(batches, seed, batch_ids)
     _cabi.require_device()
     if topk is not None:
         topk = int(topk)
         if not (1 <= topk <= 32 and 0.0 < nms_thresh <= 1.0):
             raise ValueError(f"topk={topk} must be in [1,32] and nms_thresh={nms_thresh} in (0,1]")
-    device = torch.device(device or "cuda")
-    if device.index is None:     # "cuda" = the current device; the handles and the parameters compare full device names
-        device = torch.device("cuda", torch.cuda.current_device())
+    device = _resolve_device(device)
     L_ = _cabi.lib()
     import os
     if check_padding is None:
         check_padding = os.environ.get("SEQPAN_CHECK_PADDING") == "1"
-    batches = list(host_batches)
     enc = video_encodings
     if enc is not None:
         model._check_encoded_call(enc, None, None)
@@ -276,7 +356,8 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                 raise _cabi.SeqpanError(f"batch {i} has no video_index and {B} pairs > {len(enc)} encoded clips")
     main = torch.cuda.current_stream(device)
     nstreams = max(1, int(streams))
-    counters = IouCounters(device)
+    counters = IouCounters(device, exact=seed is not None)
+    iou_counters = L_.seqpan_iou_counters_exact if counters.exact else L_.seqpan_iou_counters
     tk = None
     if topk is not None:   # one fp64 buffer [5 IoU counters | 4 R@k counters]: one all-reduce for both
         joint = torch.zeros(9, dtype=torch.float64, device=device)
@@ -290,6 +371,8 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
         info = {"h2d_bytes": 0, "d2h_bytes": 0, "wall_s": 0.0, "batches": 0}
         if tk is not None:
             info["topk"] = topk_info()
+        if seed is not None:
+            info["seed"] = seed
         return counters.result(), counters.buf, info
     lanes = [main] + [torch.cuda.Stream(device) for _ in range(nstreams - 1)]
     copy_stream = torch.cuda.Stream(device)
@@ -396,17 +479,19 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                     if profile:
                         prof[i][2].record(lane)
                     model.use_context(i % nstreams)
-                    # == F.gumbel_softmax's draw (models/SeqPAN.py:79): -empty_like(logits).exponential_().log()
-                    v["gumbel"].exponential_().log_().neg_()
-                    model.forward_into(v["words"], v["chars"], v["vfeats"], v["vmask"], v["tmask"], v["gumbel"],
-                                       v["slogits"], v["elogits"], v["match"], v["vindex"], video_encodings=enc)
                     B = v["vmask"].shape[0]
                     st = lane.cuda_stream
+                    if seed is None:
+                        # == F.gumbel_softmax's draw (models/SeqPAN.py:79): -empty_like(logits).exponential_().log()
+                        v["gumbel"].exponential_().log_().neg_()
+                    else:
+                        _cabi.check(L_.seqpan_gumbel_noise(seed, batch_ids[i], B, Lv, v["gumbel"].data_ptr(), st))
+                    model.forward_into(v["words"], v["chars"], v["vfeats"], v["vmask"], v["tmask"], v["gumbel"],
+                                       v["slogits"], v["elogits"], v["match"], v["vindex"], video_encodings=enc)
                     _cabi.check(L_.seqpan_span_decode(v["slogits"].data_ptr(), v["elogits"].data_ptr(), v["vmask"].data_ptr(),
                                                       B, Lv, None, None, v["fracs"].data_ptr(), st))
                     if v["gt"] is not None:
-                        _cabi.check(L_.seqpan_iou_counters(v["fracs"].data_ptr(), v["gt"].data_ptr(), B,
-                                                           counters.buf.data_ptr(), st))
+                        _cabi.check(iou_counters(v["fracs"].data_ptr(), v["gt"].data_ptr(), B, counters.buf.data_ptr(), st))
                     host_fracs[i, :B].copy_(v["fracs"], non_blocking=True)     # device -> host read of the step's result
                     d2h += B * 2 * 4
                     if tk is not None:
@@ -435,6 +520,8 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
                 else:
                     _allreduce_sum(joint)
             metrics = counters.result()  # synchronises
+            if seed is not None and allreduce and float(counters.buf[0]) > EXACT_MAX_SAMPLES:
+                raise ValueError(f"{int(counters.buf[0])} samples over all ranks: the exact IoU sum holds up to 2^25")
     finally:
         model.use_context(was_ctx)
         model.sync_timing = was_sync
@@ -444,6 +531,8 @@ def evaluate(model, host_batches, device=None, depth: int = 2, return_fracs: boo
             "batches": len(batches)}
     if tk is not None:
         info["topk"] = topk_info()
+    if seed is not None:
+        info["seed"] = seed
     if profile:
         info["copy_ms"] = [p[0].elapsed_time(p[1]) for p in prof]
         info["compute_ms"] = [p[2].elapsed_time(p[3]) for p in prof]
