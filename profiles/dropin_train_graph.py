@@ -54,23 +54,20 @@ class Route:
         self.ts = train._train_step_of(self.m)
         if not graph:
             self.ts.max_graphs = 0
-        replay = self.ts._replay_part1
-
-        def counted(*a, **k):
-            self.hits += "graph" in a[0]
-            return replay(*a, **k)
-        self.ts._replay_part1 = counted
 
     def step(self, bd):
         self.calls += 1
         if self.kind == "trainstep":
             return self.ts.step(bd, graph=True)[0]
         if self.kind == "engine":
+            captured = [e for e in self.ts._graphs.values() if "graph" in e]
             loss, _ = train_engine_SeqPAN(self.m, bd, self.cfg, "train")
+            used = next(reversed(self.ts._graphs.values()))          # the entry of this call: replayed if captured before it
+            self.hits += any(e is used for e in captured)
         else:
             out = self.m(bd["words_ids"], bd["char_ids"], bd["vfeats"], bd["vmasks"], bd["tmasks"])
             rec = out["slogits"].grad_fn.rec
-            self.hits += isinstance(rec, train._InFlight) and bool(rec.ent["bwd"])     # forward and backward both replay
+            self.hits += isinstance(rec, train._InFlight) and bool(rec.ent.get("bwd"))     # forward and backward both replay
             del rec
             loss = lossfun_loc(out["slogits"], out["elogits"], bd["label1ds"][:, 0, :], bd["label1ds"][:, 1, :], bd["vmasks"]) + \
                 lossfun_match(out["match_score"], out["label_embs"], bd["NER_labels"], bd["vmasks"])

@@ -920,21 +920,7 @@ def train_engine_SeqPAN(model, data, configs, runtype=None):
     training kernels (vmrframe_b200/train.py); the returned ``loss`` is attached to the parameters, so the reference's
     ``optimizer.zero_grad(); loss.backward(); clip_grad_norm_(...); optimizer.step()`` works unchanged.
     ``model.eval()`` (main.py:112-127): the fused inference forward; the loss is a value without a graph."""
-    from .engine import lossfun_loc, lossfun_match
-    data = {k: v.to(configs.device) for k, v in data.items()}
-    if model.training and "label1ds" in data and "NER_labels" in data:
-        from . import train as _train
-        start = time.time()
-        loss, output = _train.tape_loss(model, data)
-        output["consume_time"] = time.time() - start
-        return loss, output
-    output = model(data["words_ids"], data["char_ids"], data["vfeats"], data["vmasks"], data["tmasks"])
-    loss = None
-    if "label1ds" in data and "NER_labels" in data:
-        loss = lossfun_loc(output["slogits"], output["elogits"], data["label1ds"][:, 0, :], data["label1ds"][:, 1, :],
-                           data["vmasks"]) + lossfun_match(output["match_score"], output["label_embs"],
-                                                           data["NER_labels"], data["vmasks"])
-    return loss, output
+    return _train_engine_on_tape(model, data, configs, "train", _LABELS, _reference_loss)
 
 
 def infer_BaseFast(output, configs=None):
@@ -946,37 +932,43 @@ def train_engine_BaseFast(model, data, configs, runtype=None):
     """models/BaseFast.py:113-127: like ``train_engine_SeqPAN`` but the location loss sees ``sigmoid(logits)`` (``:119-120``).
     ``model.train()``: forward, losses and backward on the training kernels (``loss.backward()`` hands out the gradients);
     ``model.eval()``: fused inference forward, loss value only."""
+    return _train_engine_on_tape(model, data, configs, "train", _LABELS,
+                                 lambda output, data: _reference_loss(output, data, sigmoid_first=True))
+
+
+_LABELS = ("label1ds", "NER_labels")      # what train_engine_SeqPAN / _BaseFast compute their losses from
+
+
+def _reference_loss(output, data, sigmoid_first=False):
+    """The loss value of ``train_engine_SeqPAN`` / ``_BaseFast`` on the inference outputs: ``engine.lossfun_loc`` (on
+    ``sigmoid(logits)`` with ``sigmoid_first``) + ``lossfun_match`` in torch."""
     from .engine import lossfun_loc, lossfun_match
-    data = {k: v.to(configs.device) for k, v in data.items()}
-    if model.training and "label1ds" in data and "NER_labels" in data:
-        from . import train as _train
-        start = time.time()
-        loss, output = _train.tape_loss(model, data)
-        output["consume_time"] = time.time() - start
-        return loss, output
-    output = model(data["words_ids"], data["char_ids"], data["vfeats"], data["vmasks"], data["tmasks"])
-    loss = None
-    if "label1ds" in data and "NER_labels" in data:
-        loss = lossfun_loc(torch.sigmoid(output["slogits"]), torch.sigmoid(output["elogits"]), data["label1ds"][:, 0, :],
-                           data["label1ds"][:, 1, :], data["vmasks"]) + lossfun_match(
-                               output["match_score"], output["label_embs"], data["NER_labels"], data["vmasks"])
-    return loss, output
+    s, e = output["slogits"], output["elogits"]
+    if sigmoid_first:
+        s, e = torch.sigmoid(s), torch.sigmoid(e)
+    return lossfun_loc(s, e, data["label1ds"][:, 0, :], data["label1ds"][:, 1, :], data["vmasks"]) + lossfun_match(
+        output["match_score"], output["label_embs"], data["NER_labels"], data["vmasks"])
 
 
-def _train_engine_on_tape(model, data, configs, runtype):
-    """Common body of the train engines of the sibling models: ``model.train()`` -> forward, the model's loss terms and the
-    backward on the training kernels (``loss.backward()`` hands out the gradients); ``model.eval()`` -> fused inference forward
-    and the loss VALUE from the same loss kernels."""
+def _train_engine_on_tape(model, data, configs, runtype, labels=(), eval_loss=None):
+    """Common body of the train engines: moves the batch to ``configs.device``; ``model.train()`` -> forward, the model's loss
+    terms and the backward on the training kernels (``loss.backward()`` hands out the gradients); ``model.eval()`` -> fused
+    inference forward and the loss VALUE, ``eval_loss(output, data)`` or else from the same loss kernels as the tape.  A batch
+    without one of the keys ``labels`` runs the module's forward in either mode and has no loss."""
     from . import train as _train
     data = {k: v.to(configs.device) for k, v in data.items()}
     runtype = "train" if runtype is None else runtype
-    if model.training:
+    labelled = all(k in data for k in labels)
+    if model.training and labelled:
         start = time.time()
         loss, output = _train.tape_loss(model, data, runtype=runtype)
         output["consume_time"] = time.time() - start
         return loss, output
     output = model(data["words_ids"], data["char_ids"], data["vfeats"], data["vmasks"], data["tmasks"])
-    return _train.loss_from_outputs(model, output, data, runtype), output
+    if not labelled:
+        return None, output
+    loss = eval_loss(output, data) if eval_loss is not None else _train.loss_from_outputs(model, output, data, runtype)
+    return loss, output
 
 
 def train_engine_MultiTeacher(model, data, configs, runtype=None):

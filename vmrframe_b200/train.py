@@ -61,6 +61,31 @@ def _capture(graph, pool=None):
             gc.enable()
 
 
+def _due(ent):
+    """Whether a graph entry is due for capture (or holds its graph): after two eager runs of its key, when the lazy state of a
+    run (Adam moments, the gradient bucket, the backend's caches) exists."""
+    return ent["seen"] >= 2
+
+
+def _replay(ent, fn, data, gumbel):
+    """``fn(data, gumbel)`` replayed from the entry's CUDA graph, captured on first use.  The inputs (a dict of tensors) and the
+    Gumbel draw are staged into static clones at the capture and copied in before every replay; the dropout draws stay fresh
+    (torch's graph-safe generator).  Returns what ``fn`` returned at the capture, which the replay overwrites in place."""
+    if "graph" not in ent:
+        ent["in"] = {k: v.detach().clone() for k, v in data.items()}
+        ent["gum"] = gumbel.clone() if gumbel is not None else None
+        g = torch.cuda.CUDAGraph()
+        with _capture(g):
+            ent["out"] = fn(ent["in"], ent["gum"])
+        ent["graph"] = g
+    for k, v in data.items():
+        ent["in"][k].copy_(v, non_blocking=True)
+    if gumbel is not None:
+        ent["gum"].copy_(gumbel, non_blocking=True)
+    ent["graph"].replay()
+    return ent["out"]
+
+
 def _check_precision(precision):
     if precision not in PRECISIONS:
         raise ValueError(f"training precision {precision!r}: expected one of {PRECISIONS}")
@@ -705,7 +730,7 @@ def _text_embedding(tp, P, word_ids, char_ids):
         w = tp.embedding(P[p + ".word_emb.word_emb.weight"], word_ids.reshape(-1).contiguous())
         w = tp.reshape(w, (B, T, -1))
         # nn.Embedding(padding_idx=0): row 0 receives no gradient -- the ids are never 0 for real words and the pad rows'
-        # output gradient is scattered into row 0, which the optimizer step must ignore (handled in TrainStep)
+        # output gradient is scattered into row 0, which the optimizer step must ignore (_zero_pad_rows)
     w = tp.dropout(w)
     ce = tp.embedding(P[p + ".char_emb.char_emb.weight"], char_ids.reshape(-1).contiguous())     # [B*T*C, 100]
     ce = tp.dropout(ce)
@@ -950,6 +975,29 @@ def train_spec(model):
     return _TRAIN_SPECS[name]
 
 
+def _record_forward(model, be, named, inputs, gumbel, precision, training, mask_fn=None, needs_x=False):
+    """The model's training forward recorded on a new tape: ``inputs`` are ``(word_ids, char_ids, vfeat_in, vmask, tmask)``,
+    ``named`` the parameters by name (those that require grad receive a gradient), and ``vfeat_in`` receives one when
+    ``needs_x``.  The tape reduces in a fixed order while :func:`deterministic_mode` is on.  Returns ``(tape, params, video
+    leaf, (slogits, elogits, match_score or None))``."""
+    tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=training, mask_fn=mask_fn, precision=precision,
+                    deterministic=deterministic_mode())
+    P = _Params(tp, named)
+    word_ids, char_ids, vfeat_in, vmask, tmask = inputs
+    xv = tp.leaf(vfeat_in, needs=needs_x)
+    return tp, P, xv, forward_train(tp, P, word_ids, char_ids, xv, vmask, tmask, gumbel, **train_spec(model)["fwd"])
+
+
+_EMB_PAD_ROW = ("text_encoder.char_emb.char_emb.weight", "text_encoder.word_emb.word_emb.weight")
+
+
+def _zero_pad_rows(P):
+    """nn.Embedding(padding_idx=0): row 0 of the embedding tables gets no gradient."""
+    for k in _EMB_PAD_ROW:
+        if P.has(k) and P[k].g is not None:
+            P[k].g[0].zero_()
+
+
 # ---- losses (models/loss.py:24-54) -------------------------------------------------------------------------------------
 def loss_loc(tp, slogits, elogits, s_labels, e_labels, sigmoid_first=False):
     """``nn.CrossEntropyLoss(reduction='mean')`` with soft ``[B,L]`` targets on the UNMASKED logits, start + end.
@@ -1088,21 +1136,14 @@ class TrainStep:
 
     def loss_and_grads(self, data, gumbel=None):
         """Forward + both losses + backward.  Returns ``(loss tensor (device scalar), {name: grad}, outputs)``."""
-        be = self.be
         m = self.model
-        tp = SeqpanTape(be, droprate=m.configs.model.droprate, training=m.training, mask_fn=self.mask_fn, precision=self.precision,
-                        deterministic=deterministic_mode())
-        P = _Params(tp, self.named)
         vmask, tmask = data["vmasks"].to(torch.float32), data["tmasks"].to(torch.float32)
-        spec = train_spec(m)
-        sl, el, ms = forward_train(tp, P, data["words_ids"], data["char_ids"], data["vfeats"], vmask, tmask, gumbel, **spec["fwd"])
-        loss = compose_loss(tp, m, sl, el, ms, P["label_embs"] if spec["match_loss"] else None, data, vmask, self.runtype)
+        tp, P, _, (sl, el, ms) = _record_forward(m, self.be, self.named, (data["words_ids"], data["char_ids"], data["vfeats"], vmask,
+                                                                          tmask), gumbel, self.precision, m.training, self.mask_fn)
+        loss = compose_loss(tp, m, sl, el, ms, P["label_embs"] if train_spec(m)["match_loss"] else None, data, vmask, self.runtype)
         tp.backward(loss, torch.ones((), dtype=torch.float32, device=vmask.device))
+        _zero_pad_rows(P)
         grads = {k: v.g for k, v in P.vars.items() if v.g is not None}
-        if "text_encoder.char_emb.char_emb.weight" in grads:          # nn.Embedding(padding_idx=0): row 0 gets no gradient
-            grads["text_encoder.char_emb.char_emb.weight"][0].zero_()
-        if "text_encoder.word_emb.word_emb.weight" in grads:
-            grads["text_encoder.word_emb.word_emb.weight"][0].zero_()
         out = {"slogits": sl.v, "elogits": el.v, "vmask": data["vmasks"]}
         if ms is not None:
             out.update(match_score=ms.v, label_embs=m.label_embs)
@@ -1180,12 +1221,12 @@ class TrainStep:
         return ent
 
     def _use_graph(self, ent):
-        """Whether ``ent`` replays (and is captured first if need be): after two eager runs, and when a capture fits.  At most
+        """Whether ``ent`` replays (and is captured first if need be): once :func:`_due`, and when a capture fits.  At most
         ``max_graphs`` entries hold graphs; the least recently used one without a forward in flight gives its graphs and pool
         up (its eager count stays).  When every capture holds a forward in flight the call runs eagerly."""
         if "graph" in ent:
             return True
-        if ent["seen"] < 2:
+        if not _due(ent):
             return False
         captured = [e for e in self._graphs.values() if "graph" in e]
         while len(captured) >= self.max_graphs:
@@ -1197,34 +1238,17 @@ class TrainStep:
                 del old[k]
         return True
 
-    def _replay_part1(self, ent, data, gumbel, relayout=False):
-        """``_part1`` from the entry's graph, captured on first use.  Inputs are copied into static buffers; the dropout / Gumbel
-        draws stay fresh (torch's graph-safe generator).  The entry keeps the bucket its graph writes."""
-        if "graph" not in ent:
-            ent["in"] = {k: v.clone() for k, v in data.items()}
-            ent["gum"] = gumbel.clone() if gumbel is not None else None
-            g = torch.cuda.CUDAGraph()
-            with _capture(g):
-                ent["out"] = self._part1(ent["in"], ent["gum"], relayout)
-            ent["bucket"] = (self.flat, self.live)
-            ent["graph"] = g
-        for k, v in data.items():
-            ent["in"][k].copy_(v, non_blocking=True)
-        if gumbel is not None:
-            ent["gum"].copy_(gumbel, non_blocking=True)
-        ent["graph"].replay()
-        return ent["out"]
-
     def _engine_loss_and_grads(self, data, gumbel):
         """``loss_and_grads`` of the train engines, replayed from a CUDA graph from the third call with the same key on.  A
         replay hands out views of a fresh copy of the entry's bucket and fresh copies of the outputs: they outlive the next
-        replay, so gradients of two calls can be accumulated before one backward."""
+        replay, so gradients of two calls can be accumulated before one backward.  The entry keeps the bucket its graph
+        writes (a later eager call may lay out a new one)."""
         ent = self._entry(self._graph_key("loss", data, gumbel, self.precision, self.runtype))
         if not self._use_graph(ent):
             ent["seen"] += 1
             return self.loss_and_grads(data, gumbel)
-        loss, out = self._replay_part1(ent, data, gumbel, relayout=True)
-        flat, live = ent["bucket"]
+        loss, out, (flat, live) = _replay(ent, lambda d, g: (*self._part1(d, g, relayout=True), (self.flat, self.live)),
+                                          data, gumbel)
         grads = dict(zip(live, flat.clone().split([self.named[k].numel() for k in live])))
         out = {k: (v.clone() if k in ("slogits", "elogits", "match_score") else v) for k, v in out.items()}
         out["vmask"] = data["vmasks"]
@@ -1255,24 +1279,18 @@ class TrainStep:
             ss = self._part2(world, det)
         else:
             ent = self._entry(self._graph_key("step", data, gumbel, self.precision, self.runtype))
-            if not self._use_graph(ent):                   # two eager steps first: lazy state (Adam moments, bucket, caches) exists
+            if self._use_graph(ent):
+                loss, out = _replay(ent, self._part1, data, gumbel)
+            else:
                 ent["seen"] += 1
                 loss, out = self._part1(data, gumbel)
-            else:
-                loss, out = self._replay_part1(ent, data, gumbel)
             world = self._allreduce()
-            e2 = self._g2.setdefault(det, {"seen": 0})
-            if "graph" not in e2 and e2["seen"] < 2:
+            e2 = self._g2.setdefault(det, {"seen": 0})     # outside the LRU cache and never evicted: it holds no activations
+            if _due(e2):
+                ss = _replay(e2, lambda d, g: self._part2(world, det), {}, None)
+            else:
                 e2["seen"] += 1
                 ss = self._part2(world, det)
-            else:
-                if "graph" not in e2:
-                    g2 = torch.cuda.CUDAGraph()
-                    with _capture(g2):
-                        e2["out"] = self._part2(world, det)
-                    e2["graph"] = g2
-                e2["graph"].replay()
-                ss = e2["out"]
         if hasattr(self.model, "repack"):
             self.model.repack()           # the inference handle's packed weights follow the update (p.data edits bump no version)
         return loss, out, ss              # ss: squared gradient norm before clipping (device fp64 scalar)
@@ -1329,17 +1347,15 @@ def _can_capture(be, x, mask_fn=None):
 
 
 # ---- the training forward as one torch autograd node: any torch loss on its outputs backpropagates through the tape ----------
-_EMB_PAD_ROW = ("text_encoder.char_emb.char_emb.weight", "text_encoder.word_emb.word_emb.weight")
-
-
 class _Recording:
-    """What the node's backward needs: the tape, its output Vars, the video leaf and the parameter Vars.  The tape's nodes are
-    closures over the tape (a reference cycle); clearing them when the recording dies lets reference counting free a forward
-    that is never backpropagated as soon as its outputs are dropped, as it frees :func:`forward_only`'s."""
-    __slots__ = ("tp", "outs", "xv", "P")
+    """What the node's backward needs: the tape, its nodes as the forward left them, its output Vars, the video leaf and the
+    parameter Vars.  The tape's nodes are closures over the tape (a reference cycle); clearing them when the recording dies
+    lets reference counting free a forward that is never backpropagated as soon as its outputs are dropped, as it frees
+    :func:`forward_only`'s."""
+    __slots__ = ("tp", "nodes", "outs", "xv", "P")
 
-    def __init__(self, tp, outs, xv, P):
-        self.tp, self.outs, self.xv, self.P = tp, outs, xv, P
+    def __init__(self, tp, P, xv, outs):
+        self.tp, self.nodes, self.outs, self.xv, self.P = tp, tp.nodes, [o for o in outs if o is not None], xv, P
 
     def __del__(self):
         self.tp.nodes = []
@@ -1358,43 +1374,34 @@ class _InFlight:
         self.ent["busy"] = False
 
 
-def _capture_node_forward(ent, model, be, inputs, gumbel, named, needs_x):
-    """Record the training forward of the node inside a CUDA graph; the tape, its nodes and the static inputs stay with
-    the entry, so that backward graphs can be captured from the same recording."""
-    ent["in"] = [t.detach().clone() for t in inputs]
-    ent["gum"] = gumbel.clone() if gumbel is not None else None
-    g = torch.cuda.CUDAGraph()
-    with _capture(g):
-        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model),
-                        deterministic=deterministic_mode())
-        P = _Params(tp, named)
-        w, c, vm, tm, x = ent["in"]
-        xv = tp.leaf(x, needs=needs_x)
-        outs = [o for o in forward_train(tp, P, w, c, xv, vm, tm, ent["gum"], **train_spec(model)["fwd"]) if o is not None]
-    ent.update(graph=g, rec=_Recording(tp, outs, xv, P), nodes=list(tp.nodes), bwd={})
+def _node_backward(rec, gouts, names):
+    """The tape's adjoints from the node's outputs with cotangents ``gouts`` (None: unused); returns the gradients of
+    ``vfeat_in`` and of the parameters ``names``, None where there is none.  A recording swept before (a graph entry's, whose
+    backward is captured once per pattern of None cotangents) gets its nodes back and the gradient state that sweep left
+    cleared."""
+    if rec.tp.nodes is not rec.nodes:
+        for o, inputs, _ in rec.nodes:
+            for v in (o, *inputs):
+                v.g, v.own = None, False
+        rec.tp.nodes = rec.nodes
+    rec.tp.backward(list(zip(rec.outs, gouts)))
+    _zero_pad_rows(rec.P)
+    return [rec.xv.g] + [rec.P[k].g for k in names]
 
 
 def _graphed_node_backward(ent, gouts, names):
-    """The node's backward from a graph per pattern of cotangents (which are None): the backward issues different kernels for
-    each.  A graph is captured from the entry's recording on first use, in the forward graph's pool.  Cotangents are copied
-    into static buffers (which makes expanded views contiguous); the gradients handed back are fresh copies."""
+    """:func:`_node_backward` from a graph per pattern of cotangents (which are None): the backward issues different kernels
+    for each.  A graph is captured from the entry's recording on first use, in the forward graph's pool.  Cotangents are
+    copied into static buffers (which makes expanded views contiguous); the gradients handed back are fresh copies."""
+    bwd = ent.setdefault("bwd", {})
     bkey = tuple(g is not None for g in gouts)
-    if bkey not in ent["bwd"]:
-        rec = ent["rec"]
+    if bkey not in bwd:
         static = [None if g is None else torch.empty(g.shape, dtype=torch.float32, device=g.device) for g in gouts]
-        for o, inputs, _ in ent["nodes"]:            # the gradient state an earlier capture left on the tape's Vars
-            for v in (o, *inputs):
-                v.g, v.own = None, False
-        rec.tp.nodes = list(ent["nodes"])
         gb = torch.cuda.CUDAGraph()
         with _capture(gb, pool=ent["graph"].pool()):
-            rec.tp.backward(list(zip(rec.outs, static)))
-            grads = [rec.xv.g] + [rec.P[k].g for k in names]
-            for k in _EMB_PAD_ROW:
-                if k in rec.P.vars and rec.P[k].g is not None:
-                    rec.P[k].g[0].zero_()
-        ent["bwd"][bkey] = (gb, static, grads)
-    gb, static, grads = ent["bwd"][bkey]
+            grads = _node_backward(ent["out"], static, names)
+        bwd[bkey] = (gb, static, grads)
+    gb, static, grads = bwd[bkey]
     for s, g in zip(static, gouts):
         if s is not None:
             s.copy_(g)
@@ -1418,28 +1425,21 @@ class _TapeForward(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, be, slot, word_ids, char_ids, vmask, tmask, gumbel, vfeat_in, names, *params):
         ctx.set_materialize_grads(False)          # an output nobody used arrives as None and costs nothing
-        ctx.names, ctx.shapes = names, [p.shape for p in params]
+        ctx.names, ctx.shapes = names, [vfeat_in.shape] + [p.shape for p in params]
         ent, graphed = slot if slot is not None else (None, False)
         ctx.ent = ent
+        data = {"words_ids": word_ids, "char_ids": char_ids, "vmasks": vmask, "tmasks": tmask, "vfeats": vfeat_in}
+
+        def record(d, gum):
+            inputs = (d["words_ids"], d["char_ids"], d["vfeats"], d["vmasks"], d["tmasks"])
+            return _Recording(*_record_forward(model, be, dict(zip(names, params)), inputs, gum, train_precision(model),
+                                               model.training, needs_x=ctx.needs_input_grad[8]))
         if graphed:
-            if "graph" not in ent:
-                _capture_node_forward(ent, model, be, (word_ids, char_ids, vmask, tmask, vfeat_in), gumbel,
-                                      dict(zip(names, params)), ctx.needs_input_grad[8])
-            for s, t in zip(ent["in"], (word_ids, char_ids, vmask, tmask, vfeat_in)):
-                s.copy_(t, non_blocking=True)
-            if gumbel is not None:
-                ent["gum"].copy_(gumbel, non_blocking=True)
-            ent["graph"].replay()
+            rec = _replay(ent, record, data, gumbel)
             ctx.rec = _InFlight(ent)
-            return tuple(o.v.clone() for o in ent["rec"].outs)
-        tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=model.training, precision=train_precision(model),
-                        deterministic=deterministic_mode())
-        P = _Params(tp, dict(zip(names, params)))
-        xv = tp.leaf(vfeat_in, needs=ctx.needs_input_grad[8])
-        outs = [o for o in forward_train(tp, P, word_ids, char_ids, xv, vmask, tmask, gumbel, **train_spec(model)["fwd"])
-                if o is not None]
-        ctx.rec = _Recording(tp, outs, xv, P)
-        return tuple(o.v.view_as(o.v) for o in outs)
+            return tuple(o.v.clone() for o in rec.outs)
+        ctx.rec = rec = record(data, gumbel)
+        return tuple(o.v.view_as(o.v) for o in rec.outs)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
@@ -1451,30 +1451,22 @@ class _TapeForward(torch.autograd.Function):
         ctx.rec = None
         if isinstance(rec, _InFlight):
             grads = _graphed_node_backward(rec.ent, gouts, ctx.names)
-            res = [g.reshape(shape) if g is not None else None for g, shape in zip(grads, [rec.ent["in"][4].shape] + ctx.shapes)]
-            return (None,) * 8 + tuple(res[:1]) + (None,) + tuple(res[1:])
-        be = rec.tp.be
-        gouts = [g if g is None or g.is_contiguous() else be.ewise("COPY", g) for g in gouts]   # e.g. .sum()'s expanded views
-        rec.tp.backward(list(zip(rec.outs, gouts)))
-        grads = [rec.xv.g] + [rec.P[k].g for k in ctx.names]
-        for k in _EMB_PAD_ROW:                     # nn.Embedding(padding_idx=0): row 0 gets no gradient
-            if k in rec.P.vars and rec.P[k].g is not None:
-                rec.P[k].g[0].zero_()
-        # Every returned gradient must be a tensor of its own: AccumulateGrad may adopt it as p.grad and later add into it in
-        # place.  The tape lets siblings share one gradient tensor (a + b) and passes cotangents through untouched, so a
-        # gradient whose storage is already taken by a cotangent or an earlier gradient is copied.
-        taken = {g.untyped_storage().data_ptr() for g in gouts if g is not None}
-        res = []
-        for g, shape in zip(grads, [rec.xv.v.shape] + ctx.shapes):
-            if g is not None:
-                key = g.untyped_storage().data_ptr()
-                if key in taken:
-                    g = be.ewise("COPY", g)
-                taken.add(g.untyped_storage().data_ptr())
-                g = g.reshape(shape)
-            res.append(g)
-        if ctx.ent is not None:
-            ctx.ent["seen"] += 1                  # one more eager forward + backward of this key
+        else:
+            be = rec.tp.be
+            gouts = [g if g is None or g.is_contiguous() else be.ewise("COPY", g) for g in gouts]   # e.g. .sum()'s expanded views
+            grads = _node_backward(rec, gouts, ctx.names)
+            # Every returned gradient must be a tensor of its own: AccumulateGrad may adopt it as p.grad and later add into it
+            # in place.  The tape lets siblings share one gradient tensor (a + b) and passes cotangents through untouched, so
+            # a gradient whose storage is already taken by a cotangent or an earlier gradient is copied.
+            taken = {g.untyped_storage().data_ptr() for g in gouts if g is not None}
+            for i, g in enumerate(grads):
+                if g is not None:
+                    if g.untyped_storage().data_ptr() in taken:
+                        grads[i] = g = be.ewise("COPY", g)
+                    taken.add(g.untyped_storage().data_ptr())
+            if ctx.ent is not None:
+                ctx.ent["seen"] += 1                  # one more eager forward + backward of this key
+        res = [g.reshape(shape) if g is not None else None for g, shape in zip(grads, ctx.shapes)]
         return (None,) * 8 + tuple(res[:1]) + (None,) + tuple(res[1:])
 
 
@@ -1507,11 +1499,7 @@ def forward_only(model, word_ids, char_ids, vfeat_in, vmask, tmask, gumbel=None)
     module is in ``train()`` and no gradient is wanted (``torch.no_grad()`` / ``inference_mode()``, or nothing requires grad).
     :func:`forward_differentiable` is the same forward with a graph; :func:`tape_loss` / :class:`TrainStep` run forward, the
     reference's losses and backward in one call."""
-    be = CudaBackend(vfeat_in.device)
-    tp = SeqpanTape(be, droprate=model.configs.model.droprate, training=True, precision=train_precision(model))
-    P = _Params(tp, {k: p.detach() for k, p in model.named_parameters()})
-    for v in P.vars.values():
-        v.needs = False
-    vm, tm = vmask.to(torch.float32), tmask.to(torch.float32)
-    sl, el, ms = forward_train(tp, P, word_ids, char_ids, vfeat_in.to(torch.float32), vm, tm, gumbel, **train_spec(model)["fwd"])
+    named = {k: p.detach() for k, p in model.named_parameters()}        # leaves that need no gradient: no node is recorded
+    inputs = (word_ids, char_ids, vfeat_in.to(torch.float32), vmask.to(torch.float32), tmask.to(torch.float32))
+    _, _, _, (sl, el, ms) = _record_forward(model, CudaBackend(vfeat_in.device), named, inputs, gumbel, train_precision(model), True)
     return sl.v, el.v, (ms.v if ms is not None else None)
